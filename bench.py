@@ -298,7 +298,15 @@ def main():
                     help="BASELINE configs[4] instead of the headline: sweep n = 2^10 .. 2^22 of the pairing and MSM inner "
                          "products, ONE instance of n elements sharded over the N ranks (strong scaling), one JSON line per point; "
                          "at N = 1 the CPU restatement is timed beside it on bounded sizes")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy: "
+                         "aggregate_proof.npy = the AggregateProof bytes, one float32 per byte.  The inputs are seeded, so two "
+                         "builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config5):
+        ap.error("--dump-outputs applies to the headline GPU workload only")
     if args.impl == "reference":
         return run_reference(args)
     if args.config5:
@@ -365,12 +373,15 @@ def main():
     for s, e in ev:
         flush.zero_()
         s.record()
-        step()
+        proof = step()
         e.record()
     barrier()
     launches = ctx.launches - launches0
     ms_total = max_over_ranks(sum(s.elapsed_time(e) for s, e in ev))
     value_s = ms_total / args.steps / 1e3
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "aggregate_proof.npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float32))
 
     # per-class device time of one aggregation (instrumented pass, outside the timed region)
     ctx.set_timing(True)
