@@ -237,6 +237,41 @@ int ripp_tipp_aggregate(ripp_ctx* ctx, const void* srs_g1_dev, const void* srs_g
                         const void* b_host, const void* c_host, size_t n, uint8_t* proof_out, size_t proof_cap,
                         size_t* proof_len);
 
+/* ---- deserialisation: validated decoding of untrusted ark-serialize bytes ------------------------------------ */
+/* Points as ark-serialize 0.4 / ark-bls12-381 0.4 write them (big-endian coordinates, flags in the top three bits
+ * of byte 0: 0x80 compressed, 0x40 infinity, 0x20 lexicographically largest y).  G1: x (48 B) or x || y (96 B);
+ * G2: x.c1 || x.c0 (96 B) or x.c1 || x.c0 || y.c1 || y.c0 (192 B).  Decoding validates what deserialize_* with
+ * Validate::Yes validates -- flags, canonical field encoding, curve membership (a square root for compressed points,
+ * the root picked by the sort flag), membership of the prime-order subgroup -- on the GPU, one thread per element.
+ * Each element gets one status byte: the first check it fails, in the order of ripp_decode_status. */
+typedef enum ripp_decode_status {
+  RIPP_DECODE_OK = 0,
+  RIPP_DECODE_FLAGS = 1,           /* compression bit != mode; sort bit without compression or with infinity;
+                                      infinity with any other bit set */
+  RIPP_DECODE_NONCANONICAL = 2,    /* a coordinate >= p */
+  RIPP_DECODE_NOT_ON_CURVE = 3,    /* y^2 != x^3 + b, or (compressed) x^3 + b is not a square */
+  RIPP_DECODE_NOT_IN_SUBGROUP = 4  /* on the curve, outside the prime-order subgroup */
+} ripp_decode_status;
+
+/* n elements, element i at bytes_dev + i * stride (stride >= the element's size, so the A, B, C of packed proof
+ * records decode in place); compressed = 1 / 0 selects the mode.  Writes n affine points (Montgomery; all zero for
+ * the identity and for every rejected element) and n status bytes.  Device memory, asynchronous on the context's
+ * stream: a sharded caller decodes its own share on every rank and hands it to ripp_tipp_aggregate_sharded_dev. */
+int ripp_g1_deserialize_dev(ripp_ctx* ctx, const void* bytes_dev, size_t n, size_t stride, int compressed,
+                            void* g1_aff_out_dev, uint8_t* status_dev);
+int ripp_g2_deserialize_dev(ripp_ctx* ctx, const void* bytes_dev, size_t n, size_t stride, int compressed,
+                            void* g2_aff_out_dev, uint8_t* status_dev);
+
+/* aggregate_proofs from the proofs' bytes: proofs_host holds n ark-groth16 `Proof { a, b, c }` records back to back,
+ * each written with serialize_compressed (192 B) or serialize_uncompressed (384 B), no Vec length prefix.  One H2D
+ * copy, A, B and C decoded and validated on the GPU, then ripp_tipp_aggregate_dev on the decoded vectors (same bytes
+ * out).  proofs_len != n x record size, n < 2 and any invalid element fail with RIPP_ERR_ARG, a length that is not a
+ * power of two with RIPP_ERR_NOT_POW2 -- all before any proving kernel is queued; the message of an invalid element
+ * names the first bad proof, its component and the status, e.g. "proof 17: B not in the prime-order subgroup". */
+int ripp_tipp_aggregate_serialized(ripp_ctx* ctx, const void* srs_g1_dev, const void* srs_g2_dev, const uint8_t* proofs_host,
+                                   size_t proofs_len, size_t n, int compressed, uint8_t* proof_out, size_t proof_cap,
+                                   size_t* proof_len);
+
 /* ---- SIPP (sipp/src/lib.rs; E = BLS12-381, D = Blake2s) ---------------------------------------- */
 /* product_of_pairings_with_coeffs (lib.rs:184-217): prod_i e(r_i a_i, b_i).  Affine host inputs
  * exactly as the reference takes them (&[G1Affine], &[G2Affine], &[Fr]). */

@@ -365,6 +365,28 @@ class Context:
                                         ctypes.c_size_t(n), _p(proof), ctypes.c_size_t(cap), ctypes.byref(plen)))
         return proof[: plen.value].tobytes()
 
+    # ---- deserialisation (csrc/deserialize.cu) ------------------------------------------------------
+    def g1_deserialize_dev(self, bytes_dev, n, stride, compressed, out_dev, status_dev):
+        """Decode and validate n ark-serialize G1 points at `stride` bytes (device) into affine words + status bytes."""
+        check(lib().ripp_g1_deserialize_dev(self.handle, _p(bytes_dev), ctypes.c_size_t(n), ctypes.c_size_t(stride),
+                                            int(bool(compressed)), _p(out_dev), _p(status_dev)))
+
+    def g2_deserialize_dev(self, bytes_dev, n, stride, compressed, out_dev, status_dev):
+        check(lib().ripp_g2_deserialize_dev(self.handle, _p(bytes_dev), ctypes.c_size_t(n), ctypes.c_size_t(stride),
+                                            int(bool(compressed)), _p(out_dev), _p(status_dev)))
+
+    def tipp_aggregate_serialized(self, srs_g1, srs_g2, data, n, compressed):
+        """aggregate_proofs from n ark-groth16 Proof records (bytes, 192 B compressed / 384 B uncompressed each)."""
+        k = max(n.bit_length() - 1, 0)
+        cap = 8 * 600 + 2 * (64 + k * 6 * 600 + 8 * 600)
+        proof = np.empty(cap, dtype=np.uint8)
+        plen = ctypes.c_size_t()
+        buf = self._bytes(data)
+        check(lib().ripp_tipp_aggregate_serialized(self.handle, _p(srs_g1), _p(srs_g2), _p(buf), ctypes.c_size_t(len(data)),
+                                                   ctypes.c_size_t(n), int(bool(compressed)), _p(proof), ctypes.c_size_t(cap),
+                                                   ctypes.byref(plen)))
+        return proof[: plen.value].tobytes()
+
     def sipp_product_with_coeffs(self, a, b, r):
         out = np.empty(144, dtype=np.uint32)
         check(lib().ripp_sipp_product_with_coeffs(self.handle, _p(a), _p(b), _p(r), ctypes.c_size_t(len(a)), _p(out)))

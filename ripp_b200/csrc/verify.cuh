@@ -22,6 +22,7 @@
 // every decoded element, `validate_subgroups`, before any of them reaches the endomorphism-based MSM / fold
 // kernels, whose GLV / GLS maps are scalar multiplications only inside the r-torsion).
 #pragma once
+#include "serde.cuh"
 
 // ------------------------------------------------------------------------------------------------
 // decoding (inverse of the put_* helpers; ark-serialize 0.4 uncompressed, SURVEY.md App. A-4)
@@ -169,33 +170,15 @@ static Val val_fr(const Fr& f) {
 
 // ------------------------------------------------------------------------------------------------
 // subgroup membership of everything the readers decoded (ark-ec: is_in_correct_subgroup_assuming_on_curve;
-// PairingOutput::check).  G1: phi(P) == [x^2 - 1] P, which forces [r] P = O because phi^2 + phi + 1 = 0 on the
-// whole curve and lambda^2 + lambda + 1 = r; G2: -psi(P) == [|x|] P; GT: k_gt_check6 (pairing6.cu).  The scalar
-// multiplications here are plain double-and-add: no endomorphism is trusted before the test has passed.
+// PairingOutput::check).  G1 / G2: serde::in_prime_subgroup (serde.cuh, shared with the point decoders of
+// deserialize.cu); GT: k_gt_check6 (pairing6.cu).
 // ------------------------------------------------------------------------------------------------
 template <class F>
 __global__ void __launch_bounds__(64) k_subgroup_check(const Aff<F>* __restrict__ pts, uint32_t n, uint32_t* __restrict__ bad,
                                                        uint32_t flag) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  Aff<F> p = pts[i];
-  if (p.is_inf()) return;
-  uint32_t bits[4];
-  int nbits;
-  if (sizeof(F) == sizeof(Fq)) {
-    for (int j = 0; j < 4; j++) bits[j] = k::ENDO_LAMBDA(j);
-    nbits = 128;
-  } else {
-    bits[0] = (uint32_t)k::X_ABS;
-    bits[1] = (uint32_t)(k::X_ABS >> 32);
-    bits[2] = bits[3] = 0;
-    nbits = 64;
-  }
-  Jac<F> r = scalar_mul<F>(p, bits, nbits);
-  Aff<F> q = endo_map(p);
-  F z2 = r.z.sqr();
-  bool ok = !r.is_inf() && r.x == q.x * z2 && r.y == q.y * z2 * r.z;
-  if (!ok) atomicOr(bad, flag);
+  if (!serde::in_prime_subgroup(pts[i])) atomicOr(bad, flag);
 }
 
 // *bad_mask: bit 0 = a G1 element, bit 1 = a G2 element, bit 2 = a GT element outside its prime-order subgroup

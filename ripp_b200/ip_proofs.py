@@ -157,6 +157,22 @@ def aggregate_proofs(srs, proofs, ctx=None):
     return ctx.tipp_aggregate_dev(s1, s2, a, b, c, n)
 
 
+PROOF_RECORD_BYTES = {True: 192, False: 384}
+
+
+def aggregate_proofs_serialized(srs, data, compressed=True, ctx=None):
+    """aggregate_proofs (groth16_aggregation.rs:77-160) starting from the proofs' bytes: `data` holds ark-groth16
+    `Proof { a, b, c }` records back to back, each written by serialize_compressed (192 B) or serialize_uncompressed
+    (384 B), no length prefix.  Every point is decoded and validated on the GPU (flags, canonical coordinates, curve,
+    prime-order subgroup) before the aggregation starts; an invalid record raises RippError naming the first bad proof,
+    its component and what is wrong with it.  srs = (g_alpha_powers, h_beta_powers).  -> AggregateProof bytes."""
+    ctx = ctx or default_context()
+    n = len(data) // PROOF_RECORD_BYTES[bool(compressed)]
+    s1 = ctx.to_device(codec.g1_vec_enc(srs[0]))
+    s2 = ctx.to_device(codec.g2_vec_enc(srs[1]))
+    return ctx.tipp_aggregate_serialized(s1, s2, data, n, compressed)
+
+
 def verify_aggregate_proof(v_srs, vk, public_inputs, proof, ctx=None):
     """groth16_aggregation.rs:162-231.  public_inputs: one list of Fr per proof; proof: aggregate_proofs' bytes.  -> bool"""
     ctx = ctx or default_context()

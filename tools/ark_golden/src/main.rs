@@ -5,7 +5,9 @@
 //!   scalar(tag, i, seed) = Fr::from_le_bytes(first 31 bytes of Blake2b-512("ripp-b200/" || tag || LE64(seed) || LE64(i)))
 //!   g1_points(tag, n)[i] = scalar(tag, i) * G1::generator(),  g2_points likewise
 //!   SRS: alpha = scalar("srs-alpha", 0), beta = scalar("srs-beta", 0), powers as TIPA::setup computes them.
-//! Every value is `serialize_uncompressed` bytes, hex encoded.
+//! Every value is `serialize_uncompressed` bytes, hex encoded, except the `g*c_*` compressed encodings and the
+//! `serde_verdict_*` decoder verdicts (hex of "ok" || the decoded point uncompressed, "flags", "invalid" or "other").
+//! Usage: cargo run --release -p ark-golden -- <path of tests/golden/serde_cases.txt> > tests/golden/ark_golden.json
 use ark_bls12_381::{Bls12_381, Fr, G1Projective as G1, G2Projective as G2};
 use ark_dh_commitments::{
     afgho16::{AFGHOCommitmentG1, AFGHOCommitmentG2},
@@ -66,6 +68,19 @@ fn srs(n: usize) -> SRS<Bls12_381> {
         g_beta: g * beta,
         h_alpha: h * alpha,
     }
+}
+
+/// `serde_case_<group>_<c|u>_<name> <hex>` lines of tests/golden/serde_cases.txt; its path is the first argument.
+fn serde_cases() -> Vec<(String, Vec<u8>)> {
+    let path = std::env::args().nth(1).unwrap_or_else(|| "serde_cases.txt".into());
+    let text = std::fs::read_to_string(&path).expect("pass the path of tests/golden/serde_cases.txt");
+    let unhex = |h: &str| (0..h.len()).step_by(2).map(|i| u8::from_str_radix(&h[i..i + 2], 16).unwrap()).collect::<Vec<u8>>();
+    text.lines()
+        .filter_map(|l| {
+            let mut it = l.split_whitespace();
+            Some((it.next()?.to_string(), unhex(it.next()?)))
+        })
+        .collect()
 }
 
 type GC1 = AFGHOCommitmentG1<Bls12_381>;
@@ -181,6 +196,54 @@ fn main() {
                 r.serialize_uncompressed(&mut pb).unwrap();
             }
             out.push(("bls12_377_sipp_n8_proof".into(), pb.iter().map(|x| format!("{:02x}", x)).collect()));
+        }
+    }
+
+    // Point encodings for the validating decoders (oracle/serde.py de_g1 / de_g2, csrc/serde.cuh): compressed forms
+    // of the points above, and arkworks' verdict (deserialize_with_mode, Validate::Yes) on every encoding listed in
+    // tests/golden/serde_cases.txt (oracle/serde_cases.py named_cases: each flag rule, x = p, an x off the curve, a point
+    // off the subgroup, valid points), as `serde_verdict_<group>_<c|u>_<name>`.
+    {
+        use ark_bls12_381::{G1Affine, G2Affine};
+        use ark_serialize::{CanonicalDeserialize, Compress, SerializationError, Validate};
+        let comp = |v: &dyn Fn(&mut Vec<u8>)| -> String {
+            let mut b = Vec::new();
+            v(&mut b);
+            b.iter().map(|x| format!("{:02x}", x)).collect()
+        };
+        let g1 = g1_points("gipa-a", 1)[0].into_affine();
+        let g2 = g2_points("gipa-b", 1)[0].into_affine();
+        out.push(("g1c_gipa-a_0".into(), comp(&|b| g1.serialize_compressed(b).unwrap())));
+        out.push(("g2c_gipa-b_0".into(), comp(&|b| g2.serialize_compressed(b).unwrap())));
+        out.push(("g1c_generator".into(), comp(&|b| G1::generator().into_affine().serialize_compressed(b).unwrap())));
+        out.push(("g2c_generator".into(), comp(&|b| G2::generator().into_affine().serialize_compressed(b).unwrap())));
+        // verdicts: "ok:<uncompressed bytes of the point>" or the SerializationError variant
+        let verdict = |r: Result<Vec<u8>, SerializationError>| -> String {
+            match r {
+                Ok(b) => format!("6f6b{}", b.iter().map(|x| format!("{:02x}", x)).collect::<String>()),  // "ok" || point
+                Err(SerializationError::UnexpectedFlags) => "666c616773".into(),                          // "flags"
+                Err(SerializationError::InvalidData) => "696e76616c6964".into(),                          // "invalid"
+                Err(_) => "6f74686572".into(),                                                            // "other"
+            }
+        };
+        let cases: Vec<(String, Vec<u8>)> = serde_cases();
+        for (key, bytes) in cases {
+            let compressed = key.contains("_c_");
+            let mode = if compressed { Compress::Yes } else { Compress::No };
+            let r = if key.starts_with("serde_case_1_") {
+                G1Affine::deserialize_with_mode(&bytes[..], mode, Validate::Yes).map(|p| {
+                    let mut b = Vec::new();
+                    p.serialize_uncompressed(&mut b).unwrap();
+                    b
+                })
+            } else {
+                G2Affine::deserialize_with_mode(&bytes[..], mode, Validate::Yes).map(|p| {
+                    let mut b = Vec::new();
+                    p.serialize_uncompressed(&mut b).unwrap();
+                    b
+                })
+            };
+            out.push((key.replace("serde_case_", "serde_verdict_"), verdict(r)));
         }
     }
 

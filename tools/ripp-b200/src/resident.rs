@@ -15,7 +15,7 @@ use ark_ec::{pairing::PairingOutput, CurveGroup};
 use ark_groth16::{Proof, VerifyingKey};
 use ark_inner_products::{Error, MultiexponentiationInnerProduct, PairingInnerProduct};
 use ark_ip_proofs::tipa::{structured_scalar_message::TIPAWithSSMProof, TIPAProof, VerifierSRS};
-use ark_serialize::{CanonicalDeserialize, CanonicalSerialize};
+use ark_serialize::{CanonicalDeserialize, CanonicalSerialize, Compress};
 use blake2::Blake2b;
 use ripp_b200_sys as sys;
 use std::marker::PhantomData;
@@ -241,6 +241,33 @@ pub fn aggregate_proofs(srs: &GpuSrs, proofs: &[Proof<Bls12_381>]) -> Result<Agg
     drop(c);
     check(st, n, n)?;
     buf.truncate(len);
+    parse_aggregate(buf)
+}
+
+/// `aggregate_proofs` from the proofs' bytes, as an aggregation service receives them from untrusted provers: `proofs`
+/// holds n ark-groth16 `Proof` records back to back, each written with `serialize_with_mode(compress)` (192 B
+/// compressed, 384 B uncompressed), no length prefix.  The library decodes and validates every point on the GPU
+/// (flags, canonical coordinates, curve, prime-order subgroup: what `deserialize_with_mode(_, compress, Validate::Yes)`
+/// checks) before aggregating; an invalid record fails with a `GpuError` naming the proof, its component and the reason.
+pub fn aggregate_proofs_serialized(srs: &GpuSrs, proofs: &[u8], compress: Compress) -> Result<AggregateProofParts, Error> {
+    let record = if compress == Compress::Yes { 192 } else { 384 };
+    let n = proofs.len() / record;
+    let mut buf = vec![0u8; 8192 + 2 * proof_capacity(n)];
+    let mut len = 0usize;
+    let c = ctx();
+    let st = unsafe {
+        sys::ripp_tipp_aggregate_serialized(c.raw(), srs.g_alpha_powers.ptr(), srs.h_beta_powers.ptr(), proofs.as_ptr(),
+                                            proofs.len(), n, (compress == Compress::Yes) as i32, buf.as_mut_ptr(), buf.len(),
+                                            &mut len)
+    };
+    drop(c);
+    check(st, n, n)?;
+    buf.truncate(len);
+    parse_aggregate(buf)
+}
+
+// AggregateProof { com_a, com_b, com_c, ip_ab, agg_c, tipa_proof_ab, tipa_proof_c } (groth16_aggregation.rs:58-66)
+fn parse_aggregate(buf: Vec<u8>) -> Result<AggregateProofParts, Error> {
     let mut rd = &buf[..];
     let com_a = PairingOutput::<Bls12_381>::deserialize_uncompressed_unchecked(&mut rd)?;
     let com_b = PairingOutput::<Bls12_381>::deserialize_uncompressed_unchecked(&mut rd)?;
