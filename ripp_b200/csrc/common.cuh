@@ -131,7 +131,10 @@ bool ripp_use_l6();
 // comm.cu: all-gather of one `bytes`-sized blob per rank on ctx's stream (recv = world * bytes, rank order); world == 1 copies
 int ripp_all_gather_internal(ripp_ctx* ctx, const void* send_dev, size_t bytes, void* recv_dev);
 void ripp_comm_release(ripp_ctx* ctx);
-// msm.cu: the (up to four) folds of one GIPA round in ONE launch when the vectors are short enough for lane teams
+// msm.cu: the (up to four) folds of one GIPA round in ONE launch when the vectors are short enough for lane teams;
+// with `pre` (written by ripp_fold_pre_internal, for vectors up to ripp_fold_pre_max_n()) over precomputed bases
 int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, const void* const* lo, const void* const* cs, size_t n,
-                        void* const* out, int* fused);
+                        void* const* out, int* fused, const void* const* pre = nullptr);
+int ripp_fold_pre_internal(ripp_ctx* ctx, const int* types, const void* const* hi, size_t n, void* const* pre);
+size_t ripp_fold_pre_max_n();
 int ripp_pairing6_init_device();  // per-device kernel attributes; called by ripp_ctx_create with the device current

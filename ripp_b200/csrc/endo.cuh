@@ -122,6 +122,38 @@ RIPP_HD void endo_decompose(const uint32_t* canon, EndoBits& b) {
   }
 }
 
+// Split recoding for the fold with precomputed bases (msm.cu: k_fold_pre, k_fold4_xp<true>): the NAF of digit k is cut at
+// bit H, digits below H stay on E^k(P) and digits at H and above go to E^k(D), D = [2^H] P, at position j - H.  Cutting the
+// NAF rather than the integer keeps the sum exact when the recoding carries past bit H.  Part 2k + s holds the low (s = 0)
+// or high (s = 1) half of digit k: G1 (H = 64) four parts of <= 65 digits, G2 (H = 32) eight parts of <= 33 digits, so
+// the chain of a part is half of what it walks without D.
+template <int GROUP>
+struct SplitOf {
+  static constexpr int H = GROUP == 1 ? 64 : 32;
+  static constexpr int PARTS = GROUP == 1 ? 4 : 8;  // 2 x endo_digits' MAXD
+};
+struct EndoSplit {
+  uint32_t pos[8][3], neg[8][3];
+  int nbits[8];  // digits of each part
+};
+
+template <int GROUP>
+RIPP_HD void endo_split(const EndoBits& b, EndoSplit& s) {
+  constexpr int H = SplitOf<GROUP>::H;
+  for (int t = 0; t < 8; t++) {
+    s.nbits[t] = 0;
+    for (int w = 0; w < 3; w++) s.pos[t][w] = s.neg[t][w] = 0;
+  }
+  for (int k = 0; k < SplitOf<GROUP>::PARTS / 2; k++)
+    for (int j = 0; j < 160; j++) {
+      const bool ps = (b.pos[k][j >> 5] >> (j & 31)) & 1, ng = (b.neg[k][j >> 5] >> (j & 31)) & 1;
+      if (!(ps || ng)) continue;
+      const int t = 2 * k + (j >= H), i = j >= H ? j - H : j;  // i < 96: a digit's NAF has at most 129 positions
+      (ps ? s.pos : s.neg)[t][i >> 5] |= 1u << (i & 31);
+      if (i + 1 > s.nbits[t]) s.nbits[t] = i + 1;
+    }
+}
+
 // Same sum when every lane of a warp has its OWN scalar: one addition slot per (bit, digit) whose operand is
 // selected (+base, -base or the identity), so the warp runs the addition body once per slot instead of once per
 // distinct sign pattern.

@@ -235,7 +235,9 @@ static void gipa_challenge(const Fr& prev, const Val* com, Fr* c, Fr* c_inv) {
 // gipa.rs:261-291 for one round: A <- A_R c + A_L, B <- B_R c^-1 + B_L, v <- v_R c^-1 + v_L, w <- w_R c + w_L, in place over
 // the lower halves.  Short vectors: ONE fused launch on ctx's stream; long ones: four kernels on four streams.
 static int fold_typed(ripp_ctx* ctx, int t, char* base, size_t split, const Fr& c);
-static int fold_round(ripp_ctx* ctx, const int* types, char* const* bases, size_t split, const Fr& c, const Fr& c_inv) {
+// pre: NULL, or the [2^H] images of the upper halves that fold_pre queued (fused launch over precomputed bases)
+static int fold_round(ripp_ctx* ctx, const int* types, char* const* bases, size_t split, const Fr& c, const Fr& c_inv,
+                      void* const* pre = nullptr) {
   const void *hi[4], *lo[4], *cs[4];
   void* out[4];
   int ty[4];
@@ -248,7 +250,7 @@ static int fold_round(ripp_ctx* ctx, const int* types, char* const* bases, size_
     cs[i] = sc[i]->v;
   }
   int fused = 0;
-  OK(ripp_fold4_internal(ctx, ty, hi, lo, cs, split, out, &fused));
+  OK(ripp_fold4_internal(ctx, ty, hi, lo, cs, split, out, &fused, pre));
   if (fused) return RIPP_OK;
   ripp_ctx* k1 = ripp_child(ctx, 0);
   ripp_ctx* k2 = ripp_child(ctx, 1);
@@ -265,6 +267,25 @@ static int fold_round(ripp_ctx* ctx, const int* types, char* const* bases, size_
   OK(ripp_join(ctx, k2));
   OK(ripp_join(ctx, k3));
   return RIPP_OK;
+}
+
+// The challenge-independent half of a short round's folds: D = [2^H] of every G1 / G2 element of the upper halves, queued
+// on child 7 (eval_products and fold_round use children 0-5, tipa_prove 5) before the round's products, so that it runs
+// in the Miller / final exponentiation / hash window; the caller joins the child before fold_round reads `pre`.
+static int fold_pre(ripp_ctx* ctx, const int* types, char* const* bases, size_t split, char* buf, void** pre) {
+  int ty[4];
+  const void* hi[4];
+  size_t off = 0;
+  for (int i = 0; i < 4; i++) {
+    ty[i] = (types[i] == VT_G1 || types[i] == VT_G2) && bases[i] ? types[i] : 0;
+    hi[i] = ty[i] ? bases[i] + split * vt_size(types[i]) : nullptr;
+    pre[i] = ty[i] ? buf + off : nullptr;
+    if (ty[i]) off += split * vt_size(types[i]);
+  }
+  ripp_ctx* kid = ripp_child(ctx, 7);
+  if (!kid) return fail(RIPP_ERR_CUDA, "child context");
+  OK(ripp_fork(ctx, kid));
+  return ripp_fold_pre_internal(kid, ty, hi, split, pre);
 }
 
 static int fold_typed(ripp_ctx* ctx, int t, char* base, size_t split, const Fr& c) {
@@ -328,9 +349,24 @@ static int gipa_prove(ripp_ctx* ctx, const GipaSpec& sp, const void* a_in, const
   std::vector<Fr> transcript;
   if (pre_steps) steps = *pre_steps;
   if (pre_transcript) transcript = *pre_transcript;
+  // [2^H] images of the upper halves for the rounds with split <= pre_max (fold_pre), sized for the first of them
+  const size_t pre_max = ripp_fold_pre_max_n();
+  char* pre_buf = nullptr;
+  if (pre_max && n >= 2) {
+    const size_t first = n / 2 < pre_max ? n / 2 : pre_max;
+    size_t bytes = 0;
+    for (int t : {sp.a, sp.b, sp.v, sp.w})
+      if (t == VT_G1 || t == VT_G2) bytes += first * vt_size(t);
+    if (bytes) OK(scratch(ctx, 29, bytes, (void**)&pre_buf));
+  }
   size_t len = n;
   while (len > 1) {
     size_t split = len / 2;
+    const int types[4] = {sp.a, sp.b, sp.v, sp.w};
+    char* const bases[4] = {A, B, V, W};
+    void* pre[4];
+    const bool use_pre = pre_buf && split <= pre_max;
+    if (use_pre) OK(fold_pre(ctx, types, bases, split, pre_buf, pre));
     // gipa.rs:209-231 -- com_1 = (IP(A_R, v_L), IP(w_R, B_L), IP(A_R, B_L)); com_2 = (IP(A_L, v_R), IP(w_L, B_R), IP(A_L, B_R))
     Slice xs[6] = {at(sp.a, A, split), at(sp.w, W, split), at(sp.a, A, split), at(sp.a, A, 0), at(sp.w, W, 0), at(sp.a, A, 0)};
     Slice ys[6] = {at(sp.v, V, 0), at(sp.b, B, 0), at(sp.b, B, 0), at(sp.v, V, split), at(sp.b, B, split), at(sp.b, B, split)};
@@ -344,11 +380,8 @@ static int gipa_prove(ripp_ctx* ctx, const GipaSpec& sp, const void* a_in, const
     Fr c, c_inv;
     gipa_challenge(transcript.empty() ? (prev0 ? *prev0 : Fr::zero()) : transcript.back(), com.data(), &c, &c_inv);
     // gipa.rs:261-291 -- rescale
-    {
-      const int types[4] = {sp.a, sp.b, sp.v, sp.w};
-      char* const bases[4] = {A, B, V, W};
-      OK(fold_round(ctx, types, bases, split, c, c_inv));
-    }
+    if (use_pre) OK(ripp_join(ctx, ripp_child(ctx, 7)));
+    OK(fold_round(ctx, types, bases, split, c, c_inv, use_pre ? pre : nullptr));
     steps.push_back(com);
     transcript.push_back(c);
     len = split;

@@ -734,6 +734,9 @@ struct FoldJob {
   uint32_t n, first_block;
   EndoBits c;  // G1 / G2
   Fr s;        // Fr
+  // fold with precomputed bases (k_fold4_xp<true>): D_i = [2^H] hi_i written by k_fold_pre, and c split at bit H
+  const void* pre;
+  EndoSplit cs;
 };
 struct FoldJobs {
   FoldJob j[4];
@@ -778,22 +781,32 @@ __global__ void __launch_bounds__(32 * XT_WARPS) k_fold4_xt(const FoldJobs jobs)
 // on endomorphism part w % m of the elements of group w / m (m = 4 parts for G2: one group of 3 elements per CTA; m = 2
 // for G1: two groups of 10), every team brings its part to affine form, and after the CTA barrier the part-0 warp adds
 // lo and the m parts.  Same group element as fold_xt_body (the sum is exact), half the dependent chain.
-constexpr int XP_WARPS = 4;
-template <class F>
+// PRE: the split recoding (endo.cuh: endo_split) over the bases {E^k(hi_i), E^k(D_i)}, D_i = job.pre[i] = [2^H] hi_i
+// precomputed by k_fold_pre while the round's products ran: twice the parts (G1 4, G2 8) at half the chain, eight warps.
+template <bool PRE>
+struct XpShape {
+  static constexpr int WARPS = PRE ? 8 : 4;
+  template <class F>  // the layout does not depend on the scalar: the group's full part count
+  static constexpr int PARTS = (sizeof(F) == sizeof(Fq) ? 2 : 4) * (PRE ? 2 : 1);
+};
+constexpr int XP_WARPS = XpShape<false>::WARPS;
+template <class F, int WARPS>
 struct XpLayout {
   typedef xt::TeamOf<F> TO;
   static constexpr int AW = sizeof(Aff<F>) / 4;
   static constexpr int TEAM_WORDS = 2 * TO::BUS_WORDS + AW;
-  static constexpr int PARTS_AT = XP_WARPS * TO::PER_WARP * TEAM_WORDS;
-  static constexpr int WORDS = PARTS_AT + XP_WARPS * TO::PER_WARP * AW;  // (group, element, part) slots: groups * m = XP_WARPS
+  static constexpr int PARTS_AT = WARPS * TO::PER_WARP * TEAM_WORDS;
+  static constexpr int WORDS = PARTS_AT + WARPS * TO::PER_WARP * AW;  // (group, element, part) slots: groups * m = WARPS
 };
-template <class F>
+template <class F, bool PRE>
 __device__ __forceinline__ void fold_xp_body(uint32_t* sm, const FoldJob& job, uint32_t block) {
   typedef xt::TeamOf<F> TO;
-  typedef XpLayout<F> L;
+  constexpr int WARPS = XpShape<PRE>::WARPS;
+  typedef XpLayout<F, WARPS> L;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr int m = sizeof(F) == sizeof(Fq) ? 2 : 4;  // endo_digits' MAXD: the layout does not depend on the scalar
-  const int part = warp % m, grp = warp / m, groups = XP_WARPS / m;
+  constexpr int m = XpShape<PRE>::template PARTS<F>;
+  constexpr int mk = PRE ? m / 2 : m;  // powers of E
+  const int part = warp % m, grp = warp / m, groups = WARPS / m;
   const int vl = lane % (TO::LANES * TO::PER_WARP);
   const int e = vl / TO::LANES;
   size_t i = ((size_t)block * groups + grp) * TO::PER_WARP + e;
@@ -803,7 +816,14 @@ __device__ __forceinline__ void fold_xp_body(uint32_t* sm, const FoldJob& job, u
   uint32_t* slots = sm + L::PARTS_AT + ((grp * TO::PER_WARP + e) * m) * L::AW;
   xt::Team tm{vl % TO::LANES, scratch, 0, nullptr};
   {
-    Jac<F> acc = xt::part_mul<F>(tm, ((const Aff<F>*)job.hi)[i], job.c, m, part, scratch + 2 * TO::BUS_WORDS);
+    Jac<F> acc;
+    if (PRE) {
+      const Aff<F>* src = (const Aff<F>*)((part & 1) ? job.pre : job.hi);
+      acc = xt::naf_mul_endo<F>(tm, src[i], mk, part >> 1, job.cs.pos[part], job.cs.neg[part], job.cs.nbits[part],
+                                scratch + 2 * TO::BUS_WORDS);
+    } else {
+      acc = xt::part_mul<F>(tm, ((const Aff<F>*)job.hi)[i], job.c, mk, part, scratch + 2 * TO::BUS_WORDS);
+    }
     Aff<F> pa = xt::to_affine<F>(tm, acc);
     if (tm.t == 0 && lane == vl) xt::aff_st<F>(slots + part * L::AW, pa);
   }
@@ -816,8 +836,9 @@ __device__ __forceinline__ void fold_xp_body(uint32_t* sm, const FoldJob& job, u
     if (live && tm.t == 0) ((Aff<F>*)job.out)[i] = o;
   }
 }
-__global__ void __launch_bounds__(32 * XP_WARPS) k_fold4_xp(const FoldJobs jobs) {
-  constexpr int W1 = XpLayout<Fq>::WORDS, W2 = XpLayout<Fq2>::WORDS;
+template <bool PRE>
+__global__ void __launch_bounds__(32 * XpShape<PRE>::WARPS) k_fold4_xp(const FoldJobs jobs) {
+  constexpr int W1 = XpLayout<Fq, XpShape<PRE>::WARPS>::WORDS, W2 = XpLayout<Fq2, XpShape<PRE>::WARPS>::WORDS;
   __shared__ __align__(16) uint32_t sm[W1 > W2 ? W1 : W2];
   int k = 0;
 #pragma unroll
@@ -826,12 +847,46 @@ __global__ void __launch_bounds__(32 * XP_WARPS) k_fold4_xp(const FoldJobs jobs)
   const FoldJob& job = jobs.j[k];
   const uint32_t block = blockIdx.x - job.first_block;
   if (job.type == 1) {
-    fold_xp_body<Fq>(sm, job, block);
+    fold_xp_body<Fq, PRE>(sm, job, block);
   } else if (job.type == 2) {
-    fold_xp_body<Fq2>(sm, job, block);
+    fold_xp_body<Fq2, PRE>(sm, job, block);
   } else if (job.type == 3) {
     size_t i = (size_t)block * blockDim.x + threadIdx.x;
     if (i < job.n) ((Fr*)job.out)[i] = ((const Fr*)job.hi)[i] * job.s + ((const Fr*)job.lo)[i];
+  }
+}
+
+// D_i = [2^H] hi_i for the G1 / G2 jobs of a round (job.out = the fold's `pre`): lane teams as k_fold4_xt, no scalar.
+// Runs on its own stream while the round's products and its challenge are computed.
+__global__ void __launch_bounds__(32 * XT_WARPS) k_fold_pre(const FoldJobs jobs) {
+  constexpr int W1 = xt::TeamOf<Fq>::PER_WARP * 2 * xt::TeamOf<Fq>::BUS_WORDS;
+  constexpr int W2 = xt::TeamOf<Fq2>::PER_WARP * 2 * xt::TeamOf<Fq2>::BUS_WORDS;
+  __shared__ __align__(16) uint32_t bus[XT_WARPS * (W1 > W2 ? W1 : W2)];
+  int k = 0;
+#pragma unroll
+  for (int t = 1; t < 4; t++)
+    if (jobs.j[t].type && blockIdx.x >= jobs.j[t].first_block) k = t;
+  const FoldJob& job = jobs.j[k];
+  const uint32_t block = blockIdx.x - job.first_block;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (job.type == 1) {
+    typedef xt::TeamOf<Fq> TO;
+    const int vl = lane % (TO::LANES * TO::PER_WARP), e = vl / TO::LANES;
+    size_t i = ((size_t)block * XT_WARPS + warp) * TO::PER_WARP + e;
+    const bool live = i < job.n && lane == vl;
+    if (i >= job.n) i = job.n - 1;
+    xt::Team tm{vl % TO::LANES, bus + (warp * TO::PER_WARP + e) * 2 * TO::BUS_WORDS, 0, nullptr};
+    G1Aff d = xt::pow2_mul<Fq>(tm, ((const G1Aff*)job.hi)[i], SplitOf<1>::H);
+    if (live && tm.t == 0) ((G1Aff*)job.out)[i] = d;
+  } else if (job.type == 2) {
+    typedef xt::TeamOf<Fq2> TO;
+    const int vl = lane % (TO::LANES * TO::PER_WARP), e = vl / TO::LANES;
+    size_t i = ((size_t)block * XT_WARPS + warp) * TO::PER_WARP + e;
+    const bool live = i < job.n && lane == vl;
+    if (i >= job.n) i = job.n - 1;
+    xt::Team tm{vl % TO::LANES, bus + (warp * TO::PER_WARP + e) * 2 * TO::BUS_WORDS, 0, nullptr};
+    G2Aff d = xt::pow2_mul<Fq2>(tm, ((const G2Aff*)job.hi)[i], SplitOf<2>::H);
+    if (live && tm.t == 0) ((G2Aff*)job.out)[i] = d;
   }
 }
 // vectors up to this length fold part-parallel (RIPP_B200_XP_MAX overrides; 0 = never).  Measured on the 2^12 aggregation
@@ -845,10 +900,51 @@ static size_t xp_max_n() {
   return (size_t)v;
 }
 
+// vectors up to this length fold with precomputed bases (RIPP_B200_FOLD_PRE_MAX overrides; 0 = never); never above
+// the lane-team range, and not under a forced fold kernel.  Measured on the 2^12 aggregation (profiles/r3a_fold_pre.json):
+// 62.8 ms at 128 against 64.9 with none, 63.1 at 256, 70.1 at 1024 (there the precompute competes with the Miller kernels).
+size_t ripp_fold_pre_max_n() {
+  static const long v = [] {
+    const char* e = getenv("RIPP_B200_FOLD_PRE_MAX");
+    return e ? atol(e) : 128L;
+  }();
+  if (fold_mode() != 0 || v <= 0) return 0;
+  return (size_t)v < xt_max_n() ? (size_t)v : xt_max_n();
+}
+
+// pre[t] = [2^H] hi[t] (n elements each) for the G1 / G2 entries of types[] (others ignored), on ctx's stream
+int ripp_fold_pre_internal(ripp_ctx* ctx, const int* types, const void* const* hi, size_t n, void* const* pre) {
+  if (n == 0) return RIPP_OK;
+  CU(cudaSetDevice(ctx->device));
+  FoldJobs jobs;
+  memset(&jobs, 0, sizeof(jobs));
+  uint32_t nblocks = 0;
+  int nj = 0;
+  for (int t = 0; t < 4; t++) {
+    if ((types[t] != 1 && types[t] != 2) || !hi[t]) continue;
+    FoldJob& j = jobs.j[nj++];
+    j.type = types[t];
+    j.hi = hi[t];
+    j.out = pre[t];
+    j.n = (uint32_t)n;
+    j.first_block = nblocks;
+    const uint32_t per = types[t] == 1 ? xt::TeamOf<Fq>::PER_WARP : xt::TeamOf<Fq2>::PER_WARP;
+    const uint32_t warps = (uint32_t)((n + per - 1) / per);
+    nblocks += (warps + XT_WARPS - 1) / XT_WARPS;
+  }
+  if (!nj) return RIPP_OK;
+  TimeScope ts_(ctx, RIPP_T_FOLD);
+  k_fold_pre<<<nblocks, 32 * XT_WARPS, 0, ctx->stream>>>(jobs);
+  LAUNCHED(ctx);
+  return RIPP_OK;
+}
+
 // types[t] in {0 none, 1 G1, 2 G2, 3 Fr}; out[t][i] = hi[t][i] * c[t] + lo[t][i].  Returns RIPP_OK and *fused = 1 when the
 // fused launch was used (all vectors short enough for lane teams), *fused = 0 when the caller should fold one by one.
+// pre: NULL, or per job the [2^H] hi images that ripp_fold_pre_internal wrote (then the G1 / G2 folds run
+// k_fold4_xp<true>, whatever the part-parallel range)
 int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, const void* const* lo, const void* const* cs, size_t n,
-                        void* const* out, int* fused) {
+                        void* const* out, int* fused, const void* const* pre) {
   *fused = 0;
   if (fold_mode() != 0 || n == 0 || n > xt_max_n()) return RIPP_OK;
   CU(cudaSetDevice(ctx->device));
@@ -856,7 +952,8 @@ int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, 
   memset(&jobs, 0, sizeof(jobs));
   uint32_t nblocks = 0;
   int nj = 0;
-  const bool xp = n <= xp_max_n();
+  const bool xp = pre || n <= xp_max_n();
+  const int xp_warps = pre ? XpShape<true>::WARPS : XP_WARPS;
   for (int t = 0; t < 4; t++) {
     if (!types[t] || !hi[t]) continue;
     FoldJob& j = jobs.j[nj++];
@@ -869,15 +966,25 @@ int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, 
     uint32_t blocks;
     if (types[t] == 1) {
       j.c = endo_bits<Fq>(cs[t]);
+      if (pre) {
+        j.pre = pre[t];
+        endo_split<1>(j.c, j.cs);
+      }
       uint32_t warps = (uint32_t)((n + xt::TeamOf<Fq>::PER_WARP - 1) / xt::TeamOf<Fq>::PER_WARP);
-      blocks = xp ? (warps * 2 + XP_WARPS - 1) / XP_WARPS : (warps + XT_WARPS - 1) / XT_WARPS;
+      const int m = pre ? XpShape<true>::PARTS<Fq> : XpShape<false>::PARTS<Fq>;
+      blocks = xp ? (warps * m + xp_warps - 1) / xp_warps : (warps + XT_WARPS - 1) / XT_WARPS;
     } else if (types[t] == 2) {
       j.c = endo_bits<Fq2>(cs[t]);
+      if (pre) {
+        j.pre = pre[t];
+        endo_split<2>(j.c, j.cs);
+      }
       uint32_t warps = (uint32_t)((n + xt::TeamOf<Fq2>::PER_WARP - 1) / xt::TeamOf<Fq2>::PER_WARP);
-      blocks = xp ? (warps * 4 + XP_WARPS - 1) / XP_WARPS : (warps + XT_WARPS - 1) / XT_WARPS;
+      const int m = pre ? XpShape<true>::PARTS<Fq2> : XpShape<false>::PARTS<Fq2>;
+      blocks = xp ? (warps * m + xp_warps - 1) / xp_warps : (warps + XT_WARPS - 1) / XT_WARPS;
     } else {
       memcpy(j.s.v, cs[t], sizeof(Fr));
-      const uint32_t bt = 32 * (xp ? XP_WARPS : XT_WARPS);
+      const uint32_t bt = 32 * (xp ? xp_warps : XT_WARPS);
       blocks = (uint32_t)((n + bt - 1) / bt);
     }
     nblocks += blocks;
@@ -888,8 +995,10 @@ int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, 
   }
   // jobs are packed at the front of the array in launch order: unused slots keep type 0
   TimeScope ts_(ctx, RIPP_T_FOLD);
-  if (xp)
-    k_fold4_xp<<<nblocks, 32 * XP_WARPS, 0, ctx->stream>>>(jobs);
+  if (pre)
+    k_fold4_xp<true><<<nblocks, 32 * xp_warps, 0, ctx->stream>>>(jobs);
+  else if (xp)
+    k_fold4_xp<false><<<nblocks, 32 * xp_warps, 0, ctx->stream>>>(jobs);
   else
     k_fold4_xt<<<nblocks, 32 * XT_WARPS, 0, ctx->stream>>>(jobs);
   LAUNCHED(ctx);

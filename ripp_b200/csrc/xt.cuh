@@ -236,8 +236,10 @@ RIPP_HD Jac<F> endo_mul(const Team& tm, const Aff<F>& p, const EndoBits& c, uint
 // warp: the bit pattern of a part is the warp's control flow) and adds the parts afterwards, so the dependent chain of
 // an element is one 64-bit (G2) / 128-bit (G1) double-and-add instead of four / two interleaved ones.
 // `base`: sizeof(Aff<F>) / 4 words of the team's scratch.
+// d E^k(p) for one NAF digit set d (`nbits` digits in the bitmaps pos / neg): the chain of one part.
 template <class F>
-RIPP_HD Jac<F> part_mul(const Team& tm, const Aff<F>& p, const EndoBits& c, int m, int part, uint32_t* base) {
+RIPP_HD Jac<F> naf_mul_endo(const Team& tm, const Aff<F>& p, int m, int k, const uint32_t* pos, const uint32_t* neg, int nbits,
+                            uint32_t* base) {
   constexpr int AW = sizeof(Aff<F>) / 4;
   {
     // every lane walks the whole chain p, E(p), E^2(p), ... and keeps the image of its part (word-wise select)
@@ -248,16 +250,16 @@ RIPP_HD Jac<F> part_mul(const Team& tm, const Aff<F>& p, const EndoBits& c, int 
       uint32_t* mw = reinterpret_cast<uint32_t*>(&mine);
       const uint32_t* bw = reinterpret_cast<const uint32_t*>(&b);
 #pragma unroll
-      for (int i = 0; i < AW; i++) mw[i] = t == part ? bw[i] : mw[i];
+      for (int i = 0; i < AW; i++) mw[i] = t == k ? bw[i] : mw[i];
     }
     if (tm.t == 0) aff_st<F>(base, mine);
   }
   sync(tm);
   Jac<F> acc = Jac<F>::inf();
 #pragma unroll 1
-  for (int j = c.nbits - 1; j >= 0; j--) {
+  for (int j = nbits - 1; j >= 0; j--) {
     acc = dbl<F>(tm, acc);
-    const bool ps = (c.pos[part][j >> 5] >> (j & 31)) & 1, ng = (c.neg[part][j >> 5] >> (j & 31)) & 1;
+    const bool ps = (pos[j >> 5] >> (j & 31)) & 1, ng = (neg[j >> 5] >> (j & 31)) & 1;
     if (ps || ng) {
       Aff<F> q = aff_ld<F>(base);
       if (ng) q = q.neg();
@@ -265,6 +267,19 @@ RIPP_HD Jac<F> part_mul(const Team& tm, const Aff<F>& p, const EndoBits& c, int 
     }
   }
   return acc;
+}
+template <class F>
+RIPP_HD Jac<F> part_mul(const Team& tm, const Aff<F>& p, const EndoBits& c, int m, int part, uint32_t* base) {
+  return naf_mul_endo<F>(tm, p, m, part, c.pos[part], c.neg[part], c.nbits, base);
+}
+
+// [2^h] p in affine form: the base D of the split recoding's high parts (endo.cuh: endo_split); the identity stays the identity
+template <class F>
+RIPP_HD Aff<F> pow2_mul(const Team& tm, const Aff<F>& p, int h) {
+  Jac<F> a = Jac<F>::from_affine(p);
+#pragma unroll 1
+  for (int i = 0; i < h; i++) a = dbl<F>(tm, a);
+  return to_affine<F>(tm, a);
 }
 
 // Same sum when every TEAM has its own scalar (element-wise scalings a_i r^i, ck_i r^-i of groth16_aggregation.rs:118-131,
