@@ -272,6 +272,42 @@ int ripp_tipp_aggregate_serialized(ripp_ctx* ctx, const void* srs_g1_dev, const 
                                    size_t proofs_len, size_t n, int compressed, uint8_t* proof_out, size_t proof_cap,
                                    size_t* proof_len);
 
+/* ---- Groth16 verification: one verdict per proof ---------------------------------------------------------------- */
+/* ark-groth16 0.4 prepare_verifying_key / prepare_inputs / verify_proof for batches: proof i is accepted iff
+ *   final_exp(multi_miller_loop([A_i, P_i, C_i], [B_i, -gamma, -delta])) == e(alpha, beta),
+ *   P_i = IC_0 + sum_j x_ij IC_j  (IC = gamma_abc_g1).
+ * Each proof costs three Miller loops sharing one accumulator and one final exponentiation on a six-lane group;
+ * P_i comes from fixed-base tables (8-bit windows) of IC_1..IC_m kept in the prepared key. */
+typedef enum ripp_groth16_status {
+  RIPP_GROTH16_OK = 0,               /* 0..4 are the ripp_decode_status of the first bad point, in the order A, B, C */
+  RIPP_GROTH16_FLAGS = 1,
+  RIPP_GROTH16_NONCANONICAL = 2,
+  RIPP_GROTH16_NOT_ON_CURVE = 3,
+  RIPP_GROTH16_NOT_IN_SUBGROUP = 4,
+  RIPP_GROTH16_INPUT_NONCANONICAL = 5, /* a public input >= r */
+  RIPP_GROTH16_REJECTED = 6            /* everything decodes, the pairing equation fails */
+} ripp_groth16_status;
+
+/* Bytes of device memory a prepared key with m public inputs needs. */
+size_t ripp_groth16_pvk_bytes(size_t m);
+/* vk: the packed host layout of ripp_tipp_verify_aggregate (alpha_g1 | beta_g2 | gamma_g2 | delta_g2 |
+ * gamma_abc_g1[m + 1]; Montgomery, trusted).  Writes e(alpha, beta), -gamma, -delta, IC_0 and the fixed-base tables of
+ * IC_1..IC_m into pvk_dev (ripp_groth16_pvk_bytes(m) bytes the caller allocated, e.g. with ripp_dev_alloc); returns
+ * when the key is ready.  One key serves any number of verification calls on contexts of the same GPU. */
+int ripp_groth16_prepare_vk_dev(ripp_ctx* ctx, const void* vk, size_t m, void* pvk_dev);
+/* n proofs, device resident and trusted (affine Montgomery, as every other _dev entry); inputs_dev: n x m Fr
+ * (Montgomery, row = one proof; NULL when m = 0).  verdict_dev[i] = 1 accept / 0 reject.  Asynchronous on the
+ * context's stream. */
+int ripp_groth16_verify_batch_dev(ripp_ctx* ctx, const void* pvk_dev, size_t m, const void* inputs_dev, const void* a_dev,
+                                  const void* b_dev, const void* c_dev, size_t n, uint8_t* verdict_dev);
+/* Untrusted bytes: proofs_host as for ripp_tipp_aggregate_serialized (n records; any n); inputs_host: n x m canonical
+ * little-endian Fr (32 B each, ark-serialize, no length prefix).  status_host[i] is a ripp_groth16_status: the first
+ * failure of proof i in the order A, B, C, inputs, equation.  *n_valid counts the zeros.  A false or malformed proof is
+ * data, not an error: RIPP_ERR_ARG only for lengths that do not match n and m, null pointers and n > 2^32 - 1. */
+int ripp_groth16_verify_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host, size_t inputs_len,
+                                   const uint8_t* proofs_host, size_t proofs_len, size_t n, int compressed,
+                                   uint8_t* status_host, size_t* n_valid);
+
 /* ---- SIPP (sipp/src/lib.rs; E = BLS12-381, D = Blake2s) ---------------------------------------- */
 /* product_of_pairings_with_coeffs (lib.rs:184-217): prod_i e(r_i a_i, b_i).  Affine host inputs
  * exactly as the reference takes them (&[G1Affine], &[G2Affine], &[Fr]). */

@@ -57,6 +57,7 @@ def lib():
         L.ripp_last_error_string.restype = ctypes.c_char_p
         L.ripp_ctx_stream.restype = ctypes.c_void_p
         L.ripp_ctx_launch_count.restype = ctypes.c_uint64
+        L.ripp_groth16_pvk_bytes.restype = ctypes.c_size_t
         _lib = L
     return _lib
 
@@ -386,6 +387,31 @@ class Context:
                                                    ctypes.c_size_t(n), int(bool(compressed)), _p(proof), ctypes.c_size_t(cap),
                                                    ctypes.byref(plen)))
         return proof[: plen.value].tobytes()
+
+    # ---- Groth16 verification (csrc/groth16.cu) -----------------------------------------------------------
+    @staticmethod
+    def groth16_pvk_bytes(m):
+        return int(lib().ripp_groth16_pvk_bytes(ctypes.c_size_t(m)))
+
+    def groth16_prepare_vk_dev(self, vk_words, m, pvk_dev):
+        """vk_words: packed alpha_g1 | beta_g2 | gamma_g2 | delta_g2 | gamma_abc_g1[m + 1] (uint32 Montgomery)."""
+        vk_words = np.ascontiguousarray(vk_words, dtype=np.uint32)
+        assert vk_words.size == 24 + 3 * 48 + 24 * (m + 1)
+        check(lib().ripp_groth16_prepare_vk_dev(self.handle, _p(vk_words), ctypes.c_size_t(m), _p(pvk_dev)))
+
+    def groth16_verify_batch_dev(self, pvk_dev, m, inputs_dev, a, b, c, n, verdict_dev):
+        check(lib().ripp_groth16_verify_batch_dev(self.handle, _p(pvk_dev), ctypes.c_size_t(m), _p(inputs_dev), _p(a), _p(b),
+                                                  _p(c), ctypes.c_size_t(n), _p(verdict_dev)))
+
+    def groth16_verify_serialized(self, pvk_dev, m, inputs_bytes, data, n, compressed):
+        """-> (n status bytes (ripp_groth16_status), number of accepted proofs)."""
+        st = np.zeros(max(n, 1), dtype=np.uint8)
+        nv = ctypes.c_size_t()
+        ib, pb = self._bytes(inputs_bytes), self._bytes(data)
+        check(lib().ripp_groth16_verify_serialized(self.handle, _p(pvk_dev), ctypes.c_size_t(m), _p(ib), ctypes.c_size_t(len(inputs_bytes)),
+                                                   _p(pb), ctypes.c_size_t(len(data)), ctypes.c_size_t(n), int(bool(compressed)),
+                                                   _p(st), ctypes.byref(nv)))
+        return st[:n], nv.value
 
     def sipp_product_with_coeffs(self, a, b, r):
         out = np.empty(144, dtype=np.uint32)

@@ -17,7 +17,7 @@ using namespace ripp;
 // ------------------------------------------------------------------------------------------------
 std::string& ripp_err_slot();
 
-#define RIPP_SCRATCH_SLOTS 32
+#define RIPP_SCRATCH_SLOTS 34
 #define RIPP_MAX_BATCH 8
 #define RIPP_MAX_CHILD 8
 // per-category device-time accounting (CUDA events on the context's stream; off by default)
@@ -138,3 +138,17 @@ int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, 
 int ripp_fold_pre_internal(ripp_ctx* ctx, const int* types, const void* const* hi, size_t n, void* const* pre);
 size_t ripp_fold_pre_max_n();
 int ripp_pairing6_init_device();  // per-device kernel attributes; called by ripp_ctx_create with the device current
+// groth16.cu's kernels: fixed-base tables and prepare_inputs (setup.cu), Miller loops and checks (pairing6.cu)
+size_t ripp_groth16_table_bytes();  // one input's table
+int ripp_groth16_tables(ripp_ctx* ctx, const void* ic_dev, size_t m, void* tables_dev);
+int ripp_groth16_inputs(ripp_ctx* ctx, const void* ic0_dev, const void* tables_dev, size_t m, const void* x_dev, size_t n,
+                        void* out_dev);
+int ripp_groth16_pairings_l6(ripp_ctx* ctx, const void* a, const void* b, const void* p, const void* c, const void* neg_gamma,
+                             const void* neg_delta, const void* ab, size_t n, void* miller, const uint8_t* pre, uint8_t* out);
+// deserialize.cu: one H2D copy of n proof records (plus `extra` bytes of the caller's behind them), A, B, C decoded on
+// three streams; statuses S[0, n) A, [n, 2n) B, [2n, 3n) C
+struct DecodedProofs {
+  void *a, *b, *c, *extra;
+  uint8_t* status;
+};
+int ripp_decode_proofs(ripp_ctx* ctx, const uint8_t* proofs_host, size_t n, int compressed, size_t extra, DecodedProofs* out);

@@ -69,22 +69,13 @@ static const char* decode_status_text(uint8_t s) {
   return "invalid";
 }
 
-extern "C" int ripp_tipp_aggregate_serialized(ripp_ctx* ctx, const void* srs_g1_dev, const void* srs_g2_dev,
-                                              const uint8_t* proofs_host, size_t proofs_len, size_t n, int compressed,
-                                              uint8_t* proof_out, size_t proof_cap, size_t* proof_len) {
-  if (!ctx || !srs_g1_dev || !srs_g2_dev || !proofs_host) return fail(RIPP_ERR_ARG, "null argument");
+int ripp_decode_proofs(ripp_ctx* ctx, const uint8_t* proofs_host, size_t n, int compressed, size_t extra, DecodedProofs* out) {
   const size_t g1b = compressed ? 48 : 96, g2b = 2 * g1b, rec = 2 * g1b + g2b;
-  if (n > (size_t)0xffffffffu || proofs_len != n * rec)
-    return fail(RIPP_ERR_ARG, "proof bytes: " + std::to_string(proofs_len) + " bytes is not " + std::to_string(n) + " records of " +
-                                  std::to_string(rec) + " bytes");
-  if (n == 0 || (n & (n - 1))) return fail(RIPP_ERR_NOT_POW2, "number of proofs must be a power of two");
-  if (n < 2) return fail(RIPP_ERR_ARG, "aggregation needs at least two proofs (tipa/mod.rs:199 unwraps the first challenge)");
-  CU(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
-  const size_t o_a = up(n * rec), o_b = o_a + n * 96, o_c = o_b + n * 192, o_st = o_c + n * 96;
+  const size_t o_a = up(n * rec), o_b = o_a + n * 96, o_c = o_b + n * 192, o_st = o_c + n * 96, o_x = o_st + up(3 * n);
   void* d;
-  OK(scratch(ctx, 23, o_st + up(3 * n), &d));
+  OK(scratch(ctx, 23, o_x + extra, &d));
   char* D = (char*)d;
   uint8_t* S = (uint8_t*)(D + o_st);
   CU(cudaMemcpyAsync(D, proofs_host, n * rec, cudaMemcpyHostToDevice, st));
@@ -99,12 +90,29 @@ extern "C" int ripp_tipp_aggregate_serialized(ripp_ctx* ctx, const void* srs_g1_
   OK(ripp_g1_deserialize_dev(ctx, D, n, rec, compressed, D + o_a, S));
   OK(ripp_join(ctx, kb));
   OK(ripp_join(ctx, kc));
+  *out = DecodedProofs{D + o_a, D + o_b, D + o_c, D + o_x, S};
+  return RIPP_OK;
+}
+
+extern "C" int ripp_tipp_aggregate_serialized(ripp_ctx* ctx, const void* srs_g1_dev, const void* srs_g2_dev,
+                                              const uint8_t* proofs_host, size_t proofs_len, size_t n, int compressed,
+                                              uint8_t* proof_out, size_t proof_cap, size_t* proof_len) {
+  if (!ctx || !srs_g1_dev || !srs_g2_dev || !proofs_host) return fail(RIPP_ERR_ARG, "null argument");
+  const size_t rec = compressed ? 192 : 384;
+  if (n > (size_t)0xffffffffu || proofs_len != n * rec)
+    return fail(RIPP_ERR_ARG, "proof bytes: " + std::to_string(proofs_len) + " bytes is not " + std::to_string(n) + " records of " +
+                                  std::to_string(rec) + " bytes");
+  if (n == 0 || (n & (n - 1))) return fail(RIPP_ERR_NOT_POW2, "number of proofs must be a power of two");
+  if (n < 2) return fail(RIPP_ERR_ARG, "aggregation needs at least two proofs (tipa/mod.rs:199 unwraps the first challenge)");
+  CU(cudaSetDevice(ctx->device));
+  DecodedProofs dp;
+  OK(ripp_decode_proofs(ctx, proofs_host, n, compressed, 0, &dp));
   std::vector<uint8_t> status(3 * n);
-  CU(cudaMemcpyAsync(status.data(), S, 3 * n, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
+  CU(cudaMemcpyAsync(status.data(), dp.status, 3 * n, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
   for (size_t i = 0; i < n; i++)
     for (int c = 0; c < 3; c++)
       if (uint8_t s = status[c * n + i])
         return fail(RIPP_ERR_ARG, "proof " + std::to_string(i) + ": " + "ABC"[c] + " " + decode_status_text(s));
-  return ripp_tipp_aggregate_dev(ctx, srs_g1_dev, srs_g2_dev, D + o_a, D + o_b, D + o_c, n, proof_out, proof_cap, proof_len);
+  return ripp_tipp_aggregate_dev(ctx, srs_g1_dev, srs_g2_dev, dp.a, dp.b, dp.c, n, proof_out, proof_cap, proof_len);
 }

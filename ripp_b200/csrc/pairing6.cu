@@ -14,6 +14,7 @@ struct Miller6Batch {
   const G2Aff* q[RIPP_MAX_BATCH];
   uint32_t n, wps;  // pairs per segment, warps per segment (5 * KP pairs per warp)
   int nseg;
+  uint32_t fixed_q;  // PER_GROUP kernels: bit j set = pair j of every item has the one Q at q[j][0]
 };
 
 constexpr int M6_NREG = 2;
@@ -27,7 +28,10 @@ __global__ void k_init_g2_gen() { g_g2_gen = g2_generator(); }
 
 // KP pairs per six-lane group share one accumulator (one Fq12 squaring per bit instead of KP):
 // KP = 1 minimises latency (late GIPA rounds), KP = 4 maximises throughput (long vectors).
-template <int WARPS, int KP>
+// PER_GROUP: one Miller value per item instead of one product per warp -- group t walks pair j = (p[j][t], q[j][t]) for
+// j < KP (one segment of n items; Q of pair j is q[j][0] for every item when bit j of fixed_q is set) and writes its
+// accumulator to partials[t] (the per-proof values of a Groth16 batch, groth16.cu).
+template <int WARPS, int KP, bool PER_GROUP = false>
 __global__ void __launch_bounds__(32 * WARPS) k_miller6(Miller6Batch b, Fq12* __restrict__ partials) {
   extern __shared__ __align__(16) uint32_t smem[];
   constexpr int GW = group_words(M6_NREG, KP);
@@ -47,13 +51,14 @@ __global__ void __launch_bounds__(32 * WARPS) k_miller6(Miller6Batch b, Fq12* __
   // lane 0 of each group stages its pairs; identities / padding run on the generators and are masked
   if (c.k == 0) {
     for (int j = 0; j < KP; j++) {
-      const uint32_t i = (wl * 5 + g) * KP + j;
+      const uint32_t i = PER_GROUP ? wl * 5 + g : (wl * 5 + g) * KP + j;
+      const int sv = PER_GROUP ? j : (int)seg;
       G1Aff P = g1_generator();
       const G2Aff* Q = &g_g2_gen;
       uint32_t valid = 0;
       if (seg < (uint32_t)b.nseg && i < b.n) {
-        G1Aff p = b.p[seg][i];
-        const G2Aff* q = &b.q[seg][i];
+        G1Aff p = b.p[sv][i];
+        const G2Aff* q = &b.q[sv][PER_GROUP && ((b.fixed_q >> j) & 1) ? 0 : i];
         if (!p.is_inf() && !q->is_inf()) {
           P = p;
           Q = q;
@@ -68,6 +73,12 @@ __global__ void __launch_bounds__(32 * WARPS) k_miller6(Miller6Batch b, Fq12* __
   }
   __syncwarp();
   miller(c, pairs, KP);
+  if constexpr (PER_GROUP) {
+    const uint32_t t = wl * 5 + g;
+    if (lane < 30 && seg < (uint32_t)b.nseg && t < b.n)
+      reinterpret_cast<Fq2*>(&partials[t])[tower_slot(c.k)] = ld2(freg(c, 0) + c.k * FQ2W);
+    return;
+  }
   // product of the five groups' values: (0 <- 0*1, 2 <- 2*3), 0 <- 0*2, 0 <- 0*4; idle groups write their junk register
   uint32_t* F0 = freg(c, 0);
   uint32_t* J = freg(c, 1);
@@ -129,6 +140,29 @@ __global__ void __launch_bounds__(64) k_final_exp6(const Fq12* __restrict__ in, 
   if (live) reinterpret_cast<Fq2*>(out + s)[tower_slot(c.k)] = ld2(freg(c, 0) + c.k * FQ2W);
 }
 
+
+// The Groth16 check of one proof per group: final_exponentiation(in[t]) == e(alpha, beta) (`ab`, 576 B), compared on
+// canonical Fq values (from_mont of any 384-bit value is the fully reduced product).  out[t] = 1 / 0, or with `pre`
+// (decode statuses of the serialized entry) pre[t] when non-zero, else RIPP_GROTH16_OK / RIPP_GROTH16_REJECTED.
+__global__ void __launch_bounds__(64) k_groth16_check6(const Fq12* __restrict__ in, const Fq12* __restrict__ ab, uint32_t n,
+                                                       const uint8_t* pre, uint8_t* out) {  // pre may alias out
+  extern __shared__ __align__(16) uint32_t smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int g = lane / 6;
+  Ctx c{lane % 6, smem + (warp * 6 + g) * FE_GROUP_WORDS};
+  const uint32_t t = (blockIdx.x * 2 + warp) * 5 + g;
+  const bool live = g < 5 && t < n;
+  st2(freg(c, 0) + c.k * FQ2W, reinterpret_cast<const Fq2*>(in + (live ? t : 0))[tower_slot(c.k)]);
+  __syncwarp();
+  final_exp(c);
+  const Fq2 f = ld2(freg(c, 0) + c.k * FQ2W), e = reinterpret_cast<const Fq2*>(ab)[tower_slot(c.k)];
+  const bool eq = f.c0.from_mont() == e.c0.from_mont() && f.c1.from_mont() == e.c1.from_mont();
+  const uint32_t all = __ballot_sync(0xffffffffu, eq);
+  if (live && c.k == 0) {
+    const bool ok = ((all >> (6 * g)) & 0x3fu) == 0x3fu;
+    out[t] = pre ? (pre[t] ? pre[t] : (ok ? RIPP_GROTH16_OK : RIPP_GROTH16_REJECTED)) : (uint8_t)ok;
+  }
+}
 
 // out[i] = in[i]^sc[i] (GT exponentiation by an Fr scalar in Montgomery form); one group per element.
 // The verifiers' `mul_helper` on PairingOutput (ip_proofs/src/lib.rs:15-19 with T = GT; gipa.rs:355-357,
@@ -521,6 +555,35 @@ int ripp_final_exp_l6(ripp_ctx* ctx, const void* in, uint32_t T, void* out, int 
   return RIPP_OK;
 }
 
+// Groth16 verification of n proofs, one six-lane group per proof (groth16.cu): the three pairs (A, B), (P, -gamma),
+// (C, -delta) of a proof share one accumulator (KP = 3), then one final exponentiation and the compare per group.
+// `miller` holds n Fq12.
+int ripp_groth16_pairings_l6(ripp_ctx* ctx, const void* a, const void* b, const void* p, const void* c, const void* neg_gamma,
+                             const void* neg_delta, const void* ab, size_t n, void* miller, const uint8_t* pre, uint8_t* out) {
+  Miller6Batch mb;
+  memset(&mb, 0, sizeof(mb));
+  mb.p[0] = (const G1Aff*)a;
+  mb.q[0] = (const G2Aff*)b;
+  mb.p[1] = (const G1Aff*)p;
+  mb.q[1] = (const G2Aff*)neg_gamma;
+  mb.p[2] = (const G1Aff*)c;
+  mb.q[2] = (const G2Aff*)neg_delta;
+  mb.fixed_q = 0x6;
+  mb.n = (uint32_t)n;
+  mb.nseg = 1;
+  mb.wps = (uint32_t)((n + 4) / 5);
+  {
+    TimeScope ts_(ctx, RIPP_T_MILLER);
+    k_miller6<M6_WARPS, 3, true><<<(mb.wps + M6_WARPS - 1) / M6_WARPS, 32 * M6_WARPS, m6_smem_bytes(3), ctx->stream>>>(mb, (Fq12*)miller);
+    LAUNCHED(ctx);
+  }
+  TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
+  k_groth16_check6<<<(unsigned)((n + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)miller, (const Fq12*)ab,
+                                                                                            (uint32_t)n, pre, out);
+  LAUNCHED(ctx);
+  return RIPP_OK;
+}
+
 // Opt-in shared-memory sizes of the six-lane kernels: function attributes are per device, set once per context
 // creation (ripp_ctx_create) -- never from the launch paths, which run concurrently on several host threads.
 int ripp_pairing6_init_device() {
@@ -532,5 +595,7 @@ int ripp_pairing6_init_device() {
   CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(2)));
   CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(3)));
   CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(4)));
+  CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(3)));
+  CU(cudaFuncSetAttribute(k_groth16_check6, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 6 * FE_GROUP_WORDS * 4));
   return RIPP_OK;
 }

@@ -182,5 +182,26 @@ RIPP_FN uint8_t decode_point(const uint8_t* in, Aff<F>* out) {
   return NOT_IN_SUBGROUP;
 }
 
+// One scalar-field element as ark-serialize writes Fr (32 bytes, little-endian, no flags).  Returns whether it is
+// canonical (< r); *out is its Montgomery form, zero for a rejected element.
+RIPP_HD bool decode_fr(const uint8_t* in, Fr* out) {
+  uint32_t w[8], br = 0;
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    const uint8_t* b = in + 4 * i;
+    w[i] = (uint32_t)b[0] | ((uint32_t)b[1] << 8) | ((uint32_t)b[2] << 16) | ((uint32_t)b[3] << 24);
+    uint64_t t = (uint64_t)w[i] - k::FR_P(i) - br;
+    br = (uint32_t)(t >> 63);
+  }
+  Fr f = Fr::zero();
+  if (br) {
+#pragma unroll
+    for (int i = 0; i < 8; i++) f.v[i] = w[i];
+    f = f.to_mont();
+  }
+  *out = f;
+  return br != 0;
+}
+
 }  // namespace serde
 }  // namespace ripp

@@ -18,11 +18,15 @@ constexpr int FB_C = 8;
 constexpr int FB_NW = (255 + FB_C - 1) / FB_C;
 constexpr int FB_PER = (1 << FB_C) - 1;
 
-// exponents of the table: t[w * FB_PER + d - 1] = d 2^(c w) (Montgomery)
-__global__ void k_fb_exponents(Fr* __restrict__ t) {
+constexpr int FB_ENTRIES = FB_NW * FB_PER;
+
+// exponents of the tables: t[b * FB_ENTRIES + w * FB_PER + d - 1] = d 2^(c w) (Montgomery), b < nb; with the bases
+// (non-null) repeated alongside, pts[b * FB_ENTRIES + e] = bases[b], so that one scaling launch builds nb tables
+__global__ void k_fb_exponents(Fr* __restrict__ t, int nb, const G1Aff* __restrict__ bases, G1Aff* __restrict__ pts) {
   int g = blockIdx.x * blockDim.x + threadIdx.x;
-  if (g >= FB_NW * FB_PER) return;
-  int w = g / FB_PER, d = g % FB_PER + 1;
+  if (g >= nb * FB_ENTRIES) return;
+  if (bases) pts[g] = bases[g / FB_ENTRIES];
+  int e = g % FB_ENTRIES, w = e / FB_PER, d = e % FB_PER + 1;
   Fr v = Fr::zero();
   v.v[0] = (uint32_t)d;
   v = v.to_mont();
@@ -30,13 +34,10 @@ __global__ void k_fb_exponents(Fr* __restrict__ t) {
   t[g] = v;
 }
 
+// acc += s B, s Montgomery, from the table of B: one mixed addition per 8-bit window
 template <class F>
-__global__ void __launch_bounds__(64, 4) k_fb_msm(const Aff<F>* __restrict__ table, const Fr* __restrict__ sc, size_t n,
-                                               Aff<F>* __restrict__ out) {
-  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  Fr s = sc[i].from_mont();
-  Jac<F> acc = Jac<F>::inf();
+__device__ __forceinline__ Jac<F> fb_add(Jac<F> acc, const Aff<F>* __restrict__ table, const Fr& sc) {
+  Fr s = sc.from_mont();
   for (int w = 0; w < FB_NW; w++) {
     int o = w * FB_C, wi = o >> 5, sh = o & 31;
     uint64_t v = s.v[wi];
@@ -45,6 +46,25 @@ __global__ void __launch_bounds__(64, 4) k_fb_msm(const Aff<F>* __restrict__ tab
     Aff<F> q = d ? table[w * FB_PER + d - 1] : Aff<F>::inf();  // digit 0 adds the identity: same instruction stream
     acc = Jac<F>::add_mixed_fn(acc, q);
   }
+  return acc;
+}
+
+template <class F>
+__global__ void __launch_bounds__(64, 4) k_fb_msm(const Aff<F>* __restrict__ table, const Fr* __restrict__ sc, size_t n,
+                                               Aff<F>* __restrict__ out) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  out[i] = fb_add<F>(Jac<F>::inf(), table, sc[i]).to_affine();
+}
+
+// Groth16 prepare_inputs for n proofs: P_i = IC_0 + sum_j x_ij IC_(j+1) over the m tables of IC_1..IC_m
+// (groth16.cu); one thread per proof, m x 32 mixed additions
+__global__ void __launch_bounds__(64, 4) k_groth16_inputs(const G1Aff* __restrict__ ic0, const G1Aff* __restrict__ tables,
+                                                       const Fr* __restrict__ x, uint32_t n, uint32_t m, G1Aff* __restrict__ out) {
+  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  Jac<Fq> acc = Jac<Fq>::from_affine(*ic0);
+  for (uint32_t j = 0; j < m; j++) acc = fb_add<Fq>(acc, tables + (size_t)j * FB_ENTRIES, x[(size_t)i * m + j]);
   out[i] = acc.to_affine();
 }
 
@@ -63,6 +83,22 @@ __global__ void k_fr_power_seq(Fr s, size_t n, Fr* __restrict__ out) {
 int ripp_scale_base_g1(ripp_ctx* ctx, const G1Aff* base_or_null, const void* sc_dev, size_t n, void* out_dev);
 int ripp_scale_base_g2(ripp_ctx* ctx, const G2Aff* base_or_null, const void* sc_dev, size_t n, void* out_dev);
 
+// The fixed-base tables of nb bases (FB_ENTRIES affine points each, written to `tables`): one exponent launch and ONE
+// scaling launch for all of them.  Either one base (host, or NULL for the generator), or nb G1 bases in device memory.
+template <class F>
+static int fb_tables(ripp_ctx* ctx, const Aff<F>* base_host, const G1Aff* bases_dev, size_t nb, Aff<F>* tables) {
+  const size_t ne = nb * FB_ENTRIES, o_pts = (ne * sizeof(Fr) + 255) & ~(size_t)255;
+  void* buf;
+  OK(scratch(ctx, 31, o_pts + (bases_dev ? ne * sizeof(G1Aff) : 0), &buf));
+  Fr* ex = (Fr*)buf;
+  G1Aff* pts = bases_dev ? (G1Aff*)((char*)buf + o_pts) : nullptr;
+  k_fb_exponents<<<(unsigned)((ne + 127) / 128), 128, 0, ctx->stream>>>(ex, (int)nb, bases_dev, pts);
+  LAUNCHED(ctx);
+  if (bases_dev) return ripp_g1_scale_dev(ctx, pts, ex, ne, tables);
+  if (sizeof(F) == sizeof(Fq)) return ripp_scale_base_g1(ctx, (const G1Aff*)base_host, ex, ne, tables);
+  return ripp_scale_base_g2(ctx, (const G2Aff*)base_host, ex, ne, tables);
+}
+
 template <class F>
 static int fixed_base_msm(ripp_ctx* ctx, const void* base_host, const void* sc_dev, size_t n, void* out_dev) {
   if (!ctx || (n && (!sc_dev || !out_dev))) return fail(RIPP_ERR_ARG, "null argument");
@@ -76,16 +112,9 @@ static int fixed_base_msm(ripp_ctx* ctx, const void* base_host, const void* sc_d
     return ripp_scale_base_g2(ctx, base_host ? (const G2Aff*)&base : nullptr, sc_dev, n, out_dev);
   }
   void* buf;
-  size_t o_tab = ((size_t)FB_NW * FB_PER * sizeof(Fr) + 255) & ~(size_t)255;
-  OK(scratch(ctx, 24, o_tab + (size_t)FB_NW * FB_PER * sizeof(Aff<F>), &buf));
-  Fr* ex = (Fr*)buf;
-  Aff<F>* table = (Aff<F>*)((char*)buf + o_tab);
-  k_fb_exponents<<<(FB_NW * FB_PER + 127) / 128, 128, 0, ctx->stream>>>(ex);
-  LAUNCHED(ctx);
-  if (sizeof(F) == sizeof(Fq))
-    OK(ripp_scale_base_g1(ctx, base_host ? (const G1Aff*)&base : nullptr, ex, (size_t)FB_NW * FB_PER, table));
-  else
-    OK(ripp_scale_base_g2(ctx, base_host ? (const G2Aff*)&base : nullptr, ex, (size_t)FB_NW * FB_PER, table));
+  OK(scratch(ctx, 24, (size_t)FB_ENTRIES * sizeof(Aff<F>), &buf));
+  Aff<F>* table = (Aff<F>*)buf;
+  OK(fb_tables<F>(ctx, base_host ? &base : nullptr, nullptr, 1, table));
   TimeScope ts_(ctx, RIPP_T_SCALE);
   k_fb_msm<F><<<(unsigned)((n + 63) / 64), 64, 0, ctx->stream>>>(table, (const Fr*)sc_dev, n, (Aff<F>*)out_dev);
   LAUNCHED(ctx);
@@ -144,5 +173,22 @@ extern "C" int ripp_tipa_setup_dev(ripp_ctx* ctx, const void* alpha, const void*
   CU(cudaMemcpyAsync(g_beta_out, p + 256, 96, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaMemcpyAsync(h_alpha_out, p + 512, 192, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
+  return RIPP_OK;
+}
+
+// ---- Groth16 prepare_inputs (groth16.cu) -------------------------------------------------------------------------
+size_t ripp_groth16_table_bytes() { return (size_t)FB_ENTRIES * sizeof(G1Aff); }
+
+int ripp_groth16_tables(ripp_ctx* ctx, const void* ic_dev, size_t m, void* tables_dev) {
+  if (m == 0) return RIPP_OK;
+  return fb_tables<Fq>(ctx, nullptr, (const G1Aff*)ic_dev, m, (G1Aff*)tables_dev);
+}
+
+int ripp_groth16_inputs(ripp_ctx* ctx, const void* ic0_dev, const void* tables_dev, size_t m, const void* x_dev, size_t n,
+                        void* out_dev) {
+  TimeScope ts_(ctx, RIPP_T_SCALE);
+  k_groth16_inputs<<<(unsigned)((n + 63) / 64), 64, 0, ctx->stream>>>((const G1Aff*)ic0_dev, (const G1Aff*)tables_dev,
+                                                                      (const Fr*)x_dev, (uint32_t)n, (uint32_t)m, (G1Aff*)out_dev);
+  LAUNCHED(ctx);
   return RIPP_OK;
 }

@@ -7,7 +7,8 @@
 //!   SRS: alpha = scalar("srs-alpha", 0), beta = scalar("srs-beta", 0), powers as TIPA::setup computes them.
 //! Every value is `serialize_uncompressed` bytes, hex encoded, except the `g*c_*` compressed encodings and the
 //! `serde_verdict_*` decoder verdicts (hex of "ok" || the decoded point uncompressed, "flags", "invalid" or "other").
-//! Usage: cargo run --release -p ark-golden -- <path of tests/golden/serde_cases.txt> > tests/golden/ark_golden.json
+//! Usage: cargo run --release -p ark-golden -- <path of tests/golden/serde_cases.txt> [<path of
+//!        tests/golden/groth16_cases.txt>] > tests/golden/ark_golden.json
 use ark_bls12_381::{Bls12_381, Fr, G1Projective as G1, G2Projective as G2};
 use ark_dh_commitments::{
     afgho16::{AFGHOCommitmentG1, AFGHOCommitmentG2},
@@ -244,6 +245,34 @@ fn main() {
                 })
             };
             out.push((key.replace("serde_case_", "serde_verdict_"), verdict(r)));
+        }
+    }
+
+    // ark-groth16's own verdict (prepare_verifying_key + verify_proof) on every proof of the GPU mixed batch listed in
+    // tests/golden/groth16_cases.txt (oracle/groth16.py golden_case_lines; path = the second argument), as
+    // `groth16_verdict_<i>` = "01" accept / "00" reject.
+    if let Some(path) = std::env::args().nth(2) {
+        use ark_groth16::{Groth16, Proof, VerifyingKey};
+        use ark_serialize::CanonicalDeserialize;
+        use ark_snark::SNARK;
+        let text = std::fs::read_to_string(&path).expect("pass the path of tests/golden/groth16_cases.txt");
+        let unhex = |h: &str| (0..h.len()).step_by(2).map(|i| u8::from_str_radix(&h[i..i + 2], 16).unwrap()).collect::<Vec<u8>>();
+        let mut pvk = None;
+        for line in text.lines() {
+            let f: Vec<&str> = line.split_whitespace().collect();
+            if f.is_empty() {
+                continue;
+            }
+            if f[0] == "groth16_vk" {
+                let vk = VerifyingKey::<Bls12_381>::deserialize_compressed(&unhex(f[1])[..]).unwrap();
+                pvk = Some(Groth16::<Bls12_381>::process_vk(&vk).unwrap());
+                continue;
+            }
+            let proof = Proof::<Bls12_381>::deserialize_compressed(&unhex(f[1])[..]).unwrap();
+            let xb = if f.len() > 2 { unhex(f[2]) } else { Vec::new() };
+            let x: Vec<Fr> = xb.chunks(32).map(|c| Fr::deserialize_compressed(c).unwrap()).collect();
+            let ok = Groth16::<Bls12_381>::verify_with_processed_vk(pvk.as_ref().unwrap(), &x, &proof).unwrap_or(false);
+            out.push((f[0].replace("groth16_case_", "groth16_verdict_"), if ok { "01".into() } else { "00".into() }));
         }
     }
 

@@ -34,6 +34,9 @@ impl DeviceElem for G1Affine {
 impl DeviceElem for G2Affine {
     const BYTES: usize = 192;
 }
+impl DeviceElem for u8 {
+    const BYTES: usize = 1;
+}
 
 /// RAII handle on a device vector (`ripp_dev_alloc` / `ripp_dev_free`).
 pub struct DeviceVec<T: DeviceElem> {
@@ -328,4 +331,80 @@ pub fn gipa_prove_checked_ab(a: &DeviceVec<G1Affine>, b: &DeviceVec<G2Affine>, c
     check(st, n, b.len())?;
     buf.truncate(len);
     Ok(buf)
+}
+
+/// ark-groth16 `PreparedVerifyingKey` resident on the device (`ripp_groth16_prepare_vk_dev`): e(alpha, beta), -gamma,
+/// -delta, IC_0 and fixed-base tables of IC_1..IC_m.
+pub struct GpuPreparedVerifyingKey {
+    buf: DeviceVec<u8>,
+    m: usize,
+}
+
+impl GpuPreparedVerifyingKey {
+    /// `prepare_verifying_key`; the key is trusted, as in `verify_aggregate_proof`.
+    pub fn new(vk: &VerifyingKey<Bls12_381>) -> Result<Self, Error> {
+        assert!(!vk.gamma_abc_g1.is_empty());
+        let m = vk.gamma_abc_g1.len() - 1;
+        let mut vkw = Vec::new();
+        vkw.extend(pack::pack_g1_aff(&[vk.alpha_g1]));
+        vkw.extend(pack::pack_g2_aff(&[vk.beta_g2, vk.gamma_g2, vk.delta_g2]));
+        vkw.extend(pack::pack_g1_aff(&vk.gamma_abc_g1));
+        let buf = DeviceVec::<u8>::alloc(unsafe { sys::ripp_groth16_pvk_bytes(m) })?;
+        let c = ctx();
+        let st = unsafe { sys::ripp_groth16_prepare_vk_dev(c.raw(), vkw.as_ptr() as *const c_void, m, buf.ptr_mut()) };
+        drop(c);
+        check(st, m, m)?;
+        Ok(GpuPreparedVerifyingKey { buf, m })
+    }
+}
+
+/// `verify_proof` for every (inputs, proof) pair, one verdict per proof.  A row whose length is not the key's input
+/// count is `MessageLengthInvalid`, where ark-groth16's `prepare_inputs` fails.
+pub fn verify_proofs(pvk: &GpuPreparedVerifyingKey, public_inputs: &[Vec<Fr>], proofs: &[Proof<Bls12_381>]) -> Result<Vec<bool>, Error> {
+    let n = proofs.len();
+    if public_inputs.len() != n {
+        return check(sys::RIPP_ERR_LEN_MISMATCH, public_inputs.len(), n).map(|_| Vec::new());
+    }
+    if let Some(row) = public_inputs.iter().find(|r| r.len() != pvk.m) {
+        return check(sys::RIPP_ERR_LEN_MISMATCH, row.len(), pvk.m).map(|_| Vec::new());
+    }
+    if n == 0 {
+        return Ok(Vec::new());
+    }
+    let a = DeviceVec::<G1Affine>::upload_affine(&proofs.iter().map(|p| p.a).collect::<Vec<_>>())?;
+    let b = DeviceVec::<G2Affine>::upload_affine(&proofs.iter().map(|p| p.b).collect::<Vec<_>>())?;
+    let cc = DeviceVec::<G1Affine>::upload_affine(&proofs.iter().map(|p| p.c).collect::<Vec<_>>())?;
+    let x = DeviceVec::<Fr>::upload_fr(&public_inputs.concat())?;
+    let out = DeviceVec::<u8>::alloc(n)?;
+    let mut verdict = vec![0u8; n];
+    let c = ctx();
+    let mut st = unsafe {
+        sys::ripp_groth16_verify_batch_dev(c.raw(), pvk.buf.ptr(), pvk.m, x.ptr(), a.ptr(), b.ptr(), cc.ptr(), n, out.ptr_mut() as *mut u8)
+    };
+    if st == sys::RIPP_OK {
+        st = unsafe { sys::ripp_dev_download(c.raw(), verdict.as_mut_ptr() as *mut c_void, out.ptr(), n) };
+    }
+    drop(c);
+    check(st, n, n)?;
+    Ok(verdict.into_iter().map(|v| v == 1).collect())
+}
+
+/// `verify_proof` from untrusted bytes: `proofs` holds `Proof` records back to back (`serialize_compressed` 192 B or
+/// `serialize_uncompressed` 384 B each, no length prefix), `inputs` the m public inputs of each proof as
+/// ark-serialize `Fr` (32 B each).  One `ripp_groth16_status` per proof: 0 = valid, 1..4 = the first point of A, B, C
+/// that does not decode, 5 = an input >= r, 6 = the pairing equation fails.
+pub fn verify_proofs_serialized(pvk: &GpuPreparedVerifyingKey, inputs: &[u8], proofs: &[u8], compress: Compress) -> Result<Vec<u8>, Error> {
+    let record = if compress == Compress::Yes { 192 } else { 384 };
+    let n = proofs.len() / record;
+    let mut status = vec![0u8; n];
+    let mut n_valid = 0usize;
+    let c = ctx();
+    let st = unsafe {
+        sys::ripp_groth16_verify_serialized(c.raw(), pvk.buf.ptr(), pvk.m, inputs.as_ptr(), inputs.len(), proofs.as_ptr(),
+                                            proofs.len(), n, (compress == Compress::Yes) as i32, status.as_mut_ptr(),
+                                            &mut n_valid)
+    };
+    drop(c);
+    check(st, n, n)?;
+    Ok(status)
 }
