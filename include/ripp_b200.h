@@ -307,6 +307,22 @@ int ripp_groth16_verify_batch_dev(ripp_ctx* ctx, const void* pvk_dev, size_t m, 
 int ripp_groth16_verify_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host, size_t inputs_len,
                                    const uint8_t* proofs_host, size_t proofs_len, size_t n, int compressed,
                                    uint8_t* status_host, size_t* n_valid);
+/* Random-linear-combination verification: verdicts as ripp_groth16_verify_batch_dev, except with probability
+ * <= 2^-128 per segment; seed32: 32 caller-drawn bytes, fresh per call.  Synchronous (one host decision: which
+ * segments to re-check).  *n_rechecked = proofs that went through the per-proof fallback.
+ * Segments of s consecutive proofs (RIPP_B200_G16_RLC_SEG, default 58) are each checked as one proof whose scalars
+ * r_i (ChaCha20 keystream of the seed, 128 bits, normalised to sum to one) combine the proofs' equations; the proofs
+ * of a failing segment are then verified one by one (DESIGN.md §4 "Groth16 verification by random linear
+ * combination"). */
+int ripp_groth16_verify_rlc_dev(ripp_ctx* ctx, const void* pvk_dev, size_t m, const void* inputs_dev, const void* a_dev,
+                                const void* b_dev, const void* c_dev, size_t n, const uint8_t* seed32,
+                                uint8_t* verdict_dev, size_t* n_rechecked);
+/* Untrusted bytes as ripp_groth16_verify_serialized, same statuses; proofs with a decode or input status are left out
+ * of their segment's combination (r_i = 0, not a member) and keep that status. */
+int ripp_groth16_verify_rlc_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host,
+                                       size_t inputs_len, const uint8_t* proofs_host, size_t proofs_len, size_t n,
+                                       int compressed, const uint8_t* seed32, uint8_t* status_host, size_t* n_valid,
+                                       size_t* n_rechecked);
 
 /* ---- SIPP (sipp/src/lib.rs; E = BLS12-381, D = Blake2s) ---------------------------------------- */
 /* product_of_pairings_with_coeffs (lib.rs:184-217): prod_i e(r_i a_i, b_i).  Affine host inputs

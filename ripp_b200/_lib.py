@@ -413,6 +413,27 @@ class Context:
                                                    _p(st), ctypes.byref(nv)))
         return st[:n], nv.value
 
+    def groth16_verify_rlc_dev(self, pvk_dev, m, inputs_dev, a, b, c, n, seed, verdict_dev):
+        """Random-linear-combination verification (synchronous); seed: 32 bytes.  -> number of proofs re-checked one by
+        one."""
+        sd = self._bytes(seed) if seed is not None else None
+        nre = ctypes.c_size_t()
+        check(lib().ripp_groth16_verify_rlc_dev(self.handle, _p(pvk_dev), ctypes.c_size_t(m), _p(inputs_dev), _p(a), _p(b), _p(c),
+                                                ctypes.c_size_t(n), _p(sd), _p(verdict_dev), ctypes.byref(nre)))
+        return nre.value
+
+    def groth16_verify_rlc_serialized(self, pvk_dev, m, inputs_bytes, data, n, compressed, seed):
+        """-> (n status bytes (ripp_groth16_status), number of accepted proofs, number of proofs re-checked one by one)."""
+        st = np.zeros(max(n, 1), dtype=np.uint8)
+        nv, nre = ctypes.c_size_t(), ctypes.c_size_t()
+        ib, pb = self._bytes(inputs_bytes), self._bytes(data)
+        sd = self._bytes(seed) if seed is not None else None
+        check(lib().ripp_groth16_verify_rlc_serialized(self.handle, _p(pvk_dev), ctypes.c_size_t(m), _p(ib),
+                                                       ctypes.c_size_t(len(inputs_bytes)), _p(pb), ctypes.c_size_t(len(data)),
+                                                       ctypes.c_size_t(n), int(bool(compressed)), _p(sd), _p(st), ctypes.byref(nv),
+                                                       ctypes.byref(nre)))
+        return st[:n], nv.value, nre.value
+
     def sipp_product_with_coeffs(self, a, b, r):
         out = np.empty(144, dtype=np.uint32)
         check(lib().ripp_sipp_product_with_coeffs(self.handle, _p(a), _p(b), _p(r), ctypes.c_size_t(len(a)), _p(out)))

@@ -17,7 +17,7 @@ using namespace ripp;
 // ------------------------------------------------------------------------------------------------
 std::string& ripp_err_slot();
 
-#define RIPP_SCRATCH_SLOTS 34
+#define RIPP_SCRATCH_SLOTS 38
 #define RIPP_MAX_BATCH 8
 #define RIPP_MAX_CHILD 8
 // per-category device-time accounting (CUDA events on the context's stream; off by default)
@@ -145,6 +145,9 @@ int ripp_groth16_inputs(ripp_ctx* ctx, const void* ic0_dev, const void* tables_d
                         void* out_dev);
 int ripp_groth16_pairings_l6(ripp_ctx* ctx, const void* a, const void* b, const void* p, const void* c, const void* neg_gamma,
                              const void* neg_delta, const void* ab, size_t n, void* miller, const uint8_t* pre, uint8_t* out);
+// the segment checks of the random-linear-combination entry points: ok[t] = 1 / 0 for segment t < nseg of s proofs
+int ripp_groth16_rlc_pairings_l6(ripp_ctx* ctx, const void* ra, const void* b, const void* ps, const void* cs, const void* neg_gamma,
+                                 const void* neg_delta, const void* ab, size_t n, size_t s, size_t nseg, uint8_t* ok);
 // deserialize.cu: one H2D copy of n proof records (plus `extra` bytes of the caller's behind them), A, B, C decoded on
 // three streams; statuses S[0, n) A, [n, 2n) B, [2n, 3n) C
 struct DecodedProofs {

@@ -1,6 +1,7 @@
 // Host-side hashes for the Fiat-Shamir transcripts: BLAKE2b-512 (GIPA/TIPA/aggregation challenges,
 // gipa.rs:235-258, tipa/mod.rs:195-209, groth16_aggregation.rs:105-116), BLAKE2s-256 and the
-// ChaCha20 block function (SIPP's hash-reseeded RNG, sipp/src/rng.rs:12-73).  RFC 7693 / RFC 8439,
+// ChaCha20 block function (SIPP's hash-reseeded RNG, sipp/src/rng.rs:12-73; also called on the device for the
+// scalars of the Groth16 random-linear-combination check, groth16.cu).  RFC 7693 / RFC 8439,
 // unkeyed, written from the RFCs.
 #pragma once
 #include <stdint.h>
@@ -8,11 +9,19 @@
 
 #include <vector>
 
+#ifndef RIPP_HD  // as limb.cuh defines it
+#if defined(__CUDACC__)
+#define RIPP_HD __host__ __device__ __forceinline__
+#else
+#define RIPP_HD inline
+#endif
+#endif
+
 namespace ripp_hash {
 
 static inline uint64_t rotr64(uint64_t x, int n) { return (x >> n) | (x << (64 - n)); }
 static inline uint32_t rotr32(uint32_t x, int n) { return (x >> n) | (x << (32 - n)); }
-static inline uint32_t rotl32(uint32_t x, int n) { return (x << n) | (x >> (32 - n)); }
+RIPP_HD uint32_t rotl32(uint32_t x, int n) { return (x << n) | (x >> (32 - n)); }
 
 static const uint8_t SIGMA[12][16] = {
     {0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15}, {14, 10, 4, 8, 9, 15, 13, 6, 1, 12, 0, 2, 11, 7, 5, 3},
@@ -119,10 +128,12 @@ static inline void blake2s256(const uint8_t* data, size_t len, uint8_t out[32]) 
 }
 
 // ChaCha20 block (rand_chacha 0.3 ChaChaRng: 64-bit block counter in words 12-13, stream 0)
-static inline void chacha20_block(const uint8_t key[32], uint64_t counter, uint8_t out[64]) {
+RIPP_HD void chacha20_block(const uint8_t key[32], uint64_t counter, uint8_t out[64]) {
   uint32_t init[16], s[16];
-  static const char sigma[] = "expand 32-byte k";
-  memcpy(init, sigma, 16);
+  init[0] = 0x61707865u;  // "expand 32-byte k"
+  init[1] = 0x3320646eu;
+  init[2] = 0x79622d32u;
+  init[3] = 0x6b206574u;
   memcpy(init + 4, key, 32);
   init[12] = (uint32_t)counter;
   init[13] = (uint32_t)(counter >> 32);

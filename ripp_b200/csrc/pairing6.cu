@@ -584,6 +584,106 @@ int ripp_groth16_pairings_l6(ripp_ctx* ctx, const void* a, const void* b, const 
   return RIPP_OK;
 }
 
+// Pairs of the random-linear-combination check (groth16.cu verify_rlc): segment t of s proofs becomes sp pairs,
+// (r_i A_i, B_i) for its proofs, then (P_t, -gamma), (C_t, -delta), then masked padding up to sp, a multiple of the
+// pairs per warp, so that no warp's partial product straddles two segments.
+__global__ void __launch_bounds__(64) k_rlc_pairs(const G1Aff* __restrict__ ra, const G2Aff* __restrict__ b,
+                                                  const G1Aff* __restrict__ ps, const G1Aff* __restrict__ cs,
+                                                  const G2Aff* __restrict__ neg_gamma, const G2Aff* __restrict__ neg_delta,
+                                                  uint32_t n, uint32_t s, uint32_t sp, uint32_t nseg, G1Aff* __restrict__ P,
+                                                  G2Aff* __restrict__ Q) {
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (size_t)nseg * sp) return;
+  const uint32_t seg = (uint32_t)(t / sp), i = (uint32_t)(t % sp), lo = seg * s, len = min(s, n - lo);
+  if (i < len) {
+    P[t] = ra[lo + i];
+    Q[t] = b[lo + i];
+  } else if (i == len) {
+    P[t] = ps[seg];
+    Q[t] = *neg_gamma;
+  } else {
+    P[t] = i == len + 1 ? cs[seg] : G1Aff::inf();
+    Q[t] = *neg_delta;
+  }
+}
+
+int ripp_groth16_rlc_pairings_l6(ripp_ctx* ctx, const void* ra, const void* b, const void* ps, const void* cs, const void* neg_gamma,
+                                 const void* neg_delta, const void* ab, size_t n, size_t s, size_t nseg, uint8_t* ok) {
+  // pairs per group as ripp_pairing_batch_l6's throughput shape: the cheapest waves x warp duration, here counting each
+  // segment's padding
+  static int sms = 0;
+  if (!sms) {
+    cudaDeviceProp prop;
+    CU(cudaGetDeviceProperties(&prop, ctx->device));
+    sms = prop.multiProcessorCount;
+  }
+  const size_t resident = (size_t)sms * 2 * M6_WARPS;
+  int kp = 1;
+  double best = 0;
+  for (int k = 1; k <= 4; k++) {
+    const size_t warps = nseg * ((s + 2 + 5 * k - 1) / (5 * k));
+    const double t = (double)((warps + resident - 1) / resident) * (2040.0 + 3096.0 * k);
+    if (k == 1 || t <= best) {
+      best = t;
+      kp = k;
+    }
+  }
+  static const int force = [] {
+    const char* e = getenv("RIPP_B200_M6_KP");
+    return e ? atoi(e) : 0;
+  }();
+  if (force >= 1 && force <= 4) kp = force;
+  const size_t ppw = 5 * (size_t)kp, sp = (s + 2 + ppw - 1) / ppw * ppw, np = nseg * sp, T0 = sp / ppw;
+  void *pq, *part;
+  const size_t o_q = (np * sizeof(G1Aff) + 255) & ~(size_t)255;
+  OK(scratch(ctx, 36, o_q + np * sizeof(G2Aff), &pq));
+  const size_t o_b = (nseg * T0 * sizeof(Fq12) + 255) & ~(size_t)255;
+  OK(scratch(ctx, 37, o_b + (nseg * ((T0 + 7) / 8) + 1) * sizeof(Fq12), &part));
+  G1Aff* P = (G1Aff*)pq;
+  G2Aff* Q = (G2Aff*)((char*)pq + o_q);
+  Fq12 *src = (Fq12*)part, *dst = (Fq12*)((char*)part + o_b);
+  {
+    TimeScope ts_(ctx, RIPP_T_MILLER);
+    k_rlc_pairs<<<(unsigned)((np + 63) / 64), 64, 0, ctx->stream>>>((const G1Aff*)ra, (const G2Aff*)b, (const G1Aff*)ps,
+                                                                   (const G1Aff*)cs, (const G2Aff*)neg_gamma, (const G2Aff*)neg_delta,
+                                                                   (uint32_t)n, (uint32_t)s, (uint32_t)sp, (uint32_t)nseg, P, Q);
+    LAUNCHED(ctx);
+    Miller6Batch mb;
+    memset(&mb, 0, sizeof(mb));
+    mb.p[0] = P;
+    mb.q[0] = Q;
+    mb.n = (uint32_t)np;
+    mb.nseg = 1;
+    size_t nwarps = 0;
+    if (kp == 4)
+      OK(launch_miller6<4>(ctx, mb, np, src, &nwarps));
+    else if (kp == 3)
+      OK(launch_miller6<3>(ctx, mb, np, src, &nwarps));
+    else if (kp == 2)
+      OK(launch_miller6<2>(ctx, mb, np, src, &nwarps));
+    else
+      OK(launch_miller6<1>(ctx, mb, np, src, &nwarps));
+    // partials [seg * T + w] -> one Miller value per segment
+    const uint32_t R = 8;
+    uint32_t T = (uint32_t)T0;
+    while (T > 1) {
+      const uint32_t To = (T + R - 1) / R, tot = (uint32_t)nseg * To;
+      k_reduce6<M6_WARPS><<<(tot + 5 * M6_WARPS - 1) / (5 * M6_WARPS), 32 * M6_WARPS, M6_WARPS * 6 * R6_GROUP_WORDS * 4, ctx->stream>>>(
+          src, T, R, To, dst, tot);
+      LAUNCHED(ctx);
+      Fq12* t = src;
+      src = dst;
+      dst = t;
+      T = To;
+    }
+  }
+  TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
+  k_groth16_check6<<<(unsigned)((nseg + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>(src, (const Fq12*)ab, (uint32_t)nseg,
+                                                                                               nullptr, ok);
+  LAUNCHED(ctx);
+  return RIPP_OK;
+}
+
 // Opt-in shared-memory sizes of the six-lane kernels: function attributes are per device, set once per context
 // creation (ripp_ctx_create) -- never from the launch paths, which run concurrently on several host threads.
 int ripp_pairing6_init_device() {

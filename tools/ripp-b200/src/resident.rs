@@ -16,6 +16,7 @@ use ark_groth16::{Proof, VerifyingKey};
 use ark_inner_products::{Error, MultiexponentiationInnerProduct, PairingInnerProduct};
 use ark_ip_proofs::tipa::{structured_scalar_message::TIPAWithSSMProof, TIPAProof, VerifierSRS};
 use ark_serialize::{CanonicalDeserialize, CanonicalSerialize, Compress};
+use ark_std::rand::{CryptoRng, RngCore};
 use blake2::Blake2b;
 use ripp_b200_sys as sys;
 use std::marker::PhantomData;
@@ -407,4 +408,64 @@ pub fn verify_proofs_serialized(pvk: &GpuPreparedVerifyingKey, inputs: &[u8], pr
     drop(c);
     check(st, n, n)?;
     Ok(status)
+}
+
+/// `verify_proofs` by random linear combination (`ripp_groth16_verify_rlc_dev`): segments of proofs are checked as one
+/// combined equation each, and only the proofs of failing segments are verified one by one.  The verdicts equal
+/// `verify_proofs`' except with probability at most 2^-128 per segment.  The 32-byte seed is drawn from `rng`, after
+/// the proofs are fixed.  Returns the verdicts and the number of proofs that were verified one by one.
+pub fn verify_proofs_rlc<R: RngCore + CryptoRng>(pvk: &GpuPreparedVerifyingKey, public_inputs: &[Vec<Fr>], proofs: &[Proof<Bls12_381>],
+                                                 rng: &mut R) -> Result<(Vec<bool>, usize), Error> {
+    let n = proofs.len();
+    if public_inputs.len() != n {
+        return check(sys::RIPP_ERR_LEN_MISMATCH, public_inputs.len(), n).map(|_| (Vec::new(), 0));
+    }
+    if let Some(row) = public_inputs.iter().find(|r| r.len() != pvk.m) {
+        return check(sys::RIPP_ERR_LEN_MISMATCH, row.len(), pvk.m).map(|_| (Vec::new(), 0));
+    }
+    if n == 0 {
+        return Ok((Vec::new(), 0));
+    }
+    let mut seed = [0u8; 32];
+    rng.fill_bytes(&mut seed);
+    let a = DeviceVec::<G1Affine>::upload_affine(&proofs.iter().map(|p| p.a).collect::<Vec<_>>())?;
+    let b = DeviceVec::<G2Affine>::upload_affine(&proofs.iter().map(|p| p.b).collect::<Vec<_>>())?;
+    let cc = DeviceVec::<G1Affine>::upload_affine(&proofs.iter().map(|p| p.c).collect::<Vec<_>>())?;
+    let x = DeviceVec::<Fr>::upload_fr(&public_inputs.concat())?;
+    let out = DeviceVec::<u8>::alloc(n)?;
+    let mut verdict = vec![0u8; n];
+    let mut n_rechecked = 0usize;
+    let c = ctx();
+    let mut st = unsafe {
+        sys::ripp_groth16_verify_rlc_dev(c.raw(), pvk.buf.ptr(), pvk.m, x.ptr(), a.ptr(), b.ptr(), cc.ptr(), n, seed.as_ptr(),
+                                         out.ptr_mut() as *mut u8, &mut n_rechecked)
+    };
+    if st == sys::RIPP_OK {
+        st = unsafe { sys::ripp_dev_download(c.raw(), verdict.as_mut_ptr() as *mut c_void, out.ptr(), n) };
+    }
+    drop(c);
+    check(st, n, n)?;
+    Ok((verdict.into_iter().map(|v| v == 1).collect(), n_rechecked))
+}
+
+/// `verify_proofs_serialized` by random linear combination (`ripp_groth16_verify_rlc_serialized`): the same statuses
+/// except with probability at most 2^-128 per segment; proofs with a decode or input status take no part in the
+/// combinations.  The seed is drawn from `rng`.  Returns the statuses and the number of proofs verified one by one.
+pub fn verify_proofs_serialized_rlc<R: RngCore + CryptoRng>(pvk: &GpuPreparedVerifyingKey, inputs: &[u8], proofs: &[u8],
+                                                            compress: Compress, rng: &mut R) -> Result<(Vec<u8>, usize), Error> {
+    let record = if compress == Compress::Yes { 192 } else { 384 };
+    let n = proofs.len() / record;
+    let mut seed = [0u8; 32];
+    rng.fill_bytes(&mut seed);
+    let mut status = vec![0u8; n];
+    let (mut n_valid, mut n_rechecked) = (0usize, 0usize);
+    let c = ctx();
+    let st = unsafe {
+        sys::ripp_groth16_verify_rlc_serialized(c.raw(), pvk.buf.ptr(), pvk.m, inputs.as_ptr(), inputs.len(), proofs.as_ptr(),
+                                                proofs.len(), n, (compress == Compress::Yes) as i32, seed.as_ptr(),
+                                                status.as_mut_ptr(), &mut n_valid, &mut n_rechecked)
+    };
+    drop(c);
+    check(st, n, n)?;
+    Ok((status, n_rechecked))
 }
