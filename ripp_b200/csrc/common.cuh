@@ -121,13 +121,11 @@ struct TimeScope {
 ripp_ctx* ripp_child(ripp_ctx* ctx, int idx);          // lazily created; NULL on failure
 int ripp_fork(ripp_ctx* ctx, ripp_ctx* child);         // child's stream waits for everything queued on ctx's
 int ripp_join(ripp_ctx* ctx, ripp_ctx* child);         // ctx's stream waits for everything queued on child's
-int ripp_pairing_batch_internal(ripp_ctx* ctx, int nseg, const void* const* g1, const void* const* g2, size_t n, void* out);
 int ripp_pairing_batch_l6(ripp_ctx* ctx, int nseg, const void* const* g1, const void* const* g2, size_t n, void* out,
                           bool with_final_exp);
 int ripp_final_exp_l6(ripp_ctx* ctx, const void* in, uint32_t T, void* out, int nseg);
 int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n, void* out);
 int ripp_gt_check_l6(ripp_ctx* ctx, const void* in, size_t n, uint32_t* bad_dev, uint32_t flag);
-bool ripp_use_l6();
 // comm.cu: all-gather of one `bytes`-sized blob per rank on ctx's stream (recv = world * bytes, rank order); world == 1 copies
 int ripp_all_gather_internal(ripp_ctx* ctx, const void* send_dev, size_t bytes, void* recv_dev);
 void ripp_comm_release(ripp_ctx* ctx);

@@ -194,7 +194,7 @@ static int eval_products(ripp_ctx* ctx, int k, const Slice* xs, const Slice* ys,
     else
       OK(ripp_msm_g2_dev(kid, pts, sc, n, dst));
   }
-  if (np) OK(ripp_pairing_batch_internal(ctx, np, g1, g2, n, r));
+  if (np) OK(ripp_pairing_batch_l6(ctx, np, g1, g2, n, r, true));
   // results come back through the context's page-locked staging block: MSM-type ones join ctx's stream first, then
   // ONE copy of the whole result block and ONE synchronisation per batch
   uint8_t* pin;
@@ -893,7 +893,7 @@ extern "C" int ripp_sipp_prove(ripp_ctx* ctx, const void* a_aff, const void* b_a
     // lib.rs:77-78: z_l = prod e(a_R, b_L), z_r = prod e(a_L, b_R)
     const void* g1[2] = {Av + len * 96, Av};
     const void* g2[2] = {Bv, Bv + len * 192};
-    OK(ripp_pairing_batch_internal(ctx, 2, g1, g2, len, res));
+    OK(ripp_pairing_batch_l6(ctx, 2, g1, g2, len, res, true));
     Fq12 z[2];
     CU(cudaMemcpyAsync(z, res, 2 * 576, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));

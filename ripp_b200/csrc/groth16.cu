@@ -62,50 +62,21 @@ static int verify_batch(ripp_ctx* ctx, const void* pvk, size_t m, const void* x,
   return ripp_groth16_pairings_l6(ctx, a, b, d, c, K + PVK_NG, K + PVK_ND, K, n, (char*)d + o_m, pre, out);
 }
 
+// argument checks of the _dev entries
+static int check_dev_args(ripp_ctx* ctx, const void* pvk, size_t m, const void* x, const void* a, const void* b, const void* c,
+                          size_t n, const uint8_t* out) {
+  if (!ctx || !pvk || (n && (!a || !b || !c || !out || (m && !x)))) return fail(RIPP_ERR_ARG, "null argument");
+  if (n > (size_t)0xffffffffu) return fail(RIPP_ERR_ARG, "more than 2^32 - 1 proofs");
+  return RIPP_OK;
+}
+
 extern "C" int ripp_groth16_verify_batch_dev(ripp_ctx* ctx, const void* pvk_dev, size_t m, const void* inputs_dev,
                                              const void* a_dev, const void* b_dev, const void* c_dev, size_t n,
                                              uint8_t* verdict_dev) {
-  if (!ctx || !pvk_dev || (n && (!a_dev || !b_dev || !c_dev || !verdict_dev || (m && !inputs_dev))))
-    return fail(RIPP_ERR_ARG, "null argument");
-  if (n > (size_t)0xffffffffu) return fail(RIPP_ERR_ARG, "more than 2^32 - 1 proofs");
+  OK(check_dev_args(ctx, pvk_dev, m, inputs_dev, a_dev, b_dev, c_dev, n, verdict_dev));
   if (n == 0) return RIPP_OK;
   CU(cudaSetDevice(ctx->device));
   return verify_batch(ctx, pvk_dev, m, inputs_dev, a_dev, b_dev, c_dev, n, nullptr, verdict_dev);
-}
-
-extern "C" int ripp_groth16_verify_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host,
-                                              size_t inputs_len, const uint8_t* proofs_host, size_t proofs_len, size_t n,
-                                              int compressed, uint8_t* status_host, size_t* n_valid) {
-  if (!ctx || !pvk_dev || !n_valid || (n && (!proofs_host || !status_host || (m && !inputs_host))))
-    return fail(RIPP_ERR_ARG, "null argument");
-  if (n > (size_t)0xffffffffu) return fail(RIPP_ERR_ARG, "more than 2^32 - 1 proofs");
-  const size_t rec = compressed ? 192 : 384;
-  if (proofs_len != n * rec)
-    return fail(RIPP_ERR_ARG, "proof bytes: " + std::to_string(proofs_len) + " bytes is not " + std::to_string(n) + " records of " +
-                                  std::to_string(rec) + " bytes");
-  if (m > (((size_t)1 << 40) / 32) || inputs_len != n * m * 32)
-    return fail(RIPP_ERR_ARG, "input bytes: " + std::to_string(inputs_len) + " bytes is not " + std::to_string(n) + " x " +
-                                  std::to_string(m) + " elements of 32 bytes");
-  *n_valid = 0;
-  if (n == 0) return RIPP_OK;
-  CU(cudaSetDevice(ctx->device));
-  auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-  const size_t xb = n * m * 32;
-  DecodedProofs dp;
-  OK(ripp_decode_proofs(ctx, proofs_host, n, compressed, 2 * up(xb) + n, &dp));
-  uint8_t* xin = (uint8_t*)dp.extra;
-  Fr* x = (Fr*)(xin + up(xb));
-  uint8_t* st = xin + 2 * up(xb);
-  if (xb) CU(cudaMemcpyAsync(xin, inputs_host, xb, cudaMemcpyHostToDevice, ctx->stream));
-  k_fr_deserialize<<<(unsigned)((n + 63) / 64), 64, 0, ctx->stream>>>(xin, (uint32_t)n, (uint32_t)m, dp.status, x, st);
-  LAUNCHED(ctx);
-  OK(verify_batch(ctx, pvk_dev, m, x, dp.a, dp.b, dp.c, n, st, st));
-  CU(cudaMemcpyAsync(status_host, st, n, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  size_t ok = 0;
-  for (size_t i = 0; i < n; i++) ok += status_host[i] == RIPP_GROTH16_OK;
-  *n_valid = ok;
-  return RIPP_OK;
 }
 
 // ---- verification by random linear combination (include/ripp_b200.h "ripp_groth16_verify_rlc_dev") -----------------
@@ -277,9 +248,8 @@ static int verify_rlc(ripp_ctx* ctx, const void* pvk, size_t m, const void* x, c
 extern "C" int ripp_groth16_verify_rlc_dev(ripp_ctx* ctx, const void* pvk_dev, size_t m, const void* inputs_dev, const void* a_dev,
                                            const void* b_dev, const void* c_dev, size_t n, const uint8_t* seed32,
                                            uint8_t* verdict_dev, size_t* n_rechecked) {
-  if (!ctx || !pvk_dev || !seed32 || !n_rechecked || (n && (!a_dev || !b_dev || !c_dev || !verdict_dev || (m && !inputs_dev))))
-    return fail(RIPP_ERR_ARG, "null argument");
-  if (n > (size_t)0xffffffffu) return fail(RIPP_ERR_ARG, "more than 2^32 - 1 proofs");
+  if (!seed32 || !n_rechecked) return fail(RIPP_ERR_ARG, "null argument");
+  OK(check_dev_args(ctx, pvk_dev, m, inputs_dev, a_dev, b_dev, c_dev, n, verdict_dev));
   *n_rechecked = 0;
   if (n == 0) return RIPP_OK;
   CU(cudaSetDevice(ctx->device));
@@ -288,11 +258,12 @@ extern "C" int ripp_groth16_verify_rlc_dev(ripp_ctx* ctx, const void* pvk_dev, s
   return RIPP_OK;
 }
 
-extern "C" int ripp_groth16_verify_rlc_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host,
-                                                  size_t inputs_len, const uint8_t* proofs_host, size_t proofs_len, size_t n,
-                                                  int compressed, const uint8_t* seed32, uint8_t* status_host, size_t* n_valid,
-                                                  size_t* n_rechecked) {
-  if (!ctx || !pvk_dev || !seed32 || !n_valid || !n_rechecked || (n && (!proofs_host || !status_host || (m && !inputs_host))))
+// The serialized entries: one H2D copy of the records and one of the inputs, the decode of A, B, C and of the inputs,
+// then verify_rlc with seed32 (n_rechecked set), or verify_batch without; the statuses go back to status_host.
+static int verify_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host, size_t inputs_len,
+                             const uint8_t* proofs_host, size_t proofs_len, size_t n, int compressed, const uint8_t* seed32,
+                             uint8_t* status_host, size_t* n_valid, size_t* n_rechecked) {
+  if (!ctx || !pvk_dev || !n_valid || (n && (!proofs_host || !status_host || (m && !inputs_host))))
     return fail(RIPP_ERR_ARG, "null argument");
   if (n > (size_t)0xffffffffu) return fail(RIPP_ERR_ARG, "more than 2^32 - 1 proofs");
   const size_t rec = compressed ? 192 : 384;
@@ -303,7 +274,7 @@ extern "C" int ripp_groth16_verify_rlc_serialized(ripp_ctx* ctx, const void* pvk
     return fail(RIPP_ERR_ARG, "input bytes: " + std::to_string(inputs_len) + " bytes is not " + std::to_string(n) + " x " +
                                   std::to_string(m) + " elements of 32 bytes");
   *n_valid = 0;
-  *n_rechecked = 0;
+  if (seed32) *n_rechecked = 0;
   if (n == 0) return RIPP_OK;
   CU(cudaSetDevice(ctx->device));
   auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
@@ -316,11 +287,30 @@ extern "C" int ripp_groth16_verify_rlc_serialized(ripp_ctx* ctx, const void* pvk
   if (xb) CU(cudaMemcpyAsync(xin, inputs_host, xb, cudaMemcpyHostToDevice, ctx->stream));
   k_fr_deserialize<<<(unsigned)((n + 63) / 64), 64, 0, ctx->stream>>>(xin, (uint32_t)n, (uint32_t)m, dp.status, x, st);
   LAUNCHED(ctx);
-  OK(verify_rlc(ctx, pvk_dev, m, x, dp.a, dp.b, dp.c, n, seed32, st, st, n_rechecked));
+  if (seed32)
+    OK(verify_rlc(ctx, pvk_dev, m, x, dp.a, dp.b, dp.c, n, seed32, st, st, n_rechecked));
+  else
+    OK(verify_batch(ctx, pvk_dev, m, x, dp.a, dp.b, dp.c, n, st, st));
   CU(cudaMemcpyAsync(status_host, st, n, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
-  size_t okc = 0;
-  for (size_t i = 0; i < n; i++) okc += status_host[i] == RIPP_GROTH16_OK;
-  *n_valid = okc;
+  size_t ok = 0;
+  for (size_t i = 0; i < n; i++) ok += status_host[i] == RIPP_GROTH16_OK;
+  *n_valid = ok;
   return RIPP_OK;
+}
+
+extern "C" int ripp_groth16_verify_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host,
+                                              size_t inputs_len, const uint8_t* proofs_host, size_t proofs_len, size_t n,
+                                              int compressed, uint8_t* status_host, size_t* n_valid) {
+  return verify_serialized(ctx, pvk_dev, m, inputs_host, inputs_len, proofs_host, proofs_len, n, compressed, nullptr, status_host,
+                           n_valid, nullptr);
+}
+
+extern "C" int ripp_groth16_verify_rlc_serialized(ripp_ctx* ctx, const void* pvk_dev, size_t m, const uint8_t* inputs_host,
+                                                  size_t inputs_len, const uint8_t* proofs_host, size_t proofs_len, size_t n,
+                                                  int compressed, const uint8_t* seed32, uint8_t* status_host, size_t* n_valid,
+                                                  size_t* n_rechecked) {
+  if (!seed32 || !n_rechecked) return fail(RIPP_ERR_ARG, "null argument");
+  return verify_serialized(ctx, pvk_dev, m, inputs_host, inputs_len, proofs_host, proofs_len, n, compressed, seed32, status_host,
+                           n_valid, n_rechecked);
 }

@@ -201,45 +201,38 @@ static __device__ __forceinline__ Ctx3 ctx18(uint32_t* wsm, int group_words_no_b
   return Ctx3{vl / 3, wsm, nullptr, vl % 3, wsm + group_words_no_bus, 0, wsm + group_words_no_bus + BUS_ZERO};
 }
 constexpr int M18_WARPS = 4;
-template <int KP>
-RIPP_HD constexpr int m18_group_words() { return group_words(M6_NREG, KP) + BUS_TOTAL; }
+constexpr int M18_GROUP_WORDS = group_words(M6_NREG, 1) + BUS_TOTAL;
 
-// grid (ceil(wps / 4), nseg): warp w of segment s walks pairs [w KP, w KP + KP); the CTA's four Miller values are
-// multiplied in shared memory; one partial per CTA at partials[s * gridDim.x + blockIdx.x].
-template <int KP>
+// grid (ceil(n / 4), nseg): warp w of segment s walks pair w; the CTA's four Miller values are multiplied in shared
+// memory; one partial per CTA at partials[s * gridDim.x + blockIdx.x].
 __global__ void __launch_bounds__(32 * M18_WARPS) k_miller18(Miller6Batch b, Fq12* __restrict__ partials) {
   extern __shared__ __align__(16) uint32_t smem[];
-  constexpr int GW = m18_group_words<KP>();
   const int warp = threadIdx.x >> 5;
-  uint32_t* wsm = smem + warp * GW;
-  Ctx3 c = ctx18(wsm, group_words(M6_NREG, KP));
+  uint32_t* wsm = smem + warp * M18_GROUP_WORDS;
+  Ctx3 c = ctx18(wsm, group_words(M6_NREG, 1));
   uint32_t* pairs = c.sm + OFF_F + M6_NREG * F12W;
-  const uint32_t seg = blockIdx.y, wl = blockIdx.x * M18_WARPS + warp;
+  const uint32_t seg = blockIdx.y, i = blockIdx.x * M18_WARPS + warp;
   if (c.k == 0 && c.role == 0) {
-    for (int j = 0; j < KP; j++) {
-      const uint32_t i = wl * KP + j;
-      G1Aff P = g1_generator();
-      const G2Aff* Q = &g_g2_gen;
-      uint32_t valid = 0;
-      if (i < b.n) {
-        G1Aff p = b.p[seg][i];
-        const G2Aff* q = &b.q[seg][i];
-        if (!p.is_inf() && !q->is_inf()) {
-          P = p;
-          Q = q;
-          valid = 1;
-        }
+    G1Aff P = g1_generator();
+    const G2Aff* Q = &g_g2_gen;
+    uint32_t valid = 0;
+    if (i < b.n) {
+      G1Aff p = b.p[seg][i];
+      const G2Aff* q = &b.q[seg][i];
+      if (!p.is_inf() && !q->is_inf()) {
+        P = p;
+        Q = q;
+        valid = 1;
       }
-      uint32_t* pb = pairs + j * PAIR_WORDS;
-      stage_pair_p(pb, P);
-      set_pair_q(pb, Q);
-      pb[PB_VALID] = valid;
     }
+    stage_pair_p(pairs, P);
+    set_pair_q(pairs, Q);
+    pairs[PB_VALID] = valid;
   }
   __syncwarp();
-  miller(c, pairs, KP);
+  miller(c, pairs, 1);
   uint32_t* F0 = freg(c, 0);
-  auto other = [&](int w) { return smem + w * GW + OFF_F; };
+  auto other = [&](int w) { return smem + w * M18_GROUP_WORDS + OFF_F; };
   __syncthreads();
   if ((warp & 1) == 0) mul_p(c, F0, F0, other(warp + 1));
   __syncthreads();
@@ -353,6 +346,24 @@ int ripp_gt_check_l6(ripp_ctx* ctx, const void* in, size_t n, uint32_t* bad_dev,
   return RIPP_OK;
 }
 
+// k_reduce6 levels over nseg runs of *T partials each, run s at *src + s * *T: out[s][j] = prod in[s][j*R .. j*R+R), R = 8,
+// until at most `stop` are left per run.  The level that leaves one per run writes to `last` when given, else the levels
+// ping-pong between *src and dst.  *src and *T then hold the result.
+static int reduce6(ripp_ctx* ctx, uint32_t nseg, uint32_t stop, Fq12** src, Fq12* dst, uint32_t* T, Fq12* last = nullptr) {
+  const uint32_t R = 8;
+  while (*T > stop) {
+    const uint32_t To = (*T + R - 1) / R, tot = nseg * To;
+    Fq12* o = To == 1 && last ? last : dst;
+    k_reduce6<M6_WARPS><<<(tot + 5 * M6_WARPS - 1) / (5 * M6_WARPS), 32 * M6_WARPS, M6_WARPS * 6 * R6_GROUP_WORDS * 4, ctx->stream>>>(
+        *src, *T, R, To, o, tot);
+    LAUNCHED(ctx);
+    dst = *src;
+    *src = o;
+    *T = To;
+  }
+  return RIPP_OK;
+}
+
 // out = prod_i in[i]^sc[i]  (device memory; in: n Fq12, sc: n Fr Montgomery)
 int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n, void* out) {
   CU(cudaSetDevice(ctx->device));
@@ -373,33 +384,69 @@ int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n,
     k_gt_pow6<<<(unsigned)((n + 4) / 5), 32, 6 * GP_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)in, (const Fr*)sc, (uint32_t)n,
                                                                                     n == 1 ? (Fq12*)out : (Fq12*)bufA);
   LAUNCHED(ctx);
-  const uint32_t R = 8;
-  Fq12 *src = (Fq12*)bufA, *dst = (Fq12*)bufB;
+  Fq12* src = (Fq12*)bufA;
   uint32_t T = (uint32_t)n;
-  while (T > 1) {
-    uint32_t To = (T + R - 1) / R;
-    Fq12* o = To == 1 ? (Fq12*)out : dst;
-    unsigned blk = (To + 5 * M6_WARPS - 1) / (5 * M6_WARPS);
-    k_reduce6<M6_WARPS><<<blk, 32 * M6_WARPS, M6_WARPS * 6 * R6_GROUP_WORDS * 4, ctx->stream>>>(src, T, R, To, o, To);
-    LAUNCHED(ctx);
-    Fq12* t = src;
-    src = dst;
-    dst = t;
-    T = To;
+  return reduce6(ctx, 1, 1, &src, (Fq12*)bufB, &T, (Fq12*)out);
+}
+
+// Pairs per six-lane group for nseg segments of pairs_per_seg pairs (the pairs of a group share the accumulator's
+// squaring).  All warps of a launch do equal work, so the launch takes ceil(warps / resident warps) waves of one warp's
+// duration; per doubling step a warp spends ~2040 MAC32 on the shared squaring and ~3096 per pair (point step + sparse
+// line product).  Pick the kp in {1..4} with the cheapest waves x duration -- e.g. 12 288 pairs (TIPP 2^12, first
+// round): kp = 2 is two waves, kp = 3 one.  RIPP_B200_M6_KP pins kp; background work takes 4.  `many_waves`: a launch of
+// three or more waves at kp = 4 takes kp = 4 without the comparison.  The RLC check passes false: at n = 100 000
+// (1725 segments) that shortcut's kp = 4 measured 56.3 ms against 55.6 ms at the compared kp = 3 (DESIGN.md §6).
+static int m6_pairs_per_group(ripp_ctx* ctx, size_t nseg, size_t pairs_per_seg, bool many_waves, int* kp_out) {
+  int sms = 0;
+  CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
+  const size_t resident = (size_t)sms * 2 * M6_WARPS;  // two CTAs per SM (255 registers)
+  int kp = 4;
+  double best = 0;
+  // many waves: CTAs are scheduled as others retire, the tail of the last wave is a small share -- most sharing wins
+  // (six or eight pairs per group fit the shared memory since Q left the pair block, but measured no better: 2^18 pairs
+  // 77.3 ms at kp = 4, 80.2 at 6, 78.9 at 8; 2^16: 19.7 / 19.4 / 23.8 ms)
+  const bool many = many_waves && nseg * ((pairs_per_seg + 19) / 20) >= 3 * resident;
+  for (int k = 1; k <= 4 && !many; k++) {
+    const size_t warps = nseg * ((pairs_per_seg + 5 * k - 1) / (5 * k));
+    const double t = (double)((warps + resident - 1) / resident) * (2040.0 + 3096.0 * k);
+    if (k == 1 || t <= best) {
+      best = t;
+      kp = k;
+    }
   }
+  static const int force = [] {
+    const char* e = getenv("RIPP_B200_M6_KP");
+    return e ? atoi(e) : 0;
+  }();
+  if (force >= 1 && force <= 4) kp = force;
+  if (ctx->background) kp = 4;
+  *kp_out = kp;
   return RIPP_OK;
 }
 
 template <int KP>
-static int launch_miller6(ripp_ctx* ctx, Miller6Batch& b, size_t n, Fq12* dst, size_t* nwarps_out) {
-  constexpr int SM = m6_smem_bytes(KP);
-  b.wps = (uint32_t)((n + 5 * KP - 1) / (5 * KP));
-  size_t nwarps = (size_t)b.wps * b.nseg;
-  unsigned blocks = (unsigned)((nwarps + M6_WARPS - 1) / M6_WARPS);
-  k_miller6<M6_WARPS, KP><<<blocks, 32 * M6_WARPS, SM, ctx->stream>>>(b, dst);
+static int launch_miller6(ripp_ctx* ctx, Miller6Batch& b, Fq12* dst) {
+  b.wps = (uint32_t)(((size_t)b.n + 5 * KP - 1) / (5 * KP));
+  const size_t nwarps = (size_t)b.wps * b.nseg;
+  k_miller6<M6_WARPS, KP><<<(unsigned)((nwarps + M6_WARPS - 1) / M6_WARPS), 32 * M6_WARPS, m6_smem_bytes(KP), ctx->stream>>>(b, dst);
   LAUNCHED(ctx);
-  *nwarps_out = nwarps;
   return RIPP_OK;
+}
+
+// The six-lane products: one k_miller6 launch at kp pairs per group (one partial per warp, at *src), then reduce6 over
+// nseg equal runs of those partials down to `stop` per run.  The runs are b's segments, or (the RLC check) the
+// warp-aligned segments inside b's one segment.
+static int m6_products(ripp_ctx* ctx, Miller6Batch& b, int kp, uint32_t nseg, uint32_t stop, Fq12** src, Fq12* dst, uint32_t* T) {
+  if (kp == 4)
+    OK(launch_miller6<4>(ctx, b, *src));
+  else if (kp == 3)
+    OK(launch_miller6<3>(ctx, b, *src));
+  else if (kp == 2)
+    OK(launch_miller6<2>(ctx, b, *src));
+  else
+    OK(launch_miller6<1>(ctx, b, *src));
+  *T = (uint32_t)((size_t)b.wps * b.nseg / nseg);
+  return reduce6(ctx, nseg, stop, src, dst, T);
 }
 
 int ripp_pairing_batch_l6(ripp_ctx* ctx, int nseg, const void* const* g1, const void* const* g2, size_t n, void* out,
@@ -427,111 +474,35 @@ int ripp_pairing_batch_l6(ripp_ctx* ctx, int nseg, const void* const* g1, const 
   OK(scratch(ctx, 3, max_partials * sizeof(Fq12) / 4 + 8192, &bufB));
   Fq12 *src = (Fq12*)bufA, *dst = (Fq12*)bufB;
   uint32_t T;
-  const size_t w18 = l18_max_warps();
-  // eighteen-lane warps with ONE pair each, up to l18_max_warps pairs (two warps per sub-partition); above that the
-  // six-lane shape wins -- measured (gpurun_out/r2o): six products of 256 / 512 pairs 3.80 / 5.68 ms with 2 / 4 pairs per
-  // eighteen-lane warp, 3.18 / 3.69 ms on six lanes; TIPP 2^12 93.5 -> 87.8 ms.  RIPP_B200_L18_KP = 2 / 4 re-enables them.
-  static const int l18_kp_max = [] {
-    const char* e = getenv("RIPP_B200_L18_KP");
-    return e ? atoi(e) : 1;
-  }();
-  if (total <= (size_t)l18_kp_max * w18) {
-    // latency shape: one pair (or 2 / 4 sharing an accumulator) per eighteen-lane warp, four warps per CTA combined
-    // in shared memory, then a tree of one-warp products and one warp per final exponentiation
-    {
-      TimeScope ts_(ctx, RIPP_T_MILLER);
-      const int kp = total <= w18 ? 1 : (total <= 2 * w18 ? 2 : 4);
-      const uint32_t wps = (uint32_t)((n + kp - 1) / kp), ctas = (wps + M18_WARPS - 1) / M18_WARPS;
-      b.wps = wps;
-      dim3 grid(ctas, nseg);
-      if (kp == 1)
-        k_miller18<1><<<grid, 32 * M18_WARPS, M18_WARPS * m18_group_words<1>() * 4, ctx->stream>>>(b, src);
-      else if (kp == 2)
-        k_miller18<2><<<grid, 32 * M18_WARPS, M18_WARPS * m18_group_words<2>() * 4, ctx->stream>>>(b, src);
-      else
-        k_miller18<4><<<grid, 32 * M18_WARPS, M18_WARPS * m18_group_words<4>() * 4, ctx->stream>>>(b, src);
-      LAUNCHED(ctx);
-      T = ctas;
-      const uint32_t R = 4, stop = with_final_exp ? R : 1;
-      while (T > stop) {
-        uint32_t To = (T + R - 1) / R, tot = (uint32_t)nseg * To;
-        k_reduce18<<<(tot + M18_WARPS - 1) / M18_WARPS, 32 * M18_WARPS, M18_WARPS * R18_GROUP_WORDS * 4, ctx->stream>>>(src, T, R, To,
-                                                                                                                     dst, tot);
-        LAUNCHED(ctx);
-        Fq12* t = src;
-        src = dst;
-        dst = t;
-        T = To;
-      }
-    }
-    if (!with_final_exp) {
-      CU(cudaMemcpyAsync(out, src, (size_t)nseg * sizeof(Fq12), cudaMemcpyDeviceToDevice, ctx->stream));
-      return RIPP_OK;
-    }
-    TimeScope ts2_(ctx, RIPP_T_FINAL_EXP);
-    k_final_exp18<<<nseg, 32, FE18_GROUP_WORDS * 4, ctx->stream>>>(src, T, (Fq12*)out);
-    LAUNCHED(ctx);
-    return RIPP_OK;
-  }
-  // throughput shape.  Pairs per group (they share the accumulator's squaring): all warps of a launch do equal work, so the
-  // launch takes ceil(warps / resident warps) waves of one warp's duration; per doubling step a warp spends ~2040 MAC32
-  // on the shared squaring and ~3096 per pair (point step + sparse line product).  Pick the kp in {1..4} with the
-  // cheapest waves x duration -- e.g. 12 288 pairs (TIPP 2^12, first round): kp = 2 is two waves, kp = 3 one.
-  int kp = 4;
-  {
-    cudaDeviceProp prop;
-    static int sms = 0;
-    if (!sms) {
-      CU(cudaGetDeviceProperties(&prop, ctx->device));
-      sms = prop.multiProcessorCount;
-    }
-    const size_t resident = (size_t)sms * 2 * M6_WARPS;  // two CTAs per SM (255 registers)
-    double best = 0;
-    // many waves: CTAs are scheduled as others retire, the tail of the last wave is a small share -- most sharing wins
-    // (six or eight pairs per group fit the shared memory since Q left the pair block, but measured no better: 2^18 pairs
-    // 77.3 ms at kp = 4, 80.2 at 6, 78.9 at 8; 2^16: 19.7 / 19.4 / 23.8 ms)
-    const bool many = (size_t)nseg * ((n + 19) / 20) >= 3 * resident;
-    for (int k = 1; k <= 4 && !many; k++) {
-      const int ci = k - 1;
-      size_t warps = (size_t)nseg * ((n + 5 * k - 1) / (5 * k));
-      double t = (double)((warps + resident - 1) / resident) * (2040.0 + 3096.0 * k);
-      if (ci == 0 || t <= best) {
-        best = t;
-        kp = k;
-      }
-    }
-    static const int force = [] {
-      const char* e = getenv("RIPP_B200_M6_KP");
-      return e ? atoi(e) : 0;
-    }();
-    if (force >= 1 && force <= 4) kp = force;
-    if (ctx->background) kp = 4;
-  }
-  const uint32_t R = 8;
-  size_t nwarps = 0;
-  {
+  if (total <= l18_max_warps()) {
+    // latency shape: one pair per eighteen-lane warp, up to l18_max_warps pairs (two warps per sub-partition); four
+    // warps per CTA combined in shared memory, then a tree of one-warp products and one warp per final exponentiation.
+    // Above that the six-lane shape wins, also against two or four pairs per eighteen-lane warp -- measured: six products
+    // of 256 / 512 pairs 3.80 / 5.68 ms with 2 / 4 pairs per eighteen-lane warp, 3.18 / 3.69 ms on six lanes; TIPP 2^12
+    // 93.5 -> 87.8 ms.
     TimeScope ts_(ctx, RIPP_T_MILLER);
-    if (kp == 4)
-      OK(launch_miller6<4>(ctx, b, n, src, &nwarps));
-    else if (kp == 3)
-      OK(launch_miller6<3>(ctx, b, n, src, &nwarps));
-    else if (kp == 2)
-      OK(launch_miller6<2>(ctx, b, n, src, &nwarps));
-    else
-      OK(launch_miller6<1>(ctx, b, n, src, &nwarps));
-    T = b.wps;
-    uint32_t stop = with_final_exp ? 4 : 1;
+    const uint32_t ctas = ((uint32_t)n + M18_WARPS - 1) / M18_WARPS;
+    k_miller18<<<dim3(ctas, nseg), 32 * M18_WARPS, M18_WARPS * M18_GROUP_WORDS * 4, ctx->stream>>>(b, src);
+    LAUNCHED(ctx);
+    T = ctas;
+    const uint32_t R = 4, stop = with_final_exp ? R : 1;
     while (T > stop) {
-      uint32_t To = (T + R - 1) / R;
-      uint32_t tot = (uint32_t)nseg * To;
-      unsigned blk = (tot + 5 * M6_WARPS - 1) / (5 * M6_WARPS);
-      k_reduce6<M6_WARPS><<<blk, 32 * M6_WARPS, M6_WARPS * 6 * R6_GROUP_WORDS * 4, ctx->stream>>>(src, T, R, To, dst, tot);
+      uint32_t To = (T + R - 1) / R, tot = (uint32_t)nseg * To;
+      k_reduce18<<<(tot + M18_WARPS - 1) / M18_WARPS, 32 * M18_WARPS, M18_WARPS * R18_GROUP_WORDS * 4, ctx->stream>>>(src, T, R, To,
+                                                                                                                   dst, tot);
       LAUNCHED(ctx);
       Fq12* t = src;
       src = dst;
       dst = t;
       T = To;
     }
+  } else {
+    // throughput shape: several pairs per six-lane group, the k_reduce6 tree down to at most four partials per segment
+    // for k_final_exp18 (one without it)
+    int kp;
+    OK(m6_pairs_per_group(ctx, nseg, n, true, &kp));
+    TimeScope ts_(ctx, RIPP_T_MILLER);
+    OK(m6_products(ctx, b, kp, nseg, with_final_exp ? 4 : 1, &src, dst, &T));
   }
   if (!with_final_exp) {
     CU(cudaMemcpyAsync(out, src, (size_t)nseg * sizeof(Fq12), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -609,30 +580,8 @@ __global__ void __launch_bounds__(64) k_rlc_pairs(const G1Aff* __restrict__ ra, 
 
 int ripp_groth16_rlc_pairings_l6(ripp_ctx* ctx, const void* ra, const void* b, const void* ps, const void* cs, const void* neg_gamma,
                                  const void* neg_delta, const void* ab, size_t n, size_t s, size_t nseg, uint8_t* ok) {
-  // pairs per group as ripp_pairing_batch_l6's throughput shape: the cheapest waves x warp duration, here counting each
-  // segment's padding
-  static int sms = 0;
-  if (!sms) {
-    cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, ctx->device));
-    sms = prop.multiProcessorCount;
-  }
-  const size_t resident = (size_t)sms * 2 * M6_WARPS;
-  int kp = 1;
-  double best = 0;
-  for (int k = 1; k <= 4; k++) {
-    const size_t warps = nseg * ((s + 2 + 5 * k - 1) / (5 * k));
-    const double t = (double)((warps + resident - 1) / resident) * (2040.0 + 3096.0 * k);
-    if (k == 1 || t <= best) {
-      best = t;
-      kp = k;
-    }
-  }
-  static const int force = [] {
-    const char* e = getenv("RIPP_B200_M6_KP");
-    return e ? atoi(e) : 0;
-  }();
-  if (force >= 1 && force <= 4) kp = force;
+  int kp;
+  OK(m6_pairs_per_group(ctx, nseg, s + 2, false, &kp));  // a segment's s proofs and two fixed-Q pairs, before padding
   const size_t ppw = 5 * (size_t)kp, sp = (s + 2 + ppw - 1) / ppw * ppw, np = nseg * sp, T0 = sp / ppw;
   void *pq, *part;
   const size_t o_q = (np * sizeof(G1Aff) + 255) & ~(size_t)255;
@@ -654,28 +603,9 @@ int ripp_groth16_rlc_pairings_l6(ripp_ctx* ctx, const void* ra, const void* b, c
     mb.q[0] = Q;
     mb.n = (uint32_t)np;
     mb.nseg = 1;
-    size_t nwarps = 0;
-    if (kp == 4)
-      OK(launch_miller6<4>(ctx, mb, np, src, &nwarps));
-    else if (kp == 3)
-      OK(launch_miller6<3>(ctx, mb, np, src, &nwarps));
-    else if (kp == 2)
-      OK(launch_miller6<2>(ctx, mb, np, src, &nwarps));
-    else
-      OK(launch_miller6<1>(ctx, mb, np, src, &nwarps));
-    // partials [seg * T + w] -> one Miller value per segment
-    const uint32_t R = 8;
-    uint32_t T = (uint32_t)T0;
-    while (T > 1) {
-      const uint32_t To = (T + R - 1) / R, tot = (uint32_t)nseg * To;
-      k_reduce6<M6_WARPS><<<(tot + 5 * M6_WARPS - 1) / (5 * M6_WARPS), 32 * M6_WARPS, M6_WARPS * 6 * R6_GROUP_WORDS * 4, ctx->stream>>>(
-          src, T, R, To, dst, tot);
-      LAUNCHED(ctx);
-      Fq12* t = src;
-      src = dst;
-      dst = t;
-      T = To;
-    }
+    // partials [seg * T0 + w] -> one Miller value per segment
+    uint32_t T;
+    OK(m6_products(ctx, mb, kp, (uint32_t)nseg, 1, &src, dst, &T));
   }
   TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
   k_groth16_check6<<<(unsigned)((nseg + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>(src, (const Fq12*)ab, (uint32_t)nseg,

@@ -163,49 +163,6 @@ __global__ void k_normalize(const Jac<F>* __restrict__ in, Aff<F>* __restrict__ 
 }
 
 // ------------------------------------------------------------------------------------------------
-// kernels: multi-Miller loop.  One (G1, G2) pair per thread; the 32 Miller values of a warp are
-// multiplied with a shuffle butterfly and lane 0 writes one Fq12 partial per warp.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ Fq12 shfl_xor_fq12(const Fq12& a, int m) {
-  Fq12 r;
-  const uint32_t* pa = reinterpret_cast<const uint32_t*>(&a);
-  uint32_t* pr = reinterpret_cast<uint32_t*>(&r);
-#pragma unroll
-  for (int i = 0; i < 144; i++) pr[i] = __shfl_xor_sync(0xffffffffu, pa[i], m);
-  return r;
-}
-
-#ifndef RIPP_MILLER_THREADS_PER_SM
-#define RIPP_MILLER_THREADS_PER_SM 256
-#endif
-template <int BLOCK>
-__global__ void __launch_bounds__(BLOCK, RIPP_MILLER_THREADS_PER_SM / BLOCK) k_miller(const G1Aff* __restrict__ ps, const G2Aff* __restrict__ qs, size_t n,
-                                                 Fq12* __restrict__ partials) {
-  size_t i = (size_t)blockIdx.x * BLOCK + threadIdx.x;
-  Fq12 f = Fq12::one();
-  if (i < n) f = miller_loop(ps[i], qs[i]);
-#pragma unroll 1
-  for (int m = 16; m >= 1; m >>= 1) f = f * shfl_xor_fq12(f, m);
-  if ((threadIdx.x & 31) == 0) partials[i >> 5] = f;
-}
-
-// out[t] = prod in[t*R .. min(m, t*R+R))
-__global__ void k_fq12_reduce(const Fq12* __restrict__ in, size_t m, int R, Fq12* __restrict__ out) {
-  size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  size_t lo = t * R;
-  if (lo >= m) return;
-  size_t hi = lo + R < m ? lo + R : m;
-  Fq12 f = in[lo];
-  for (size_t j = lo + 1; j < hi; j++) f = f * in[j];
-  out[t] = f;
-}
-
-__global__ void k_final_exp(const Fq12* __restrict__ in, Fq12* __restrict__ out, size_t n) {
-  size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t < n) out[t] = final_exponentiation(in[t]);
-}
-
-// ------------------------------------------------------------------------------------------------
 // kernels: element-wise scalar multiplication with distinct scalars (K8)
 // ------------------------------------------------------------------------------------------------
 template <class F, bool GEN>
@@ -626,167 +583,25 @@ extern "C" int ripp_bench_imad(ripp_ctx* ctx, int kind, int iters, double* macs_
 }
 
 // ------------------------------------------------------------------------------------------------
-// L1: pairing inner product
+// L1: pairing inner product (the lane engines of pairing6.cu)
 // ------------------------------------------------------------------------------------------------
-static const int MILLER_BLOCK = 64;
-
-static int miller_partial(ripp_ctx* ctx, const G1Aff* p, const G2Aff* q, size_t n, Fq12* out_dev) {
-  if (ripp_use_l6()) {
-    const void* g1[1] = {p};
-    const void* g2[1] = {q};
-    return ripp_pairing_batch_l6(ctx, 1, g1, g2, n, out_dev, false);
-  }
-  if (n == 0) {
-    Fq12 one = Fq12::one();
-    CU(cudaMemcpyAsync(out_dev, &one, sizeof(one), cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return RIPP_OK;
-  }
-  size_t nblocks = (n + MILLER_BLOCK - 1) / MILLER_BLOCK;
-  size_t nwarps = nblocks * (MILLER_BLOCK / 32);
-  const int R = 8;
-  void *bufA, *bufB;
-  OK(scratch(ctx, 2, nwarps * sizeof(Fq12), &bufA));
-  OK(scratch(ctx, 3, ((nwarps + R - 1) / R) * sizeof(Fq12) + 256, &bufB));
-  TimeScope ts_(ctx, RIPP_T_MILLER);
-  k_miller<MILLER_BLOCK><<<(unsigned)nblocks, MILLER_BLOCK, 0, ctx->stream>>>(p, q, n, (Fq12*)bufA);
-  LAUNCHED(ctx);
-  size_t m = nwarps;
-  Fq12 *src = (Fq12*)bufA, *dst = (Fq12*)bufB;
-  while (m > 1) {
-    size_t mo = (m + R - 1) / R;
-    Fq12* o = (mo == 1) ? out_dev : dst;
-    k_fq12_reduce<<<(unsigned)((mo + 63) / 64), 64, 0, ctx->stream>>>(src, m, R, o);
-    LAUNCHED(ctx);
-    Fq12* t = src;
-    src = dst;
-    dst = t;
-    m = mo;
-  }
-  if (nwarps == 1) CU(cudaMemcpyAsync(out_dev, bufA, sizeof(Fq12), cudaMemcpyDeviceToDevice, ctx->stream));
-  return RIPP_OK;
-}
-
-// ---- batched products: several equal-length (G1, G2) vector pairs in one Miller launch ----------
-struct MillerBatch {
-  const G1Aff* p[RIPP_MAX_BATCH];
-  const G2Aff* q[RIPP_MAX_BATCH];
-  uint32_t n, wps;  // pairs per segment, warps per segment
-  int nseg;
-};
-
-template <int BLOCK>
-__global__ void __launch_bounds__(BLOCK, RIPP_MILLER_THREADS_PER_SM / BLOCK) k_miller_batch(MillerBatch b, Fq12* __restrict__ partials) {
-  uint32_t gw = (blockIdx.x * BLOCK + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-  uint32_t seg = gw / b.wps, i = (gw % b.wps) * 32 + lane;
-  Fq12 f = Fq12::one();
-  if (seg < (uint32_t)b.nseg && i < b.n) f = miller_loop(b.p[seg][i], b.q[seg][i]);
-#pragma unroll 1
-  for (int m = 16; m >= 1; m >>= 1) f = f * shfl_xor_fq12(f, m);
-  if (lane == 0 && seg < (uint32_t)b.nseg) partials[gw] = f;
-}
-
-// out[s][k] = prod in[s][k*R .. min(T, k*R+R))
-__global__ void k_fq12_reduce_seg(const Fq12* __restrict__ in, uint32_t T, uint32_t R, uint32_t To, Fq12* __restrict__ out,
-                                  size_t total) {
-  size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= total) return;
-  uint32_t s = (uint32_t)(t / To), k = (uint32_t)(t % To);
-  uint32_t lo = k * R, hi = lo + R < T ? lo + R : T;
-  Fq12 f = in[(size_t)s * T + lo];
-  for (uint32_t j = lo + 1; j < hi; j++) f = f * in[(size_t)s * T + j];
-  out[t] = f;
-}
-
-// out[s] = final_exp(prod_j in[s][j]), j < T (T small)
-__global__ void k_final_exp_seg(const Fq12* __restrict__ in, uint32_t T, Fq12* __restrict__ out, int nseg) {
-  int s = blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= nseg) return;
-  Fq12 f = in[(size_t)s * T];
-  for (uint32_t j = 1; j < T; j++) f = f * in[(size_t)s * T + j];
-  out[s] = final_exponentiation(f);
-}
-
-bool ripp_use_l6() {
-  static const bool v = [] {  // thread-safe one-time initialisation
-    const char* e = getenv("RIPP_B200_PAIRING");  // "thread" selects the one-thread-per-pair kernels (A/B runs)
-    return !(e && strcmp(e, "thread") == 0);
-  }();
-  return v;
-}
-
-int ripp_pairing_batch_internal(ripp_ctx* ctx, int nseg, const void* const* g1, const void* const* g2, size_t n, void* out) {
-  if (ripp_use_l6()) return ripp_pairing_batch_l6(ctx, nseg, g1, g2, n, out, true);
-  if (nseg <= 0 || nseg > RIPP_MAX_BATCH) return fail(RIPP_ERR_ARG, "bad segment count");
-  CU(cudaSetDevice(ctx->device));
-  if (n == 0) {
-    Fq12 one[RIPP_MAX_BATCH];
-    for (int s = 0; s < nseg; s++) one[s] = Fq12::one();
-    CU(cudaMemcpyAsync(out, one, nseg * sizeof(Fq12), cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return RIPP_OK;
-  }
-  MillerBatch b;
-  b.nseg = nseg;
-  b.n = (uint32_t)n;
-  b.wps = (uint32_t)((n + 31) / 32);
-  for (int s = 0; s < nseg; s++) {
-    b.p[s] = (const G1Aff*)g1[s];
-    b.q[s] = (const G2Aff*)g2[s];
-  }
-  size_t nwarps = (size_t)b.wps * nseg;
-  void *bufA, *bufB;
-  OK(scratch(ctx, 2, nwarps * sizeof(Fq12), &bufA));
-  OK(scratch(ctx, 3, nwarps * sizeof(Fq12) / 4 + 4096, &bufB));
-  const int WPB = MILLER_BLOCK / 32;
-  uint32_t T = b.wps;
-  const uint32_t R = 8;
-  Fq12 *src = (Fq12*)bufA, *dst = (Fq12*)bufB;
-  {
-    TimeScope ts_(ctx, RIPP_T_MILLER);
-    k_miller_batch<MILLER_BLOCK><<<(unsigned)((nwarps + WPB - 1) / WPB), MILLER_BLOCK, 0, ctx->stream>>>(b, (Fq12*)bufA);
-    LAUNCHED(ctx);
-    while (T > R) {
-      uint32_t To = (T + R - 1) / R;
-      size_t tot = (size_t)nseg * To;
-      k_fq12_reduce_seg<<<(unsigned)((tot + 63) / 64), 64, 0, ctx->stream>>>(src, T, R, To, dst, tot);
-      LAUNCHED(ctx);
-      Fq12* t = src;
-      src = dst;
-      dst = t;
-      T = To;
-    }
-  }
-  TimeScope ts2_(ctx, RIPP_T_FINAL_EXP);
-  k_final_exp_seg<<<1, 32, 0, ctx->stream>>>(src, T, (Fq12*)out, nseg);
-  LAUNCHED(ctx);
-  return RIPP_OK;
-}
-
 extern "C" int ripp_pairing_ip_batch_dev(ripp_ctx* ctx, int nseg, const void* const* g1_aff_dev, const void* const* g2_aff_dev,
                                          size_t n, void* gt_out_dev) {
   if (!ctx || !g1_aff_dev || !g2_aff_dev || !gt_out_dev) return fail(RIPP_ERR_ARG, "null argument");
-  return ripp_pairing_batch_internal(ctx, nseg, g1_aff_dev, g2_aff_dev, n, gt_out_dev);
+  return ripp_pairing_batch_l6(ctx, nseg, g1_aff_dev, g2_aff_dev, n, gt_out_dev, true);
 }
 
 extern "C" int ripp_miller_partial_dev(ripp_ctx* ctx, const void* g1, const void* g2, size_t n, void* out) {
   if (!ctx || !out || (n && (!g1 || !g2))) return fail(RIPP_ERR_ARG, "null argument");
   CU(cudaSetDevice(ctx->device));
-  return miller_partial(ctx, (const G1Aff*)g1, (const G2Aff*)g2, n, (Fq12*)out);
+  const void* a1[1] = {g1};
+  const void* a2[1] = {g2};
+  return ripp_pairing_batch_l6(ctx, 1, a1, a2, n, out, false);
 }
 
 extern "C" int ripp_gt_combine_dev(ripp_ctx* ctx, const void* partials, size_t count, void* out) {
   if (!ctx || !out || !partials || count == 0) return fail(RIPP_ERR_ARG, "bad argument");
-  CU(cudaSetDevice(ctx->device));
-  void* tmp;
-  if (ripp_use_l6() && count <= 8) return ripp_final_exp_l6(ctx, partials, (uint32_t)count, out, 1);
-  OK(scratch(ctx, 3, sizeof(Fq12) + 256, &tmp));
-  TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
-  k_fq12_reduce<<<1, 32, 0, ctx->stream>>>((const Fq12*)partials, count, (int)count, (Fq12*)tmp);
-  LAUNCHED(ctx);
-  k_final_exp<<<1, 32, 0, ctx->stream>>>((const Fq12*)tmp, (Fq12*)out, 1);
-  LAUNCHED(ctx);
-  return RIPP_OK;
+  return ripp_final_exp_l6(ctx, partials, (uint32_t)count, out, 1);
 }
 
 // ---- batch primitives of the sharded (multi-GPU) provers: DESIGN.md §5 ---------------------------------------
@@ -836,18 +651,9 @@ extern "C" int ripp_seg_sum_dev(ripp_ctx* ctx, int type, const void* in, size_t 
 extern "C" int ripp_pairing_ip_dev(ripp_ctx* ctx, const void* g1, const void* g2, size_t n, void* out) {
   if (!ctx || !out || (n && (!g1 || !g2))) return fail(RIPP_ERR_ARG, "null argument");
   CU(cudaSetDevice(ctx->device));
-  void* part;
-  OK(scratch(ctx, 1, sizeof(Fq12) + 256, &part));
-  if (ripp_use_l6()) {
-    const void* a1[1] = {g1};
-    const void* a2[1] = {g2};
-    return ripp_pairing_batch_l6(ctx, 1, a1, a2, n, out, true);
-  }
-  OK(miller_partial(ctx, (const G1Aff*)g1, (const G2Aff*)g2, n, (Fq12*)part));
-  TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
-  k_final_exp<<<1, 32, 0, ctx->stream>>>((const Fq12*)part, (Fq12*)out, 1);
-  LAUNCHED(ctx);
-  return RIPP_OK;
+  const void* a1[1] = {g1};
+  const void* a2[1] = {g2};
+  return ripp_pairing_batch_l6(ctx, 1, a1, a2, n, out, true);
 }
 
 static int pairing_ip_host(ripp_ctx* ctx, const void* g1, size_t nl, const void* g2, size_t nr, void* gt_out, bool jac) {

@@ -524,7 +524,7 @@ static int kzg_checks(ripp_ctx* ctx, const VerifierSRS& vs, const G2Aff& ck_a, c
   const void* g1[4] = {G1s(0), G1s(4), G1s(5), G1s(3)};
   const void* g2[4] = {G2s(4), G2s(3), G2s(0), G2s(5)};
   char* res = D + 16384;
-  OK(ripp_pairing_batch_internal(ctx, two ? 4 : 2, g1, g2, 1, res));
+  OK(ripp_pairing_batch_l6(ctx, two ? 4 : 2, g1, g2, 1, res, true));
   Fq12 out[4];
   CU(cudaMemcpyAsync(out, res, (two ? 4 : 2) * 576, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));

@@ -87,14 +87,18 @@ def test_pairing_ip_bilinearity_at_scale(ctx, logn):
 
 
 def test_sharded_partials_combine(ctx):
-    """SURVEY.md §8e: slices -> Miller partials (no final exp) -> combine == whole product."""
+    """SURVEY.md §8e: slices -> Miller partials (no final exp) -> combine == whole product; 3 and 9 slices (more than
+    eight partials, one of them empty)."""
     n = 96
     a, b = synth.g1_points_dev(ctx, "sh-a", n), synth.g2_points_dev(ctx, "sh-b", n)
     whole = ctx.alloc(576)
     ctx.pairing_ip_dev(a, b, n, whole)
-    parts = ctx.alloc(576 * 3)
-    for r, (lo, hi) in enumerate(((0, 40), (40, 41), (41, 96))):
-        ctx.miller_partial_dev(a.ptr + 96 * lo, b.ptr + 192 * lo, hi - lo, parts.ptr + 576 * r)
-    comb = ctx.alloc(576)
-    ctx.gt_combine_dev(parts, 3, comb)
-    assert (comb.download(144) == whole.download(144)).all()
+    for cuts in ((0, 40, 41, 96), (0, 1, 10, 20, 20, 33, 50, 64, 80, 96)):
+        k = len(cuts) - 1
+        parts = ctx.alloc(576 * k)
+        for r in range(k):
+            lo, hi = cuts[r], cuts[r + 1]
+            ctx.miller_partial_dev(a.ptr + 96 * lo, b.ptr + 192 * lo, hi - lo, parts.ptr + 576 * r)
+        comb = ctx.alloc(576)
+        ctx.gt_combine_dev(parts, k, comb)
+        assert (comb.download(144) == whole.download(144)).all(), k

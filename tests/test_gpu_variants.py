@@ -1,10 +1,8 @@
 """The retained A/B code paths (environment switches read once per process) stay correct: a slice of the GPU suite
-re-run in a subprocess with the non-default kernels selected -- thread-per-pair Miller / final exponentiation
-(RIPP_B200_PAIRING=thread), the one-thread-per-element fold kernels with and without the endomorphisms
-(RIPP_B200_FOLD=endo / plain), three-warp teams (RIPP_B200_FOLD=w3), one thread per element for the scalings, and the
-six-lane shape everywhere (RIPP_B200_L18_WARPS=0), several pairs per
-eighteen-lane warp (RIPP_B200_L18_KP=4), and the fused folds of a round without / always with one team per
-endomorphism part (RIPP_B200_XP_MAX=0 / 100000)."""
+re-run in a subprocess with the non-default kernels selected -- the one-thread-per-element fold kernels with and without
+the endomorphisms (RIPP_B200_FOLD=endo / plain), three-warp teams (RIPP_B200_FOLD=w3), one thread per element for the
+scalings, the six-lane shape everywhere (RIPP_B200_L18_WARPS=0), and the fused folds of a round without / always with
+one team per endomorphism part (RIPP_B200_XP_MAX=0 / 100000)."""
 import os
 import subprocess
 import sys
@@ -16,14 +14,12 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.parametrize("env", [
-    {"RIPP_B200_PAIRING": "thread"},
     {"RIPP_B200_FOLD": "endo"},
     {"RIPP_B200_FOLD": "plain"},
     {"RIPP_B200_FOLD": "w3"},
     {"RIPP_B200_SCALE_PARTS_MAX": "0"},
     {"RIPP_B200_SCALE_PARTS_MAX": "0", "RIPP_B200_SCALE_XT_MAX": "100000"},
     {"RIPP_B200_L18_WARPS": "0"},
-    {"RIPP_B200_L18_KP": "4"},
     {"RIPP_B200_XP_MAX": "0"},
     {"RIPP_B200_XP_MAX": "100000"},
 ], ids=lambda e: ",".join("%s=%s" % kv for kv in e.items()))
