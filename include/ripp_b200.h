@@ -433,6 +433,27 @@ int ripp_tipa_verify(ripp_ctx* ctx, int kind, const void* vsrs, const uint8_t* c
 int ripp_tipp_verify_aggregate(ripp_ctx* ctx, const void* vsrs, const void* vk, size_t m, const void* public_inputs,
                                size_t n, const uint8_t* proof, size_t proof_len, int* accept);
 
+/* verify_aggregate_proof for `count` aggregates under one VerifierSRS and one VerifyingKey, one status per aggregate.
+ * status_out[k] is what ripp_tipp_verify_aggregate reports for aggregate k alone: */
+typedef enum ripp_agg_status {
+  RIPP_AGG_OK = 0,              /* accepted */
+  RIPP_AGG_MALFORMED = 1,       /* the bytes do not decode (length, non-canonical field element, off the curve) */
+  RIPP_AGG_NOT_IN_SUBGROUP = 2, /* a G1 / G2 / GT element outside the prime-order subgroup */
+  RIPP_AGG_REJECTED = 3         /* decodes, verify_aggregate_proof returns false */
+} ripp_agg_status;
+/* vsrs, vk, m: as ripp_tipp_verify_aggregate, shared by all aggregates.  n[k]: aggregate k's number of Groth16
+ * proofs (may differ between aggregates).  public_inputs: the rows of all aggregates back to back, sum_k n[k] rows of
+ * m Fr (host, Montgomery).  proofs: the AggregateProof bytes back to back, proof_lens[k] bytes for aggregate k,
+ * proofs_len in all.  *n_accepted counts the RIPP_AGG_OK.  A bad aggregate is data, not an error: the call fails
+ * with RIPP_ERR_ARG only for null pointers, n[k] == 0, m outside 1..1024, proof_lens that do not sum to proofs_len
+ * and count > 2^24; count == 0 returns RIPP_OK.  Deterministic (no randomness), and no status depends on the other
+ * members.  The kernel launches do not grow with count (subgroup checks, one G1 scaling, segmented sums, the GT folds,
+ * one Miller and one final-exponentiation launch for all aggregates: DESIGN.md §4); two host synchronisations. */
+int ripp_tipp_verify_aggregate_batch(ripp_ctx* ctx, const void* vsrs, const void* vk, size_t m, size_t count,
+                                     const size_t* n, const void* public_inputs, const uint8_t* proofs,
+                                     size_t proofs_len, const size_t* proof_lens, uint8_t* status_out,
+                                     size_t* n_accepted);
+
 /* SIPP::verify (sipp/src/lib.rs:109-180): inputs as ripp_sipp_prove, proof = its output. */
 int ripp_sipp_verify(ripp_ctx* ctx, const void* a_aff, const void* b_aff, const void* r, size_t n, const void* value_gt,
                      const uint8_t* proof, size_t proof_len, int* accept);

@@ -506,6 +506,24 @@ class Context:
                                                ctypes.c_size_t(n), _p(pb), ctypes.c_size_t(len(proof)), ctypes.byref(acc)))
         return bool(acc.value)
 
+    def tipp_verify_aggregate_batch(self, vsrs, vk, inputs_list, proofs):
+        """inputs_list[k]: (n_k, m, 8) uint32 Montgomery Fr of aggregate k; proofs[k]: its bytes.  -> np.uint8 array of
+        ripp_agg_status, one per aggregate."""
+        count = len(proofs)
+        m = inputs_list[0].shape[1] if count else 1
+        ns = np.array([x.shape[0] for x in inputs_list] or [0], dtype=np.uintp)
+        lens = np.array([len(p) for p in proofs] or [0], dtype=np.uintp)
+        inp = np.ascontiguousarray(np.concatenate([x.reshape(-1) for x in inputs_list]) if count else np.zeros(8, np.uint32),
+                                   dtype=np.uint32)
+        data = b"".join(bytes(p) for p in proofs)
+        pb = self._bytes(data)
+        st = np.zeros(max(count, 1), dtype=np.uint8)
+        acc = ctypes.c_size_t()
+        check(lib().ripp_tipp_verify_aggregate_batch(self.handle, _p(vsrs), _p(vk), ctypes.c_size_t(m), ctypes.c_size_t(count),
+                                                     _p(ns), _p(inp), _p(pb), ctypes.c_size_t(len(data)), _p(lens),
+                                                     _p(st), ctypes.byref(acc)))
+        return st[:count]
+
     def sipp_verify(self, a, b, r, value, proof):
         acc = ctypes.c_int(0)
         pb = self._bytes(proof)

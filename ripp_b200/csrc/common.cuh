@@ -17,7 +17,7 @@ using namespace ripp;
 // ------------------------------------------------------------------------------------------------
 std::string& ripp_err_slot();
 
-#define RIPP_SCRATCH_SLOTS 38
+#define RIPP_SCRATCH_SLOTS 41
 #define RIPP_MAX_BATCH 8
 #define RIPP_MAX_CHILD 8
 // per-category device-time accounting (CUDA events on the context's stream; off by default)
@@ -124,8 +124,10 @@ int ripp_join(ripp_ctx* ctx, ripp_ctx* child);         // ctx's stream waits for
 int ripp_pairing_batch_l6(ripp_ctx* ctx, int nseg, const void* const* g1, const void* const* g2, size_t n, void* out,
                           bool with_final_exp);
 int ripp_final_exp_l6(ripp_ctx* ctx, const void* in, uint32_t T, void* out, int nseg);
-int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n, void* out);
-int ripp_gt_check_l6(ripp_ctx* ctx, const void* in, size_t n, uint32_t* bad_dev, uint32_t flag);
+int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n, void* out, int nseg = 1);
+int ripp_gt_check_l6(ripp_ctx* ctx, const void* in, size_t n, uint32_t* bad_dev, uint32_t flag, const uint32_t* owner_dev = nullptr);
+// the aggregate verifier's pairing equations (verify_batch.cuh): p, q are 3 x n pairs, tgt n targets, ok n verdicts
+int ripp_pairing_checks_l6(ripp_ctx* ctx, const void* p, const void* q, size_t n, void* miller, const void* tgt, uint8_t* ok);
 // comm.cu: all-gather of one `bytes`-sized blob per rank on ctx's stream (recv = world * bytes, rank order); world == 1 copies
 int ripp_all_gather_internal(ripp_ctx* ctx, const void* send_dev, size_t bytes, void* recv_dev);
 void ripp_comm_release(ripp_ctx* ctx);

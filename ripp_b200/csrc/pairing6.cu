@@ -144,8 +144,9 @@ __global__ void __launch_bounds__(64) k_final_exp6(const Fq12* __restrict__ in, 
 // The Groth16 check of one proof per group: final_exponentiation(in[t]) == e(alpha, beta) (`ab`, 576 B), compared on
 // canonical Fq values (from_mont of any 384-bit value is the fully reduced product).  out[t] = 1 / 0, or with `pre`
 // (decode statuses of the serialized entry) pre[t] when non-zero, else RIPP_GROTH16_OK / RIPP_GROTH16_REJECTED.
-__global__ void __launch_bounds__(64) k_groth16_check6(const Fq12* __restrict__ in, const Fq12* __restrict__ ab, uint32_t n,
-                                                       const uint8_t* pre, uint8_t* out) {  // pre may alias out
+// ab_stride 1: one target per item, ab[t] (the pairing equations of the aggregate verifier, ripp_pairing_checks_l6).
+__global__ void __launch_bounds__(64) k_groth16_check6(const Fq12* __restrict__ in, const Fq12* __restrict__ ab, uint32_t ab_stride,
+                                                       uint32_t n, const uint8_t* pre, uint8_t* out) {  // pre may alias out
   extern __shared__ __align__(16) uint32_t smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = lane / 6;
@@ -155,7 +156,7 @@ __global__ void __launch_bounds__(64) k_groth16_check6(const Fq12* __restrict__ 
   st2(freg(c, 0) + c.k * FQ2W, reinterpret_cast<const Fq2*>(in + (live ? t : 0))[tower_slot(c.k)]);
   __syncwarp();
   final_exp(c);
-  const Fq2 f = ld2(freg(c, 0) + c.k * FQ2W), e = reinterpret_cast<const Fq2*>(ab)[tower_slot(c.k)];
+  const Fq2 f = ld2(freg(c, 0) + c.k * FQ2W), e = reinterpret_cast<const Fq2*>(ab + (live ? t : 0) * ab_stride)[tower_slot(c.k)];
   const bool eq = f.c0.from_mont() == e.c0.from_mont() && f.c1.from_mont() == e.c1.from_mont();
   const uint32_t all = __ballot_sync(0xffffffffu, eq);
   if (live && c.k == 0) {
@@ -319,11 +320,11 @@ static size_t l18_max_warps() {
 // GT membership of untrusted Fq12 values (what ark-serialize's Valid::check establishes for PairingOutput when the
 // reference deserialises a proof): f is in the cyclotomic subgroup, f^(p^4) f == f^(p^2), and f^p == f^x
 // (Scott, ePrint 2021/1130; oracle: gt_in_subgroup_fast, checked there against f^r == 1).  One group per element;
-// a failing element ORs `flag` into *bad.
+// a failing element ORs `flag` into bad[0], or into bad[owner[i]] when owner is given (one word per aggregate).
 constexpr int GC_NREG = 3;
 constexpr int GC_GROUP_WORDS = group_words(GC_NREG, 0) + BUS_TOTAL;
 __global__ void __launch_bounds__(32) k_gt_check18(const Fq12* __restrict__ in, uint32_t n, uint32_t* __restrict__ bad,
-                                                   uint32_t flag) {
+                                                   uint32_t flag, const uint32_t* __restrict__ owner) {
   extern __shared__ __align__(16) uint32_t smem[];
   Ctx3 c = ctx18(smem, group_words(GC_NREG, 0));
   const Fq2* src = reinterpret_cast<const Fq2*>(in + blockIdx.x);
@@ -337,11 +338,11 @@ __global__ void __launch_bounds__(32) k_gt_check18(const Fq12* __restrict__ in, 
   exp_by_x(c, 2, 0);  // cyclotomic squarings: meaningful only when the first test passed, and only then consulted
   frob(c, 1, 0, 1);
   ne = ne || !(ld2(freg(c, 2) + c.k * FQ2W) == ld2(freg(c, 1) + c.k * FQ2W));
-  if (ne) atomicOr(bad, flag);
+  if (ne) atomicOr(bad + (owner ? owner[blockIdx.x] : 0), flag);
 }
-int ripp_gt_check_l6(ripp_ctx* ctx, const void* in, size_t n, uint32_t* bad_dev, uint32_t flag) {
+int ripp_gt_check_l6(ripp_ctx* ctx, const void* in, size_t n, uint32_t* bad_dev, uint32_t flag, const uint32_t* owner_dev) {
   if (n == 0) return RIPP_OK;
-  k_gt_check18<<<(unsigned)n, 32, GC_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)in, (uint32_t)n, bad_dev, flag);
+  k_gt_check18<<<(unsigned)n, 32, GC_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)in, (uint32_t)n, bad_dev, flag, owner_dev);
   LAUNCHED(ctx);
   return RIPP_OK;
 }
@@ -364,8 +365,8 @@ static int reduce6(ripp_ctx* ctx, uint32_t nseg, uint32_t stop, Fq12** src, Fq12
   return RIPP_OK;
 }
 
-// out = prod_i in[i]^sc[i]  (device memory; in: n Fq12, sc: n Fr Montgomery)
-int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n, void* out) {
+// out[s] = prod_i in[s * n + i]^sc[s * n + i], s < nseg  (device memory; in: nseg x n Fq12, sc: nseg x n Fr Montgomery)
+int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n, void* out, int nseg) {
   CU(cudaSetDevice(ctx->device));
   if (n == 0) {
     Fq12 one = Fq12::one();
@@ -373,20 +374,21 @@ int ripp_gt_multiexp_l6(ripp_ctx* ctx, const void* in, const void* sc, size_t n,
     CU(cudaStreamSynchronize(ctx->stream));
     return RIPP_OK;
   }
+  const size_t total = (size_t)nseg * n;
   void *bufA, *bufB;
-  OK(scratch(ctx, 17, n * sizeof(Fq12) + 4096, &bufA));
-  OK(scratch(ctx, 18, n * sizeof(Fq12) / 4 + 8192, &bufB));
+  OK(scratch(ctx, 17, total * sizeof(Fq12) + 4096, &bufA));
+  OK(scratch(ctx, 18, total * sizeof(Fq12) / 4 + 8192, &bufB));
   TimeScope ts_(ctx, RIPP_T_OTHER);
-  if (n <= l18_max_warps())
-    k_gt_pow18<<<(unsigned)n, 32, GP18_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)in, (const Fr*)sc, (uint32_t)n,
-                                                                     n == 1 ? (Fq12*)out : (Fq12*)bufA);
+  if (total <= l18_max_warps())
+    k_gt_pow18<<<(unsigned)total, 32, GP18_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)in, (const Fr*)sc, (uint32_t)total,
+                                                                         n == 1 ? (Fq12*)out : (Fq12*)bufA);
   else
-    k_gt_pow6<<<(unsigned)((n + 4) / 5), 32, 6 * GP_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)in, (const Fr*)sc, (uint32_t)n,
-                                                                                    n == 1 ? (Fq12*)out : (Fq12*)bufA);
+    k_gt_pow6<<<(unsigned)((total + 4) / 5), 32, 6 * GP_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)in, (const Fr*)sc,
+                                                                                        (uint32_t)total, n == 1 ? (Fq12*)out : (Fq12*)bufA);
   LAUNCHED(ctx);
   Fq12* src = (Fq12*)bufA;
   uint32_t T = (uint32_t)n;
-  return reduce6(ctx, 1, 1, &src, (Fq12*)bufB, &T, (Fq12*)out);
+  return reduce6(ctx, (uint32_t)nseg, 1, &src, (Fq12*)bufB, &T, (Fq12*)out);
 }
 
 // Pairs per six-lane group for nseg segments of pairs_per_seg pairs (the pairs of a group share the accumulator's
@@ -549,8 +551,32 @@ int ripp_groth16_pairings_l6(ripp_ctx* ctx, const void* a, const void* b, const 
     LAUNCHED(ctx);
   }
   TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
-  k_groth16_check6<<<(unsigned)((n + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)miller, (const Fq12*)ab,
+  k_groth16_check6<<<(unsigned)((n + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)miller, (const Fq12*)ab, 0,
                                                                                             (uint32_t)n, pre, out);
+  LAUNCHED(ctx);
+  return RIPP_OK;
+}
+
+// n pairing equations prod_{j < 3} e(p[j * n + t], q[j * n + t]) == tgt[t], one six-lane group per equation (the three
+// pairs share one accumulator; a pair with an identity is left out); ok[t] = 1 / 0.  `miller` holds n Fq12.
+int ripp_pairing_checks_l6(ripp_ctx* ctx, const void* p, const void* q, size_t n, void* miller, const void* tgt, uint8_t* ok) {
+  Miller6Batch mb;
+  memset(&mb, 0, sizeof(mb));
+  for (int j = 0; j < 3; j++) {
+    mb.p[j] = (const G1Aff*)p + j * n;
+    mb.q[j] = (const G2Aff*)q + j * n;
+  }
+  mb.n = (uint32_t)n;
+  mb.nseg = 1;
+  mb.wps = (uint32_t)((n + 4) / 5);
+  {
+    TimeScope ts_(ctx, RIPP_T_MILLER);
+    k_miller6<M6_WARPS, 3, true><<<(mb.wps + M6_WARPS - 1) / M6_WARPS, 32 * M6_WARPS, m6_smem_bytes(3), ctx->stream>>>(mb, (Fq12*)miller);
+    LAUNCHED(ctx);
+  }
+  TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
+  k_groth16_check6<<<(unsigned)((n + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>((const Fq12*)miller, (const Fq12*)tgt, 1,
+                                                                                            (uint32_t)n, nullptr, ok);
   LAUNCHED(ctx);
   return RIPP_OK;
 }
@@ -608,7 +634,7 @@ int ripp_groth16_rlc_pairings_l6(ripp_ctx* ctx, const void* ra, const void* b, c
     OK(m6_products(ctx, mb, kp, (uint32_t)nseg, 1, &src, dst, &T));
   }
   TimeScope ts_(ctx, RIPP_T_FINAL_EXP);
-  k_groth16_check6<<<(unsigned)((nseg + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>(src, (const Fq12*)ab, (uint32_t)nseg,
+  k_groth16_check6<<<(unsigned)((nseg + 9) / 10), 64, 2 * 6 * FE_GROUP_WORDS * 4, ctx->stream>>>(src, (const Fq12*)ab, 0, (uint32_t)nseg,
                                                                                                nullptr, ok);
   LAUNCHED(ctx);
   return RIPP_OK;

@@ -173,12 +173,13 @@ static Val val_fr(const Fr& f) {
 // PairingOutput::check).  G1 / G2: serde::in_prime_subgroup (serde.cuh, shared with the point decoders of
 // deserialize.cu); GT: k_gt_check6 (pairing6.cu).
 // ------------------------------------------------------------------------------------------------
+// a failing point ORs `flag` into bad[0], or into bad[owner[i]] when owner is given (one word per aggregate)
 template <class F>
 __global__ void __launch_bounds__(64) k_subgroup_check(const Aff<F>* __restrict__ pts, uint32_t n, uint32_t* __restrict__ bad,
-                                                       uint32_t flag) {
+                                                       uint32_t flag, const uint32_t* __restrict__ owner) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  if (!serde::in_prime_subgroup(pts[i])) atomicOr(bad, flag);
+  if (!serde::in_prime_subgroup(pts[i])) atomicOr(bad + (owner ? owner[i] : 0), flag);
 }
 
 // *bad_mask: bit 0 = a G1 element, bit 1 = a G2 element, bit 2 = a GT element outside its prime-order subgroup
@@ -203,12 +204,12 @@ static int validate_subgroups(ripp_ctx* ctx, std::initializer_list<Reader*> read
   CU(cudaMemsetAsync(flag, 0, 4, st));
   if (!g1.empty()) {
     CU(cudaMemcpyAsync(D, g1.data(), g1.size() * 96, cudaMemcpyHostToDevice, st));
-    k_subgroup_check<Fq><<<(unsigned)((g1.size() + 63) / 64), 64, 0, st>>>((const G1Aff*)D, (uint32_t)g1.size(), flag, 1u);
+    k_subgroup_check<Fq><<<(unsigned)((g1.size() + 63) / 64), 64, 0, st>>>((const G1Aff*)D, (uint32_t)g1.size(), flag, 1u, nullptr);
     LAUNCHED(ctx);
   }
   if (!g2.empty()) {
     CU(cudaMemcpyAsync(D + o_g2, g2.data(), g2.size() * 192, cudaMemcpyHostToDevice, st));
-    k_subgroup_check<Fq2><<<(unsigned)((g2.size() + 63) / 64), 64, 0, st>>>((const G2Aff*)(D + o_g2), (uint32_t)g2.size(), flag, 2u);
+    k_subgroup_check<Fq2><<<(unsigned)((g2.size() + 63) / 64), 64, 0, st>>>((const G2Aff*)(D + o_g2), (uint32_t)g2.size(), flag, 2u, nullptr);
     LAUNCHED(ctx);
   }
   if (!gt.empty()) {
@@ -298,22 +299,29 @@ static int combine(ripp_ctx* ctx, int t, const std::vector<Val>& elems, const st
   return RIPP_OK;
 }
 
-// base commitments of gipa.rs:355-357 after all rounds: com + sum_k (c_k com_1[k] + c_k^-1 com_2[k]), per component
+// the 2k + 1 terms of component j's base commitment (gipa.rs:355-357 after all rounds): com + sum_k (c_k com_1[k] +
+// c_k^-1 com_2[k])
+static void fold_terms(const GipaProofP& pf, const std::vector<Fr>& c_round, const std::vector<Fr>& cinv_round, const Val& com,
+                       int j, std::vector<Val>* el, std::vector<Fr>* sc) {
+  size_t k = pf.steps.size();
+  el->assign(1, com);
+  sc->assign(1, Fr::one());
+  for (size_t rd = 0; rd < k; rd++) {
+    const std::vector<Val>& st = pf.steps[k - 1 - rd];
+    el->push_back(st[j]);
+    sc->push_back(c_round[rd]);
+    el->push_back(st[3 + j]);
+    sc->push_back(cinv_round[rd]);
+  }
+}
+
+// base commitments of gipa.rs:355-357 after all rounds, per component
 static int fold_commitments(ripp_ctx* ctx, const GipaProofP& pf, const std::vector<Fr>& c_round,
                             const std::vector<Fr>& cinv_round, const Val com[3], Val base[3]) {
-  size_t k = pf.steps.size();
   for (int j = 0; j < 3; j++) {
     std::vector<Val> el;
     std::vector<Fr> sc;
-    el.push_back(com[j]);
-    sc.push_back(Fr::one());
-    for (size_t rd = 0; rd < k; rd++) {
-      const std::vector<Val>& st = pf.steps[k - 1 - rd];
-      el.push_back(st[j]);
-      sc.push_back(c_round[rd]);
-      el.push_back(st[3 + j]);
-      sc.push_back(cinv_round[rd]);
-    }
+    fold_terms(pf, c_round, cinv_round, com[j], j, &el, &sc);
     OK(combine(ctx, com[j].t, el, sc, &base[j]));
   }
   return RIPP_OK;
@@ -631,6 +639,37 @@ __global__ void __launch_bounds__(128) k_input_column_ip(const Fr* __restrict__ 
   if (threadIdx.x == 0) out[j] = part[0];
 }
 
+// AggregateProof { com_a, com_b, com_c, ip_ab, agg_c, tipa_proof_ab, tipa_proof_c } (:58-66)
+struct AggregateProofP {
+  Val com_a, com_b, com_c, ip_ab, agg_c;
+  TipaProofP pab, pc;
+};
+static bool parse_aggregate_proof(Reader& rp, AggregateProofP* a) {
+  GipaSpec sp_ab, sp_c;
+  gipa_spec(RIPP_GIPA_PAIRING, &sp_ab);
+  gipa_spec(RIPP_GIPA_MULTIEXP_SSM, &sp_c);
+  return get_val(rp, VT_GT, &a->com_a) && get_val(rp, VT_GT, &a->com_b) && get_val(rp, VT_GT, &a->com_c) &&
+         get_val(rp, VT_GT, &a->ip_ab) && get_val(rp, VT_G1, &a->agg_c) && parse_tipa_proof(rp, sp_ab, &a->pab) &&
+         parse_tipa_proof(rp, sp_c, &a->pc) && rp.done();
+}
+// :174-186 r
+static Fr aggregate_challenge(const Val& com_a, const Val& com_b, const Val& com_c) {
+  Bytes parts;
+  put_val(parts, com_a);
+  put_val(parts, com_b);
+  put_val(parts, com_c);
+  return challenge_from_random_bytes(parts);
+}
+// :210-212 r_sum = (r^n - 1) / (r - 1)
+static Fr aggregate_r_sum(const Fr& r, size_t n) {
+  Fr rn = Fr::one(), b = r;
+  for (size_t e = n; e; e >>= 1) {
+    if (e & 1) rn = rn * b;
+    b = b * b;
+  }
+  return (rn - Fr::one()) * (r - Fr::one()).inv();
+}
+
 extern "C" int ripp_tipp_verify_aggregate(ripp_ctx* ctx, const void* vsrs, const void* vk, size_t m,
                                           const void* public_inputs, size_t n, const uint8_t* proof, size_t proof_len,
                                           int* accept) {
@@ -643,23 +682,15 @@ extern "C" int ripp_tipp_verify_aggregate(ripp_ctx* ctx, const void* vsrs, const
   GipaSpec sp_ab, sp_c;
   gipa_spec(RIPP_GIPA_PAIRING, &sp_ab);
   gipa_spec(RIPP_GIPA_MULTIEXP_SSM, &sp_c);
-  // AggregateProof { com_a, com_b, com_c, ip_ab, agg_c, tipa_proof_ab, tipa_proof_c } (:58-66)
   Reader rp(proof, proof_len);
-  Val com_a, com_b, com_c, ip_ab, agg_c;
-  TipaProofP pab, pc;
-  if (!get_val(rp, VT_GT, &com_a) || !get_val(rp, VT_GT, &com_b) || !get_val(rp, VT_GT, &com_c) ||
-      !get_val(rp, VT_GT, &ip_ab) || !get_val(rp, VT_G1, &agg_c) || !parse_tipa_proof(rp, sp_ab, &pab) ||
-      !parse_tipa_proof(rp, sp_c, &pc) || !rp.done())
-    return fail(RIPP_ERR_ARG, "malformed AggregateProof bytes");
+  AggregateProofP ap;
+  if (!parse_aggregate_proof(rp, &ap)) return fail(RIPP_ERR_ARG, "malformed AggregateProof bytes");
+  const Val &com_a = ap.com_a, &com_b = ap.com_b, &com_c = ap.com_c, &ip_ab = ap.ip_ab, &agg_c = ap.agg_c;
+  const TipaProofP &pab = ap.pab, &pc = ap.pc;
   uint32_t bad = 0;
   OK(validate_subgroups(ctx, {&rp}, &bad));
   if (bad) return subgroup_error(bad);
-  // :174-186 r
-  Bytes parts;
-  put_val(parts, com_a);
-  put_val(parts, com_b);
-  put_val(parts, com_c);
-  Fr r = challenge_from_random_bytes(parts);
+  Fr r = aggregate_challenge(com_a, com_b, com_c);
   // :189-206 the two TIPA proofs
   bool ok_ab = false, ok_c = false;
   {
@@ -670,13 +701,7 @@ extern "C" int ripp_tipp_verify_aggregate(ripp_ctx* ctx, const void* vsrs, const
     Val cm[3] = {com_c, val_fr(Fr::zero()), agg_c};
     OK(tipa_verify_parsed(ctx, sp_c, vs, cm, r, pc.gipa, pc.ck_a, nullptr, pc.pi_a, nullptr, &ok_c));
   }
-  // :210-212 r_sum = (r^n - 1) / (r - 1)
-  Fr rn = Fr::one(), b = r;
-  for (size_t e = n; e; e >>= 1) {
-    if (e & 1) rn = rn * b;
-    b = b * b;
-  }
-  Fr r_sum = (rn - Fr::one()) * (r - Fr::one()).inv();
+  Fr r_sum = aggregate_r_sum(r, n);
   // vk: alpha_g1 | beta_g2 | gamma_g2 | delta_g2 | gamma_abc_g1[m + 1]
   const char* vkp = (const char*)vk;
   const size_t o_alpha = 0, o_beta = 96, o_gamma = 288, o_delta = 480, o_abc = 672;

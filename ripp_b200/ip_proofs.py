@@ -182,6 +182,29 @@ def verify_aggregate_proof(v_srs, vk, public_inputs, proof, ctx=None):
     return ctx.tipp_verify_aggregate(vsrs_enc(v_srs), np.ascontiguousarray(vk_enc(vk)), inp, proof)
 
 
+# ripp_agg_status: what verify_aggregate_proof reports for one aggregate
+AGG_OK, AGG_MALFORMED, AGG_NOT_IN_SUBGROUP, AGG_REJECTED = range(4)
+AGG_STATUS_NAMES = ("OK", "MALFORMED", "NOT_IN_SUBGROUP", "REJECTED")
+
+
+def verify_aggregate_proofs(v_srs, vk, public_inputs_list, proofs, ctx=None):
+    """verify_aggregate_proof for many aggregates under one v_srs and one vk, their checks sharing one set of GPU
+    launches.  public_inputs_list[k]: aggregate k's public inputs (one list of Fr per Groth16 proof); proofs[k]: its
+    bytes.  -> np.ndarray of uint8 statuses (AGG_OK .. AGG_REJECTED above), one per aggregate: AGG_OK where
+    verify_aggregate_proof accepts, AGG_REJECTED where it returns false, AGG_MALFORMED / AGG_NOT_IN_SUBGROUP where the
+    bytes do not deserialize."""
+    ctx = ctx or default_context()
+    if len(public_inputs_list) != len(proofs):
+        raise ValueError("%d lists of public inputs for %d aggregates" % (len(public_inputs_list), len(proofs)))
+    m = len(vk["gamma_abc_g1"]) - 1
+    inputs = []
+    for k, rows in enumerate(public_inputs_list):
+        if not rows or any(len(row) != m for row in rows):
+            raise ValueError("aggregate %d: need at least one row of %d public inputs" % (k, m))  # :214
+        inputs.append(np.stack([codec.fr_vec_enc(row) for row in rows]).reshape(len(rows), m, 8))
+    return ctx.tipp_verify_aggregate_batch(vsrs_enc(v_srs), np.ascontiguousarray(vk_enc(vk)), inputs, proofs)
+
+
 def structured_generators_scalar_power(num, g, s, group, ctx=None):
     """tipa/mod.rs:372-391: [g * s^i for i < num] (g: affine tuple or None = the generator; group 1 / 2).  -> list of points"""
     ctx = ctx or default_context()

@@ -311,6 +311,43 @@ pub fn verify_aggregate_proof(v_srs: &VerifierSRS<Bls12_381>, vk: &VerifyingKey<
     Ok(accept == 1)
 }
 
+/// `verify_aggregate_proof` for many aggregates under one `VerifierSRS` and one `VerifyingKey`, as a node that receives
+/// aggregates from many provers runs it: `aggregates[k]` = (aggregate k's public inputs, one row per Groth16 proof;
+/// its `AggregateProof` bytes).  One `ripp_agg_status` per aggregate, exactly what `verify_aggregate_proof` reports for
+/// it alone: 0 = accepted, 1 = the bytes do not decode, 2 = an element outside the prime-order subgroup, 3 = rejected.
+/// The checks of all aggregates share one set of GPU launches.
+pub fn verify_aggregate_proofs(v_srs: &VerifierSRS<Bls12_381>, vk: &VerifyingKey<Bls12_381>,
+                               aggregates: &[(&[Vec<Fr>], &[u8])]) -> Result<Vec<u8>, Error> {
+    let mut vsrs = Vec::with_capacity(72);
+    vsrs.extend(pack::pack_g1_aff(&[v_srs.g.into_affine()]));
+    vsrs.extend(pack::pack_g2_aff(&[v_srs.h.into_affine()]));
+    vsrs.extend(pack::pack_g1_aff(&[v_srs.g_beta.into_affine()]));
+    vsrs.extend(pack::pack_g2_aff(&[v_srs.h_alpha.into_affine()]));
+    let mut vkw = Vec::new();
+    vkw.extend(pack::pack_g1_aff(&[vk.alpha_g1]));
+    vkw.extend(pack::pack_g2_aff(&[vk.beta_g2, vk.gamma_g2, vk.delta_g2]));
+    vkw.extend(pack::pack_g1_aff(&vk.gamma_abc_g1));
+    let m = vk.gamma_abc_g1.len() - 1;
+    let ns: Vec<usize> = aggregates.iter().map(|(rows, _)| rows.len()).collect();
+    let lens: Vec<usize> = aggregates.iter().map(|(_, b)| b.len()).collect();
+    let inputs: Vec<u64> = aggregates.iter().flat_map(|(rows, _)| rows.iter().flat_map(|row| {
+        assert_eq!(row.len(), m); // groth16_aggregation.rs:214
+        pack::pack_fr(row)
+    })).collect();
+    let bytes: Vec<u8> = aggregates.iter().flat_map(|(_, b)| b.iter().copied()).collect();
+    let mut status = vec![0u8; aggregates.len()];
+    let mut accepted = 0usize;
+    let c = ctx();
+    let st = unsafe {
+        sys::ripp_tipp_verify_aggregate_batch(c.raw(), vsrs.as_ptr() as *const c_void, vkw.as_ptr() as *const c_void, m,
+                                              aggregates.len(), ns.as_ptr(), inputs.as_ptr() as *const c_void, bytes.as_ptr(),
+                                              bytes.len(), lens.as_ptr(), status.as_mut_ptr(), &mut accepted)
+    };
+    drop(c);
+    check(st, aggregates.len(), aggregates.len())?;
+    Ok(status)
+}
+
 /// `GIPA::prove` for the pairing instantiation (`gipa.rs:108-133`): the statement (com_a, com_b, t) is checked on the
 /// device before proving; a false statement returns `InnerProductArgumentError::InnerProductInvalid`.
 pub fn gipa_prove_checked_ab(a: &DeviceVec<G1Affine>, b: &DeviceVec<G2Affine>, ck_a: &DeviceVec<G2Affine>,
