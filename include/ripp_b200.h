@@ -112,6 +112,14 @@ int ripp_msm_g2(ripp_ctx* ctx, const void* g2_jac, size_t n_left, const void* fr
  * KZG opening MSM of tipa/mod.rs:333-334. */
 int ripp_msm_g1_dev(ripp_ctx* ctx, const void* g1_aff_dev, const void* fr_dev, size_t n, void* g1_aff_out_dev);
 int ripp_msm_g2_dev(ripp_ctx* ctx, const void* g2_aff_dev, const void* fr_dev, size_t n, void* g2_aff_out_dev);
+/* nseg MSMs of n terms in one segmented pass: out[s] = sum_i fr[s*n + i] * bases[s*bases_stride + i], s < nseg (device
+ * memory, affine bases, Montgomery scalars, nseg affine results).  bases_stride = 0: one base vector shared by all
+ * segments (KZG openings over one SRS).  nseg at most 2^16 and nseg * n at most 2^24 (RIPP_ERR_ARG): a short segment
+ * needs ~65 KB of workspace (G2), a long one about what one MSM over all nseg * n points needs. */
+int ripp_msm_g1_batch_dev(ripp_ctx* ctx, const void* g1_aff_dev, size_t bases_stride, const void* fr_dev, size_t n, size_t nseg,
+                          void* g1_aff_out_dev);
+int ripp_msm_g2_batch_dev(ripp_ctx* ctx, const void* g2_aff_dev, size_t bases_stride, const void* fr_dev, size_t n, size_t nseg,
+                          void* g2_aff_out_dev);
 /* ScalarInnerProduct::inner_product (lib.rs:149-166): sum_i a[i] * b[i] in Fr. */
 int ripp_scalar_ip(ripp_ctx* ctx, const void* fr_a, size_t n_left, const void* fr_b, size_t n_right, void* fr_out);
 int ripp_scalar_ip_dev(ripp_ctx* ctx, const void* fr_a_dev, const void* fr_b_dev, size_t n, void* fr_out_dev);
@@ -236,6 +244,23 @@ int ripp_tipp_aggregate_dev(ripp_ctx* ctx, const void* srs_g1_dev, const void* s
 int ripp_tipp_aggregate(ripp_ctx* ctx, const void* srs_g1_dev, const void* srs_g2_dev, const void* a_host,
                         const void* b_host, const void* c_host, size_t n, uint8_t* proof_out, size_t proof_cap,
                         size_t* proof_len);
+
+/* aggregate_proofs for `count` independent batches of n proofs each, under one SRS (at least 2n - 1 powers, as
+ * ripp_tipp_aggregate_dev).  a, c: count x n G1 affine, b: count x n G2 affine, batch k at element k * n.  proofs_out
+ * receives count AggregateProofs back to back, each *proof_len bytes (the length depends on n only), and proof k is
+ * byte for byte what ripp_tipp_aggregate_dev returns for batch k alone.  The GIPA rounds of all batches run in lock
+ * step: the number of launches and host synchronisations does not grow with count.
+ * n: a power of two (RIPP_ERR_NOT_POW2), at least 2 (RIPP_ERR_ARG); count == 0: RIPP_OK with *proof_len = 0;
+ * count * n at most 2^20 and count at most 2^16 (RIPP_ERR_ARG; the device workspace then stays below ~41 GB, kept on
+ * the context for the next call); proofs_cap < count * *proof_len: RIPP_ERR_ARG with *proof_len set.
+ * RIPP_ERR_INNER_PRODUCT names the batch whose :133-136 self-check failed. */
+int ripp_tipp_aggregate_batch_dev(ripp_ctx* ctx, const void* srs_g1_dev, const void* srs_g2_dev, size_t count, size_t n,
+                                  const void* a_dev, const void* b_dev, const void* c_dev, uint8_t* proofs_out,
+                                  size_t proofs_cap, size_t* proof_len);
+/* Same with the proofs in host memory (three packed arrays, one H2D copy each), as ripp_tipp_aggregate. */
+int ripp_tipp_aggregate_batch(ripp_ctx* ctx, const void* srs_g1_dev, const void* srs_g2_dev, size_t count, size_t n,
+                              const void* a_host, const void* b_host, const void* c_host, uint8_t* proofs_out,
+                              size_t proofs_cap, size_t* proof_len);
 
 /* ---- deserialisation: validated decoding of untrusted ark-serialize bytes ------------------------------------ */
 /* Points as ark-serialize 0.4 / ark-bls12-381 0.4 write them (big-endian coordinates, flags in the top three bits

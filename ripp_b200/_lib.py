@@ -207,6 +207,15 @@ class Context:
     def msm_g2_dev(self, bases_dev, fr_dev, n, out_dev):
         check(lib().ripp_msm_g2_dev(self.handle, _p(bases_dev), _p(fr_dev), ctypes.c_size_t(n), _p(out_dev)))
 
+    def msm_g1_batch_dev(self, bases_dev, bases_stride, fr_dev, n, nseg, out_dev):
+        """out[s] = sum_i fr[s*n + i] * bases[s*bases_stride + i], s < nseg (bases_stride 0: one shared base vector)."""
+        check(lib().ripp_msm_g1_batch_dev(self.handle, _p(bases_dev), ctypes.c_size_t(bases_stride), _p(fr_dev), ctypes.c_size_t(n),
+                                          ctypes.c_size_t(nseg), _p(out_dev)))
+
+    def msm_g2_batch_dev(self, bases_dev, bases_stride, fr_dev, n, nseg, out_dev):
+        check(lib().ripp_msm_g2_batch_dev(self.handle, _p(bases_dev), ctypes.c_size_t(bases_stride), _p(fr_dev), ctypes.c_size_t(n),
+                                          ctypes.c_size_t(nseg), _p(out_dev)))
+
     def scalar_ip(self, a, b):
         out = np.empty(8, dtype=np.uint32)
         check(lib().ripp_scalar_ip(self.handle, _p(a), ctypes.c_size_t(len(a)), _p(b), ctypes.c_size_t(len(b)), _p(out)))
@@ -365,6 +374,27 @@ class Context:
         check(lib().ripp_tipp_aggregate(self.handle, _p(srs_g1), _p(srs_g2), _p(a_host), _p(b_host), _p(c_host),
                                         ctypes.c_size_t(n), _p(proof), ctypes.c_size_t(cap), ctypes.byref(plen)))
         return proof[: plen.value].tobytes()
+
+    def _aggregate_batch(self, fn, srs_g1, srs_g2, count, n, a, b, c):
+        k = max(n.bit_length() - 1, 0)
+        per = 8 * 600 + 2 * (64 + k * 6 * 600 + 8 * 600)
+        proofs = np.empty(max(count * per, 1), dtype=np.uint8)
+        plen = ctypes.c_size_t()
+        check(fn(self.handle, _p(srs_g1), _p(srs_g2), ctypes.c_size_t(count), ctypes.c_size_t(n), _p(a), _p(b), _p(c), _p(proofs),
+                 ctypes.c_size_t(proofs.size), ctypes.byref(plen)))
+        ln = plen.value
+        return [proofs[i * ln:(i + 1) * ln].tobytes() for i in range(count)]
+
+    def tipp_aggregate_batch_dev(self, srs_g1, srs_g2, a, b, c, count, n):
+        """aggregate_proofs for `count` batches of n proofs (device: a, c count*n G1, b count*n G2, batch k at element k*n)
+        in one call, their GIPA rounds in lock step.  -> list of `count` AggregateProof bytes."""
+        return self._aggregate_batch(lib().ripp_tipp_aggregate_batch_dev, srs_g1, srs_g2, count, n, a, b, c)
+
+    def tipp_aggregate_batch(self, srs_g1, srs_g2, a_host, b_host, c_host, count):
+        """tipp_aggregate_batch_dev with the proofs in host memory: a_host, c_host (count*n, 24), b_host (count*n, 48) uint32."""
+        n = len(a_host) // count if count else 2
+        return self._aggregate_batch(lib().ripp_tipp_aggregate_batch, srs_g1, srs_g2, count, n, np.ascontiguousarray(a_host),
+                                     np.ascontiguousarray(b_host), np.ascontiguousarray(c_host))
 
     # ---- deserialisation (csrc/deserialize.cu) ------------------------------------------------------
     def g1_deserialize_dev(self, bytes_dev, n, stride, compressed, out_dev, status_dev):

@@ -17,7 +17,7 @@ using namespace ripp;
 // ------------------------------------------------------------------------------------------------
 std::string& ripp_err_slot();
 
-#define RIPP_SCRATCH_SLOTS 41
+#define RIPP_SCRATCH_SLOTS 48
 #define RIPP_MAX_BATCH 8
 #define RIPP_MAX_CHILD 8
 // per-category device-time accounting (CUDA events on the context's stream; off by default)
@@ -56,6 +56,9 @@ struct ripp_ctx {
   // work nothing waits for (the aggregation's side products): the pairing engine packs it into the fewest CTAs so that
   // the lone warps of the critical path keep sub-partitions to themselves
   int background;
+  // page-locked staging grown on demand: the per-round results of the batch prover (aggregate_batch.cuh)
+  uint8_t* pinned_big;
+  size_t pinned_big_bytes;
 };
 #define RIPP_PINNED_BYTES 16384
 
@@ -137,6 +140,27 @@ int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, 
                         void* const* out, int* fused, const void* const* pre = nullptr);
 int ripp_fold_pre_internal(ripp_ctx* ctx, const int* types, const void* const* hi, size_t n, void* const* pre);
 size_t ripp_fold_pre_max_n();
+// the folds of the lock-step batch prover (aggregate_batch.cuh): section s (0 G1, 1 G2, 2 Fr) has ngroups[s] groups of K
+// jobs; job (g, k) folds base[s][g] + k stride[s][g] (hi at + n elements) with scalar record sc[s][g][k] (device: EndoBits
+// for G1 / G2, Fr for Fr).  bpj / first_block / blocks are filled by ripp_fold_table_internal.
+struct FoldTable {
+  char* base[3][3];
+  size_t stride[3][3];
+  const void* sc[3][3];
+  int ngroups[3];
+  uint32_t K, n;
+  uint32_t bpj[3], first_block[3], blocks[3];
+};
+int ripp_fold_table_internal(ripp_ctx* ctx, FoldTable t);
+namespace ripp {
+struct EndoBits;
+}
+void ripp_endo_bits(int group, const void* fr_mont_host, EndoBits* out);  // group 1 / 2: the fold recoding of a G1 / G2 scalar
+int ripp_msm_batch_internal(ripp_ctx* ctx, int group, const void* bases, size_t bases_stride, const void* sc, size_t sc_stride,
+                            size_t n, size_t nseg, void* out);
+// nseg pairing products of n pairs each, segment s = (segs[2s], segs[2s+1]) (G1, G2 device pointers, read from device
+// memory); out[s] = final_exponentiation(prod e(P_i, Q_i))
+int ripp_pairing_table_l6(ripp_ctx* ctx, const void* segs_dev, size_t nseg, size_t n, void* out, int slot0);
 int ripp_pairing6_init_device();  // per-device kernel attributes; called by ripp_ctx_create with the device current
 // groth16.cu's kernels: fixed-base tables and prepare_inputs (setup.cu), Miller loops and checks (pairing6.cu)
 size_t ripp_groth16_table_bytes();  // one input's table

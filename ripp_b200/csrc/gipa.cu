@@ -929,4 +929,5 @@ extern "C" int ripp_sipp_prove(ripp_ctx* ctx, const void* a_aff, const void* b_a
 
 #include "verify.cuh"
 #include "verify_batch.cuh"
+#include "aggregate_batch.cuh"
 #include "sharded.cuh"

@@ -30,7 +30,11 @@ struct MsmPlan {
 };
 
 #define MSM_SMALL_N ((size_t)1 << 16)
-static MsmPlan msm_plan(size_t n, int bits = 255) {
+// seg: one segment of a segmented MSM (nseg > 1).  A short segment then takes its window from its own length, down to
+// c = 2 + 1, instead of the single MSM's floor of 6 + 1: the floor's nw x 64 buckets and 2 nw x 32 partials (~370 KB for
+// a G2 segment) would dwarf a segment of a few points, and a batch of 2^20 such segments would not fit the GPU.  The
+// window width does not change the result.
+static MsmPlan msm_plan(size_t n, int bits = 255, bool seg = false) {
   int lg = 0;
   while (((size_t)2 << lg) <= n) lg++;
   MsmPlan p;
@@ -43,7 +47,8 @@ static MsmPlan msm_plan(size_t n, int bits = 255) {
   // short inputs (the KZG openings and the MSM-type products of the GIPA rounds) are latency chains on an empty GPU:
   // ~4 points per bucket keeps the per-bucket chain short; below 2^6 points the window only sets the Horner tail
   p.c = lg - (n <= MSM_SMALL_N ? 2 : shift);
-  if (p.c < (n <= MSM_SMALL_N ? 6 : 4)) p.c = n <= MSM_SMALL_N ? 6 : 4;
+  const int c_min = n <= MSM_SMALL_N ? (seg ? 2 : 6) : 4;
+  if (p.c < c_min) p.c = c_min;
   if (p.c > 15) p.c = 15;
   // signed digits d_w in (-2^(c-1), 2^(c-1)] (the negative of a point is free): half the buckets of an unsigned window
   // for the same c, i.e. one more bit per window at equal bucket count.  The recoding may carry out of the top digit:
@@ -75,18 +80,22 @@ __device__ __forceinline__ uint32_t msm_sdigit(const uint32_t* s, int w, int c, 
   return neg ? (1u << c) - raw : raw;
 }
 
-// canonical scalars + per-(window, bucket) histogram
+// canonical scalars + per-(segment, window, bucket) histogram; n = nseg x seg_n scalars, segment s's at sc + s sc_stride
+// (SEG = false: one segment, seg_n = n; the single MSM's code)
+template <bool SEG>
 __global__ void k_msm_prepare(const Fr* __restrict__ sc, size_t n, Fr* __restrict__ canon, uint32_t* __restrict__ counts,
-                              int c, int nw, int is_mont) {
+                              int c, int nw, int is_mont, size_t seg_n, size_t sc_stride) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  Fr s = is_mont ? sc[i].from_mont() : sc[i];
+  const size_t seg = SEG ? i / seg_n : 0;
+  const Fr v = sc[seg * sc_stride + (i - seg * seg_n)];
+  Fr s = is_mont ? v.from_mont() : v;
   canon[i] = s;
   uint32_t B = 1u << (c - 1), carry = 0;
   for (int w = 0; w < nw; w++) {
     bool neg;
     uint32_t d = msm_sdigit(s.v, w, c, carry, neg);
-    if (d) atomicAdd(&counts[(size_t)w * B + d - 1], 1u);
+    if (d) atomicAdd(&counts[(seg * nw + w) * B + d - 1], 1u);
   }
 }
 
@@ -103,7 +112,8 @@ struct FatBucket {
   uint32_t bucket, first_item, nchunks;
 };
 
-// exclusive scan of counts within each window (one block per window) -> offsets into idx[w*n ..]
+// exclusive scan of counts within each window (one block per window; the nseg x nw windows of a segmented MSM in
+// segment-major order) -> offsets into idx[w*n ..], n = points per segment
 __global__ void k_msm_scan(const uint32_t* __restrict__ counts, uint32_t* __restrict__ offsets,
                            uint32_t* __restrict__ cursor, uint32_t B, size_t n, uint32_t* __restrict__ fat_counters,
                            FatItem* __restrict__ items, FatBucket* __restrict__ fats, uint32_t max_items,
@@ -143,16 +153,20 @@ __global__ void k_msm_scan(const uint32_t* __restrict__ counts, uint32_t* __rest
   }
 }
 
+// index entries are positions within the segment (the segment's bases are found from the bucket id)
+template <bool SEG>
 __global__ void k_msm_scatter(const Fr* __restrict__ canon, size_t n, uint32_t* __restrict__ cursor,
-                              uint32_t* __restrict__ idx, int c, int nw) {
+                              uint32_t* __restrict__ idx, int c, int nw, size_t seg_n) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
+  const size_t seg = SEG ? i / seg_n : 0;
   Fr s = canon[i];
   uint32_t B = 1u << (c - 1), carry = 0;
   for (int w = 0; w < nw; w++) {
     bool neg;
     uint32_t d = msm_sdigit(s.v, w, c, carry, neg);
-    if (d) idx[atomicAdd(&cursor[(size_t)w * B + d - 1], 1u)] = (uint32_t)i | (neg ? 0x80000000u : 0u);  // bit 31: subtract
+    if (d)  // bit 31: subtract
+      idx[atomicAdd(&cursor[(seg * nw + w) * B + d - 1], 1u)] = (uint32_t)(i - seg * seg_n) | (neg ? 0x80000000u : 0u);
   }
 }
 
@@ -184,15 +198,18 @@ __global__ void k_msm_size_scatter(const uint32_t* __restrict__ counts, size_t t
 }
 
 // one thread per non-empty bucket, in order of decreasing size (`order`, n_sorted = *n_sorted_dev entries): sum of the
-// bucket's points; bit 31 of an index entry = the point enters negated (signed window digits)
-template <class F>
+// bucket's points; bit 31 of an index entry = the point enters negated (signed window digits).  Bucket b belongs to
+// segment b / seg_buckets, whose bases start at bases + segment * bases_stride.
+template <class F, bool SEG>
 __global__ void __launch_bounds__(128) k_msm_accumulate(const Aff<F>* __restrict__ bases, const uint32_t* __restrict__ idx,
                                                         const uint32_t* __restrict__ offsets,
                                                         const uint32_t* __restrict__ counts, Jac<F>* __restrict__ buckets,
-                                                        const uint32_t* __restrict__ order, const uint32_t* __restrict__ n_sorted_dev) {
+                                                        const uint32_t* __restrict__ order, const uint32_t* __restrict__ n_sorted_dev,
+                                                        uint32_t seg_buckets, size_t bases_stride) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= *n_sorted_dev) return;
   const uint32_t b = order[t];
+  if (SEG) bases += (size_t)(b / seg_buckets) * bases_stride;
   uint32_t start = offsets[b], cnt = counts[b];
   Jac<F> acc = Jac<F>::inf();
   for (uint32_t j = 0; j < cnt; j++) {
@@ -205,22 +222,24 @@ __global__ void __launch_bounds__(128) k_msm_accumulate(const Aff<F>* __restrict
 }
 
 // one block per (fat bucket, chunk): strided partial sums, then a shared-memory tree
-template <class F>
+template <class F, bool SEG>
 __global__ void __launch_bounds__(128) k_msm_fat_chunks(const Aff<F>* __restrict__ bases, const uint32_t* __restrict__ idx,
                                                         const uint32_t* __restrict__ offsets,
                                                         const uint32_t* __restrict__ counts,
                                                         const uint32_t* __restrict__ fat_counters,
-                                                        const FatItem* __restrict__ items, Jac<F>* __restrict__ partials) {
+                                                        const FatItem* __restrict__ items, Jac<F>* __restrict__ partials,
+                                                        uint32_t seg_buckets, size_t bases_stride) {
   __shared__ Jac<F> sh[128];
   for (uint32_t it = blockIdx.x; it < fat_counters[0]; it += gridDim.x) {
     FatItem w = items[it];
+    const Aff<F>* bs = SEG ? bases + (size_t)(w.bucket / seg_buckets) * bases_stride : bases;
     uint32_t start = offsets[w.bucket] + w.chunk * MSM_FAT_CHUNK;
     uint32_t end = offsets[w.bucket] + counts[w.bucket];
     if (end > start + MSM_FAT_CHUNK) end = start + MSM_FAT_CHUNK;
     Jac<F> acc = Jac<F>::inf();
     for (uint32_t j = start + threadIdx.x; j < end; j += 128) {
       uint32_t e = idx[j];
-      Aff<F> p = bases[e & 0x7fffffffu];
+      Aff<F> p = bs[e & 0x7fffffffu];
       if (e >> 31) p = p.neg();
       acc = acc.add_mixed(p);
     }
@@ -313,9 +332,12 @@ __global__ void __launch_bounds__(WSUM_THREADS<F>::N) k_msm_window_sum(const Jac
   if (threadIdx.x == 0) out[blockIdx.x] = sh[0];
 }
 
+// Horner tails: one block per segment, block s reads window sums [s nw, s nw + nw) and writes out[s]
 template <class F>
 __global__ void k_msm_horner(const Jac<F>* __restrict__ sums, int nw, int c, Aff<F>* __restrict__ out) {
-  if (threadIdx.x || blockIdx.x) return;
+  if (threadIdx.x) return;
+  sums += (size_t)blockIdx.x * nw;
+  out += blockIdx.x;
   Jac<F> acc = sums[nw - 1];
   for (int w = nw - 2; w >= 0; w--) {
     for (int j = 0; j < c; j++) acc = acc.dbl();
@@ -345,6 +367,8 @@ static size_t w3_max_n() {
 // Horner tail on one three-warp team (<<<1, 96>>>; all lanes hold the same values)
 template <class XF>
 __global__ void __maxnreg__(255) k_msm_horner_x3(const Jac<XF>* __restrict__ sums, int nw, int c, Aff<XF>* __restrict__ out) {
+  sums += (size_t)blockIdx.x * nw;
+  out += blockIdx.x;
   Jac<XF> acc = sums[nw - 1];
   for (int w = nw - 2; w >= 0; w--) {
     for (int j = 0; j < c; j++) acc = x3::Ops<XF>::dbl(acc);
@@ -362,6 +386,8 @@ __global__ void __launch_bounds__(32 * 9) k_msm_horner_xt(const Jac<F>* __restri
   constexpr int AW = sizeof(Aff<F>) / 4;
   extern __shared__ __align__(16) uint32_t hsm[];
   const int warps = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  sums += (size_t)blockIdx.x * nw;
+  out += blockIdx.x;
   uint32_t* aff = hsm;                                        // nw affine window sums
   uint32_t* bus = hsm + ((nw * AW + 3) & ~3);                 // per team: 2 bus buffers
   const int vl = lane % (TO::LANES * TO::PER_WARP), e = vl / TO::LANES;
@@ -399,68 +425,87 @@ template <> struct X3Of<Fq2> { typedef x3::Fq2x3 type; };
 
 // sum_i s_i P_i = sum_i sum_t d_{i,t} E^t(P_i): m n points with short (128- / 64-bit) scalars, which cuts the
 // Horner tail (the latency floor of every MSM) from 255 to 128 / 64 doublings at the same bucket work
+// Segmented (nseg segments of n; segment s at bases + s bases_stride, sc + s sc_stride): segment s expands into the m n
+// entries [s m n, s m n + m n) of canon2 and, with bases_stride != 0, of bases2; with bases_stride = 0 (one base vector
+// for all segments) only segment 0 writes its m n bases.
 template <class F>
 __global__ void __launch_bounds__(128) k_msm_endo_expand(const Aff<F>* __restrict__ bases, const Fr* __restrict__ sc, size_t n,
-                                                         Aff<F>* __restrict__ bases2, Fr* __restrict__ canon2, int m) {
+                                                         Aff<F>* __restrict__ bases2, Fr* __restrict__ canon2, int m, size_t nseg,
+                                                         size_t bases_stride, size_t sc_stride) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  Fr s = sc[i].from_mont();
+  if (i >= n * nseg) return;
+  const size_t seg = i / n, e = i - seg * n, o = seg * m * n;
+  Fr s = sc[seg * sc_stride + e].from_mont();
   uint32_t digits[4][4];
   int mm;
   endo_digits<sizeof(F) == sizeof(Fq) ? 1 : 2>(s.v, digits, &mm);
-  Aff<F> p = bases[i];
+  Aff<F> p = bases[seg * bases_stride + e];
+  const bool put_bases = bases_stride || seg == 0;
   for (int t = 0; t < m; t++) {
     Fr d = Fr::zero();
     for (int j = 0; j < 4; j++) d.v[j] = digits[t][j];
-    bases2[(size_t)t * n + i] = p;
-    canon2[(size_t)t * n + i] = d;
+    if (put_bases) bases2[(bases_stride ? o : 0) + (size_t)t * n + e] = p;
+    canon2[o + (size_t)t * n + e] = d;
     if (t + 1 < m) p = endo_map(p);
   }
 }
 
 template <class F>
-static int msm_core(ripp_ctx* ctx, const Aff<F>* bases, const Fr* sc, size_t n, Aff<F>* out, int bits, int is_mont);
+static int msm_core(ripp_ctx* ctx, const Aff<F>* bases, size_t bases_stride, const Fr* sc, size_t sc_stride, size_t n, size_t nseg,
+                    Aff<F>* out, int bits, int is_mont);
 
+// out[s] = sum_i sc[s sc_stride + i] bases[s bases_stride + i], i < n, s < nseg (bases_stride 0: one base vector shared
+// by all segments).  nseg = 1 is the single MSM.
 template <class F>
-static int msm_dev(ripp_ctx* ctx, const Aff<F>* bases, const Fr* sc, size_t n, Aff<F>* out) {
+static int msm_dev(ripp_ctx* ctx, const Aff<F>* bases, const Fr* sc, size_t n, Aff<F>* out, size_t nseg = 1, size_t bases_stride = 0,
+                   size_t sc_stride = 0) {
   CU(cudaSetDevice(ctx->device));
   if (n == 0) {
-    CU(cudaMemsetAsync(out, 0, sizeof(Aff<F>), ctx->stream));
+    CU(cudaMemsetAsync(out, 0, nseg * sizeof(Aff<F>), ctx->stream));
     return RIPP_OK;
   }
-  if (!use_endo()) return msm_core<F>(ctx, bases, sc, n, out, 255, 1);
+  if (!use_endo()) return msm_core<F>(ctx, bases, bases_stride, sc, sc_stride, n, nseg, out, 255, 1);
   const int m = sizeof(F) == sizeof(Fq) ? 2 : 4;
+  const size_t mn = (size_t)m * n;
   void* ex;
-  size_t pts_bytes = ((size_t)m * n * sizeof(Aff<F>) + 255) & ~(size_t)255;
-  OK(scratch(ctx, 16, pts_bytes + (size_t)m * n * sizeof(Fr) + 256, &ex));
+  size_t pts_bytes = ((bases_stride ? nseg : 1) * mn * sizeof(Aff<F>) + 255) & ~(size_t)255;
+  OK(scratch(ctx, 16, pts_bytes + nseg * mn * sizeof(Fr) + 256, &ex));
   Aff<F>* bases2 = (Aff<F>*)ex;
   Fr* canon2 = (Fr*)((char*)ex + pts_bytes);
   {
     TimeScope ts_(ctx, RIPP_T_MSM_SORT);
-    k_msm_endo_expand<F><<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(bases, sc, n, bases2, canon2, m);
+    k_msm_endo_expand<F><<<(unsigned)((nseg * n + 127) / 128), 128, 0, ctx->stream>>>(bases, sc, n, bases2, canon2, m, nseg,
+                                                                                    bases_stride, sc_stride);
     LAUNCHED(ctx);
   }
-  return msm_core<F>(ctx, bases2, canon2, (size_t)m * n, out, m == 2 ? 128 : 64, 0);
+  return msm_core<F>(ctx, bases2, bases_stride ? mn : 0, canon2, mn, mn, nseg, out, m == 2 ? 128 : 64, 0);
 }
 
+// Segmented Pippenger: nseg independent MSMs of n points in one pass.  Every phase runs over the nseg x nw windows as one
+// set, a bucket keyed by (segment, window, digit); the plan (window width, chunks) is that of ONE segment of n points, so
+// a segment gets the buckets its own MSM would have and the launch sequence is that of the single MSM.
 template <class F>
-static int msm_core(ripp_ctx* ctx, const Aff<F>* bases, const Fr* sc, size_t n, Aff<F>* out, int bits, int is_mont) {
-  MsmPlan p = msm_plan(n, bits);
-  size_t WB = (size_t)p.nw * p.B;
+static int msm_core(ripp_ctx* ctx, const Aff<F>* bases, size_t bases_stride, const Fr* sc, size_t sc_stride, size_t n, size_t nseg,
+                    Aff<F>* out, int bits, int is_mont) {
+  MsmPlan p = msm_plan(n, bits, nseg > 1);
+  const size_t seg_buckets = (size_t)p.nw * p.B;  // buckets of one segment
+  const size_t nw = nseg * p.nw;                  // windows of all segments
+  const size_t N = nseg * n;                      // points of all segments
+  size_t WB = nw * p.B;
   void *canon, *cnt, *idx, *bkt, *parts;
-  OK(scratch(ctx, 4, n * sizeof(Fr), &canon));
+  OK(scratch(ctx, 4, N * sizeof(Fr), &canon));
   OK(scratch(ctx, 5, 3 * WB * sizeof(uint32_t), &cnt));
-  OK(scratch(ctx, 6, (size_t)p.nw * n * sizeof(uint32_t), &idx));
+  OK(scratch(ctx, 6, nw * n * sizeof(uint32_t), &idx));
   OK(scratch(ctx, 7, WB * sizeof(Jac<F>), &bkt));
-  OK(scratch(ctx, 8, 2 * (size_t)p.nw * p.T * sizeof(Jac<F>), &parts));
+  OK(scratch(ctx, 8, 2 * nw * p.T * sizeof(Jac<F>), &parts));
   uint32_t* counts = (uint32_t*)cnt;
   uint32_t* offsets = counts + WB;
   uint32_t* cursor = offsets + WB;
   cudaStream_t st = ctx->stream;
   // fat-bucket bookkeeping: at most nw*n/MSM_FAT fat buckets, nw*(n/CHUNK + n/FAT) chunk items
   const uint32_t fat_min = n <= MSM_SMALL_N ? 16u : MSM_FAT;
-  uint32_t max_fat = (uint32_t)((size_t)p.nw * n / fat_min + p.nw + 1);
-  uint32_t max_items = (uint32_t)((size_t)p.nw * n / MSM_FAT_CHUNK + max_fat + 1);
+  uint32_t max_fat = (uint32_t)(nw * n / fat_min + nw + 1);
+  uint32_t max_items = (uint32_t)(nw * n / MSM_FAT_CHUNK + max_fat + 1);
   void* fatbuf;
   OK(scratch(ctx, 15, 64 + (size_t)max_items * (sizeof(FatItem) + sizeof(Jac<F>)) + (size_t)max_fat * sizeof(FatBucket) + 1024, &fatbuf));
   uint32_t* fat_counters = (uint32_t*)fatbuf;
@@ -471,15 +516,18 @@ static int msm_core(ripp_ctx* ctx, const Aff<F>* bases, const Fr* sc, size_t n, 
   ts_.emplace(ctx, RIPP_T_MSM_SORT);
   CU(cudaMemsetAsync(fat_counters, 0, 64, st));
   CU(cudaMemsetAsync(counts, 0, WB * sizeof(uint32_t), st));
-  k_msm_prepare<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(sc, n, (Fr*)canon, counts, p.c, p.nw, is_mont);
+  const bool seg = nseg > 1;
+  (seg ? k_msm_prepare<true> : k_msm_prepare<false>)<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(sc, N, (Fr*)canon, counts, p.c, p.nw,
+                                                                                                  is_mont, n, sc_stride);
   LAUNCHED(ctx);
   // "fat" = far above the mean bucket size (and never below MSM_FAT points)
   uint32_t fat_threshold = (uint32_t)(4 * (n >> (p.c - 1)));  // 4 x the mean bucket size
   if (fat_threshold < fat_min) fat_threshold = fat_min;
-  k_msm_scan<<<p.nw, 256, 0, st>>>(counts, offsets, cursor, p.B, n, fat_counters, fat_items, fat_buckets, max_items,
+  k_msm_scan<<<(unsigned)nw, 256, 0, st>>>(counts, offsets, cursor, p.B, n, fat_counters, fat_items, fat_buckets, max_items,
                                    fat_threshold);
   LAUNCHED(ctx);
-  k_msm_scatter<<<(unsigned)((n + 127) / 128), 128, 0, st>>>((const Fr*)canon, n, cursor, (uint32_t*)idx, p.c, p.nw);
+  (seg ? k_msm_scatter<true> : k_msm_scatter<false>)<<<(unsigned)((N + 127) / 128), 128, 0, st>>>((const Fr*)canon, N, cursor,
+                                                                                                  (uint32_t*)idx, p.c, p.nw, n);
   LAUNCHED(ctx);
   // buckets by decreasing size; empty ones stay the identity (all-zero Jacobian: Z = 0)
   void* ordbuf;
@@ -497,39 +545,40 @@ static int msm_core(ripp_ctx* ctx, const Aff<F>* bases, const Fr* sc, size_t n, 
   LAUNCHED(ctx);
   ts_.reset();
   ts_.emplace(ctx, RIPP_T_MSM);
-  k_msm_accumulate<F><<<(unsigned)((WB + 127) / 128), 128, 0, st>>>(bases, (const uint32_t*)idx, offsets, counts,
-                                                                   (Jac<F>*)bkt, order, size_hist);
+  (seg ? k_msm_accumulate<F, true> : k_msm_accumulate<F, false>)<<<(unsigned)((WB + 127) / 128), 128, 0, st>>>(bases, (const uint32_t*)idx, offsets, counts,
+                                                                   (Jac<F>*)bkt, order, size_hist, (uint32_t)seg_buckets,
+                                                                   bases_stride);
   LAUNCHED(ctx);
   {
     unsigned fat_grid = max_items < 1184u ? max_items : 1184u;  // grid-stride over the item list; 8 blocks per SM
-    k_msm_fat_chunks<F><<<fat_grid, 128, 0, st>>>(bases, (const uint32_t*)idx, offsets, counts, fat_counters, fat_items,
-                                                  fat_partials);
+    (seg ? k_msm_fat_chunks<F, true> : k_msm_fat_chunks<F, false>)<<<fat_grid, 128, 0, st>>>(bases, (const uint32_t*)idx, offsets, counts, fat_counters, fat_items,
+                                                  fat_partials, (uint32_t)seg_buckets, bases_stride);
     LAUNCHED(ctx);
     k_msm_fat_combine<F><<<max_fat < 256u ? max_fat : 256u, 64, 0, st>>>(fat_counters, fat_buckets, fat_partials, (Jac<F>*)bkt);
     LAUNCHED(ctx);
   }
   ts_.reset();
   ts_.emplace(ctx, RIPP_T_MSM_REDUCE);
-  size_t WT = (size_t)p.nw * p.T;
+  size_t WT = nw * p.T;
   Jac<F>* pa = (Jac<F>*)parts;
   Jac<F>* pb = pa + WT;
   k_msm_bucket_reduce<F><<<(unsigned)((WT + 127) / 128), 128, 0, st>>>((const Jac<F>*)bkt, p.B, p.L, p.T, pa, WT);
   LAUNCHED(ctx);
   // window sums: one block per window (strided partial sums, then a shared-memory tree) instead of a ladder of
   // log_8(T) launches of a few warps each
-  k_msm_window_sum<F><<<p.nw, WSUM_THREADS<F>::N, 0, st>>>(pa, p.T, pb);
+  k_msm_window_sum<F><<<(unsigned)nw, WSUM_THREADS<F>::N, 0, st>>>(pa, p.T, pb);
   LAUNCHED(ctx);
   pa = pb;
   if (fold_mode() == 0) {
     typedef xt::TeamOf<F> TO;
     int warps = (p.nw + TO::PER_WARP - 1) / TO::PER_WARP;
     if (warps > 9) warps = 9;
-    k_msm_horner_xt<F><<<1, 32 * warps, horner_xt_smem<F>(p.nw), st>>>(pa, p.nw, p.c, out);
+    k_msm_horner_xt<F><<<(unsigned)nseg, 32 * warps, horner_xt_smem<F>(p.nw), st>>>(pa, p.nw, p.c, out);
   } else if (fold_mode() == 1) {
     typedef typename X3Of<F>::type XF;
-    k_msm_horner_x3<XF><<<1, 96, 0, st>>>((const Jac<XF>*)pa, p.nw, p.c, (Aff<XF>*)out);
+    k_msm_horner_x3<XF><<<(unsigned)nseg, 96, 0, st>>>((const Jac<XF>*)pa, p.nw, p.c, (Aff<XF>*)out);
   } else {
-    k_msm_horner<F><<<1, 32, 0, st>>>(pa, p.nw, p.c, out);
+    k_msm_horner<F><<<(unsigned)nseg, 32, 0, st>>>(pa, p.nw, p.c, out);
   }
   LAUNCHED(ctx);
   return RIPP_OK;
@@ -542,6 +591,31 @@ extern "C" int ripp_msm_g1_dev(ripp_ctx* ctx, const void* bases, const void* sc,
 extern "C" int ripp_msm_g2_dev(ripp_ctx* ctx, const void* bases, const void* sc, size_t n, void* out) {
   if (!ctx || !out || (n && (!bases || !sc))) return fail(RIPP_ERR_ARG, "null argument");
   return msm_dev<Fq2>(ctx, (const G2Aff*)bases, (const Fr*)sc, n, (G2Aff*)out);
+}
+
+// nseg MSMs in one pass (segmented Pippenger above); the scalars of segment s at sc + s sc_stride
+int ripp_msm_batch_internal(ripp_ctx* ctx, int group, const void* bases, size_t bases_stride, const void* sc, size_t sc_stride,
+                            size_t n, size_t nseg, void* out) {
+  if (nseg == 0) return RIPP_OK;
+  if (group == 1) return msm_dev<Fq>(ctx, (const G1Aff*)bases, (const Fr*)sc, n, (G1Aff*)out, nseg, bases_stride, sc_stride);
+  return msm_dev<Fq2>(ctx, (const G2Aff*)bases, (const Fr*)sc, n, (G2Aff*)out, nseg, bases_stride, sc_stride);
+}
+static int msm_batch_entry(ripp_ctx* ctx, int group, const void* bases, size_t bases_stride, const void* sc, size_t n, size_t nseg,
+                           void* out) {
+  if (!ctx || (nseg && !out) || (n && nseg && (!bases || !sc))) return fail(RIPP_ERR_ARG, "null argument");
+  // the workspace grows with both: ~65 KB per short G2 segment (window by segment length), and for long ones that of
+  // one MSM over all nseg x n points
+  if (nseg > ((size_t)1 << 16)) return fail(RIPP_ERR_ARG, "batch MSM: more than 2^16 segments");
+  if (n && nseg > ((size_t)1 << 24) / n) return fail(RIPP_ERR_ARG, "batch MSM: segments x length over 2^24");
+  return ripp_msm_batch_internal(ctx, group, bases, bases_stride, sc, n, n, nseg, out);
+}
+extern "C" int ripp_msm_g1_batch_dev(ripp_ctx* ctx, const void* bases, size_t bases_stride, const void* sc, size_t n, size_t nseg,
+                                     void* out) {
+  return msm_batch_entry(ctx, 1, bases, bases_stride, sc, n, nseg, out);
+}
+extern "C" int ripp_msm_g2_batch_dev(ripp_ctx* ctx, const void* bases, size_t bases_stride, const void* sc, size_t n, size_t nseg,
+                                     void* out) {
+  return msm_batch_entry(ctx, 2, bases, bases_stride, sc, n, nseg, out);
 }
 
 template <class F>
@@ -1003,6 +1077,128 @@ int ripp_fold4_internal(ripp_ctx* ctx, const int* types, const void* const* hi, 
     k_fold4_xt<<<nblocks, 32 * XT_WARPS, 0, ctx->stream>>>(jobs);
   LAUNCHED(ctx);
   *fused = 1;
+  return RIPP_OK;
+}
+
+// ---- the folds of many GIPA recursions from a device table (the lock-step batch prover, aggregate_batch.cuh) ------------
+// Sections by element type (G1, G2, Fr); within a section, group g of K jobs folds the vector at base[g] + k stride[g]
+// (instance k) with the scalar record sc[g][k] (EndoBits for G1 / G2, Fr for Fr).  All jobs have the same length n, so a
+// block finds its job from its section's first block and the blocks per job; the job itself is built in registers and
+// handed to the bodies of k_fold4_xt / k_fold4_xp.
+__device__ __forceinline__ bool fold_tab_job(const FoldTable& t, uint32_t blk, int type, FoldJob& job, uint32_t* block) {
+  const int s = type - 1;
+  if (blk < t.first_block[s] || blk >= t.first_block[s] + t.blocks[s]) return false;
+  const uint32_t r = blk - t.first_block[s], j = r / t.bpj[s], g = j / t.K, k = j % t.K;
+  const size_t esz = type == 1 ? sizeof(G1Aff) : type == 2 ? sizeof(G2Aff) : sizeof(Fr);
+  char* lo = t.base[s][g] + (size_t)k * t.stride[s][g];
+  job.type = type;
+  job.lo = lo;
+  job.hi = lo + (size_t)t.n * esz;
+  job.out = lo;
+  job.n = t.n;
+  if (type == 3)
+    job.s = ((const Fr*)t.sc[s][g])[k];
+  else
+    job.c = ((const EndoBits*)t.sc[s][g])[k];
+  *block = r - j * t.bpj[s];
+  return true;
+}
+template <bool XP>
+__global__ void __launch_bounds__(32 * (XP ? XP_WARPS : XT_WARPS)) k_fold_tab(const FoldTable t) {
+  constexpr int W1 = XP ? XpLayout<Fq, XP_WARPS>::WORDS : FOLD4_BUS_WORDS_G1;
+  constexpr int W2 = XP ? XpLayout<Fq2, XP_WARPS>::WORDS : FOLD4_BUS_WORDS_G2;
+  __shared__ __align__(16) uint32_t sm[W1 > W2 ? W1 : W2];
+  FoldJob job;
+  uint32_t block;
+  if (fold_tab_job(t, blockIdx.x, 1, job, &block)) {
+    if constexpr (XP) fold_xp_body<Fq, false>(sm, job, block);
+    else fold_xt_body<Fq>(sm, job, block);
+  } else if (fold_tab_job(t, blockIdx.x, 2, job, &block)) {
+    if constexpr (XP) fold_xp_body<Fq2, false>(sm, job, block);
+    else fold_xt_body<Fq2>(sm, job, block);
+  } else if (fold_tab_job(t, blockIdx.x, 3, job, &block)) {
+    size_t i = (size_t)block * blockDim.x + threadIdx.x;
+    if (i < job.n) ((Fr*)job.out)[i] = ((const Fr*)job.hi)[i] * job.s + ((const Fr*)job.lo)[i];
+  }
+}
+// long vectors (above the lane-team range): one thread per element, one launch per element type; the table holds only
+// that type's section at first block 0
+template <class F>
+__global__ void __launch_bounds__(64, 4) k_fold_tab_endo(const FoldTable t) {
+  constexpr int type = sizeof(F) == sizeof(Fq) ? 1 : 2;
+  FoldJob job;
+  uint32_t block;
+  if (!fold_tab_job(t, blockIdx.x, type, job, &block)) return;
+  size_t i = (size_t)block * blockDim.x + threadIdx.x;
+  if (i >= job.n) return;
+  Jac<F> acc = endo_mul<F>(((const Aff<F>*)job.hi)[i], job.c);
+  acc = acc.add_mixed(((const Aff<F>*)job.lo)[i]);
+  ((Aff<F>*)job.out)[i] = acc.to_affine();
+}
+__global__ void k_fold_tab_fr(const FoldTable t) {
+  FoldJob job;
+  uint32_t block;
+  if (!fold_tab_job(t, blockIdx.x, 3, job, &block)) return;
+  size_t i = (size_t)block * blockDim.x + threadIdx.x;
+  if (i < job.n) ((Fr*)job.out)[i] = ((const Fr*)job.hi)[i] * job.s + ((const Fr*)job.lo)[i];
+}
+
+// host side of the scalar records
+void ripp_endo_bits(int group, const void* fr_mont_host, EndoBits* out) {
+  *out = group == 1 ? endo_bits<Fq>(fr_mont_host) : endo_bits<Fq2>(fr_mont_host);
+}
+
+// One round's folds of every job in t (t.base / stride / sc / ngroups / K / n filled by the caller): one launch while
+// the vectors are short enough for lane teams, else one launch per element type.  The RIPP_B200_FOLD override of the
+// single path (A/B runs of the fold kernels) does not apply here: the batch always runs these kernels, and the result
+// does not depend on the kernel.
+int ripp_fold_table_internal(ripp_ctx* ctx, FoldTable t) {
+  const size_t n = t.n;
+  if (n == 0) return RIPP_OK;
+  CU(cudaSetDevice(ctx->device));
+  TimeScope ts_(ctx, RIPP_T_FOLD);
+  if (n <= xt_max_n()) {
+    const bool xp = n <= xp_max_n();
+    const uint32_t bt = 32 * (xp ? XP_WARPS : XT_WARPS);
+    uint32_t nblocks = 0;
+    for (int s = 0; s < 3; s++) {
+      uint32_t bpj;
+      if (s < 2) {
+        const uint32_t per = s == 0 ? xt::TeamOf<Fq>::PER_WARP : xt::TeamOf<Fq2>::PER_WARP;
+        const uint32_t warps = (uint32_t)((n + per - 1) / per);
+        const int m = s == 0 ? XpShape<false>::PARTS<Fq> : XpShape<false>::PARTS<Fq2>;
+        bpj = xp ? (warps * m + XP_WARPS - 1) / XP_WARPS : (warps + XT_WARPS - 1) / XT_WARPS;
+      } else {
+        bpj = (uint32_t)((n + bt - 1) / bt);
+      }
+      t.bpj[s] = bpj;
+      t.first_block[s] = nblocks;
+      t.blocks[s] = bpj * t.K * t.ngroups[s];
+      nblocks += t.blocks[s];
+    }
+    if (xp)
+      k_fold_tab<true><<<nblocks, bt, 0, ctx->stream>>>(t);
+    else
+      k_fold_tab<false><<<nblocks, bt, 0, ctx->stream>>>(t);
+    LAUNCHED(ctx);
+    return RIPP_OK;
+  }
+  for (int s = 0; s < 3; s++) {
+    if (!t.ngroups[s]) continue;
+    FoldTable u = t;
+    const uint32_t bt = s < 2 ? 64 : 128;
+    for (int o = 0; o < 3; o++) u.blocks[o] = 0;
+    u.bpj[s] = (uint32_t)((n + bt - 1) / bt);
+    u.first_block[s] = 0;
+    u.blocks[s] = u.bpj[s] * t.K * t.ngroups[s];
+    if (s == 0)
+      k_fold_tab_endo<Fq><<<u.blocks[s], bt, 0, ctx->stream>>>(u);
+    else if (s == 1)
+      k_fold_tab_endo<Fq2><<<u.blocks[s], bt, 0, ctx->stream>>>(u);
+    else
+      k_fold_tab_fr<<<u.blocks[s], bt, 0, ctx->stream>>>(u);
+    LAUNCHED(ctx);
+  }
   return RIPP_OK;
 }
 

@@ -16,6 +16,12 @@ struct Miller6Batch {
   int nseg;
   uint32_t fixed_q;  // PER_GROUP kernels: bit j set = pair j of every item has the one Q at q[j][0]
 };
+// TAB kernels (k_miller6<.., .., false, true>): any number of segments, segment s's P and Q base pointers at
+// segs[2 s], segs[2 s + 1] in device memory (b.p[0] holds segs); b.nseg segments of b.n pairs
+struct M6Seg {
+  const G1Aff* p;
+  const G2Aff* q;
+};
 
 constexpr int M6_NREG = 2;
 constexpr int M6_WARPS = 4;
@@ -31,7 +37,8 @@ __global__ void k_init_g2_gen() { g_g2_gen = g2_generator(); }
 // PER_GROUP: one Miller value per item instead of one product per warp -- group t walks pair j = (p[j][t], q[j][t]) for
 // j < KP (one segment of n items; Q of pair j is q[j][0] for every item when bit j of fixed_q is set) and writes its
 // accumulator to partials[t] (the per-proof values of a Groth16 batch, groth16.cu).
-template <int WARPS, int KP, bool PER_GROUP = false>
+// TAB: the segments' base pointers come from the device table at b.p[0] (M6Seg), the segment from the flat warp index.
+template <int WARPS, int KP, bool PER_GROUP = false, bool TAB = false>
 __global__ void __launch_bounds__(32 * WARPS) k_miller6(Miller6Batch b, Fq12* __restrict__ partials) {
   extern __shared__ __align__(16) uint32_t smem[];
   constexpr int GW = group_words(M6_NREG, KP);
@@ -56,7 +63,18 @@ __global__ void __launch_bounds__(32 * WARPS) k_miller6(Miller6Batch b, Fq12* __
       G1Aff P = g1_generator();
       const G2Aff* Q = &g_g2_gen;
       uint32_t valid = 0;
-      if (seg < (uint32_t)b.nseg && i < b.n) {
+      if constexpr (TAB) {
+        if (seg < (uint32_t)b.nseg && i < b.n) {
+          const M6Seg sg = reinterpret_cast<const M6Seg*>(b.p[0])[seg];
+          G1Aff p = sg.p[i];
+          const G2Aff* q = &sg.q[i];
+          if (!p.is_inf() && !q->is_inf()) {
+            P = p;
+            Q = q;
+            valid = 1;
+          }
+        }
+      } else if (seg < (uint32_t)b.nseg && i < b.n) {
         G1Aff p = b.p[sv][i];
         const G2Aff* q = &b.q[sv][PER_GROUP && ((b.fixed_q >> j) & 1) ? 0 : i];
         if (!p.is_inf() && !q->is_inf()) {
@@ -426,11 +444,12 @@ static int m6_pairs_per_group(ripp_ctx* ctx, size_t nseg, size_t pairs_per_seg, 
   return RIPP_OK;
 }
 
-template <int KP>
+template <int KP, bool TAB = false>
 static int launch_miller6(ripp_ctx* ctx, Miller6Batch& b, Fq12* dst) {
   b.wps = (uint32_t)(((size_t)b.n + 5 * KP - 1) / (5 * KP));
   const size_t nwarps = (size_t)b.wps * b.nseg;
-  k_miller6<M6_WARPS, KP><<<(unsigned)((nwarps + M6_WARPS - 1) / M6_WARPS), 32 * M6_WARPS, m6_smem_bytes(KP), ctx->stream>>>(b, dst);
+  k_miller6<M6_WARPS, KP, false, TAB><<<(unsigned)((nwarps + M6_WARPS - 1) / M6_WARPS), 32 * M6_WARPS, m6_smem_bytes(KP), ctx->stream>>>(
+      b, dst);
   LAUNCHED(ctx);
   return RIPP_OK;
 }
@@ -438,15 +457,16 @@ static int launch_miller6(ripp_ctx* ctx, Miller6Batch& b, Fq12* dst) {
 // The six-lane products: one k_miller6 launch at kp pairs per group (one partial per warp, at *src), then reduce6 over
 // nseg equal runs of those partials down to `stop` per run.  The runs are b's segments, or (the RLC check) the
 // warp-aligned segments inside b's one segment.
+template <bool TAB = false>
 static int m6_products(ripp_ctx* ctx, Miller6Batch& b, int kp, uint32_t nseg, uint32_t stop, Fq12** src, Fq12* dst, uint32_t* T) {
   if (kp == 4)
-    OK(launch_miller6<4>(ctx, b, *src));
+    OK((launch_miller6<4, TAB>(ctx, b, *src)));
   else if (kp == 3)
-    OK(launch_miller6<3>(ctx, b, *src));
+    OK((launch_miller6<3, TAB>(ctx, b, *src)));
   else if (kp == 2)
-    OK(launch_miller6<2>(ctx, b, *src));
+    OK((launch_miller6<2, TAB>(ctx, b, *src)));
   else
-    OK(launch_miller6<1>(ctx, b, *src));
+    OK((launch_miller6<1, TAB>(ctx, b, *src)));
   *T = (uint32_t)((size_t)b.wps * b.nseg / nseg);
   return reduce6(ctx, nseg, stop, src, dst, T);
 }
@@ -514,6 +534,34 @@ int ripp_pairing_batch_l6(ripp_ctx* ctx, int nseg, const void* const* g1, const 
   k_final_exp18<<<nseg, 32, FE18_GROUP_WORDS * 4, ctx->stream>>>(src, T, (Fq12*)out);
   LAUNCHED(ctx);
   return RIPP_OK;
+}
+
+// nseg products of n pairs with the segments' pointers in device memory (M6Seg table, any nseg): one k_miller6<.., TAB>
+// launch at the pairs-per-group rule's kp, the k_reduce6 tree down to at most four partials per segment, one final
+// exponentiation launch.  The launch count depends on n and kp, not on nseg beyond the kp choice.  Scratch slots
+// slot0, slot0 + 1.
+int ripp_pairing_table_l6(ripp_ctx* ctx, const void* segs_dev, size_t nseg, size_t n, void* out, int slot0) {
+  if (nseg == 0) return RIPP_OK;
+  if (n == 0 || nseg > 0xffffffffu / ((n + 4) / 5)) return fail(RIPP_ERR_ARG, "bad pairing table shape");
+  CU(cudaSetDevice(ctx->device));
+  Miller6Batch b;
+  memset(&b, 0, sizeof(b));
+  b.p[0] = (const G1Aff*)segs_dev;
+  b.n = (uint32_t)n;
+  b.nseg = (int)nseg;
+  int kp;
+  OK(m6_pairs_per_group(ctx, nseg, n, true, &kp));
+  const size_t max_partials = nseg * ((n + 4) / 5);
+  void *bufA, *bufB;
+  OK(scratch(ctx, slot0, max_partials * sizeof(Fq12) + 4096, &bufA));
+  OK(scratch(ctx, slot0 + 1, nseg * (((n + 4) / 5 + 7) / 8) * sizeof(Fq12) + 8192, &bufB));  // the first k_reduce6 level
+  Fq12 *src = (Fq12*)bufA, *dst = (Fq12*)bufB;
+  uint32_t T;
+  {
+    TimeScope ts_(ctx, RIPP_T_MILLER);
+    OK(m6_products<true>(ctx, b, kp, (uint32_t)nseg, 4, &src, dst, &T));
+  }
+  return ripp_final_exp_l6(ctx, src, T, out, (int)nseg);
 }
 
 // out[s] = final_exponentiation(prod_j in[s*T + j])
@@ -652,6 +700,10 @@ int ripp_pairing6_init_device() {
   CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(3)));
   CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(4)));
   CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(3)));
+  CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(1)));
+  CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(2)));
+  CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 3, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(3)));
+  CU(cudaFuncSetAttribute(k_miller6<M6_WARPS, 4, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, m6_smem_bytes(4)));
   CU(cudaFuncSetAttribute(k_groth16_check6, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 6 * FE_GROUP_WORDS * 4));
   return RIPP_OK;
 }

@@ -64,6 +64,7 @@ extern "C" void ripp_ctx_destroy(ripp_ctx* ctx) {
     if (ctx->scratch[i]) cudaFree(ctx->scratch[i]);
   cudaStreamDestroy(ctx->own_stream);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
+  if (ctx->pinned_big) cudaFreeHost(ctx->pinned_big);
   if (ctx->recs) {
     for (auto& r : *ctx->recs) {
       cudaEventDestroy(r.a);

@@ -157,6 +157,25 @@ def aggregate_proofs(srs, proofs, ctx=None):
     return ctx.tipp_aggregate_dev(s1, s2, a, b, c, n)
 
 
+def aggregate_proofs_batch(srs, batches, ctx=None):
+    """aggregate_proofs for many batches of Groth16 proofs under one SRS in one call, the GIPA rounds of all batches in
+    lock step.  srs = (g_alpha_powers, h_beta_powers); batches: lists of (A, B, C), all of the same power-of-two length.
+    -> list of AggregateProof bytes, element k equal to aggregate_proofs(srs, batches[k])."""
+    ctx = ctx or default_context()
+    if not batches:
+        return []
+    n = len(batches[0])
+    if any(len(b) != n for b in batches):
+        raise ValueError("all batches must have the same number of proofs")
+    flat = [p for b in batches for p in b]
+    a = ctx.to_device(codec.g1_vec_enc([p[0] for p in flat]))
+    b = ctx.to_device(codec.g2_vec_enc([p[1] for p in flat]))
+    c = ctx.to_device(codec.g1_vec_enc([p[2] for p in flat]))
+    s1 = ctx.to_device(codec.g1_vec_enc(srs[0]))
+    s2 = ctx.to_device(codec.g2_vec_enc(srs[1]))
+    return ctx.tipp_aggregate_batch_dev(s1, s2, a, b, c, len(batches), n)
+
+
 PROOF_RECORD_BYTES = {True: 192, False: 384}
 
 

@@ -248,6 +248,35 @@ pub fn aggregate_proofs(srs: &GpuSrs, proofs: &[Proof<Bls12_381>]) -> Result<Agg
     parse_aggregate(buf)
 }
 
+/// `aggregate_proofs` for many batches of proofs under one SRS in one call (one aggregate per client, circuit batch or
+/// block), their GIPA rounds in lock step on the GPU.  All batches must have the same power-of-two length; element k
+/// of the result is what `aggregate_proofs(srs, batches[k])` returns.
+pub fn aggregate_proofs_batch(srs: &GpuSrs, batches: &[&[Proof<Bls12_381>]]) -> Result<Vec<AggregateProofParts>, Error> {
+    let count = batches.len();
+    if count == 0 {
+        return Ok(Vec::new());
+    }
+    let n = batches[0].len();
+    if let Some(b) = batches.iter().find(|b| b.len() != n) {
+        return Err(Box::new(ark_ip_proofs::InnerProductArgumentError::MessageLengthInvalid(n, b.len())));
+    }
+    let all: Vec<&Proof<Bls12_381>> = batches.iter().flat_map(|b| b.iter()).collect();
+    let a = pack::pack_g1_aff(&all.iter().map(|p| p.a).collect::<Vec<_>>());
+    let b = pack::pack_g2_aff(&all.iter().map(|p| p.b).collect::<Vec<_>>());
+    let cc = pack::pack_g1_aff(&all.iter().map(|p| p.c).collect::<Vec<_>>());
+    let mut buf = vec![0u8; count * (8192 + 2 * proof_capacity(n))];
+    let mut len = 0usize;
+    let c = ctx();
+    let st = unsafe {
+        sys::ripp_tipp_aggregate_batch(c.raw(), srs.g_alpha_powers.ptr(), srs.h_beta_powers.ptr(), count, n,
+                                       a.as_ptr() as *const c_void, b.as_ptr() as *const c_void, cc.as_ptr() as *const c_void,
+                                       buf.as_mut_ptr(), buf.len(), &mut len)
+    };
+    drop(c);
+    check(st, n, n)?;
+    (0..count).map(|k| parse_aggregate(buf[k * len..(k + 1) * len].to_vec())).collect()
+}
+
 /// `aggregate_proofs` from the proofs' bytes, as an aggregation service receives them from untrusted provers: `proofs`
 /// holds n ark-groth16 `Proof` records back to back, each written with `serialize_with_mode(compress)` (192 B
 /// compressed, 384 B uncompressed), no length prefix.  The library decodes and validates every point on the GPU
