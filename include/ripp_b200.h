@@ -483,6 +483,63 @@ int ripp_tipp_verify_aggregate_batch(ripp_ctx* ctx, const void* vsrs, const void
 int ripp_sipp_verify(ripp_ctx* ctx, const void* a_aff, const void* b_aff, const void* r, size_t n, const void* value_gt,
                      const uint8_t* proof, size_t proof_len, int* accept);
 
+/* ---- polynomial commitments (ip_proofs/src/applications/poly_commit/{mod,transparent}.rs; BLS12-381) ---------------- */
+/* Coefficient layout.  A bivariate polynomial is ONE device array of `len` Fr (Montgomery), read row-major with row
+ * length m = y_degree + 1: coefficient j of Y polynomial i sits at i * m + j, and everything at or beyond `len` is zero.
+ * With n = x_degree + 1 rows, len <= n * m.  A univariate polynomial of degree < n * m is already in this layout: it is
+ * the bivariate form UnivariatePolynomialCommitment builds (mod.rs:286-377), opened at (z^m, z), so the univariate and
+ * transparent-univariate wrappers map degrees and the point only.  Ragged Y polynomials are padded to m by the caller.
+ * n and m must be powers of two (RIPP_ERR_NOT_POW2); n <= 2^16, n * m <= 2^24 (the segmented MSM's limits), null
+ * pointers and len > n * m give RIPP_ERR_ARG.  The limits cover univariate degree 2^24 - 1, i.e. (255, 65535). */
+typedef enum ripp_pc_kind {
+  RIPP_PC_TRUSTED = 0,    /* BivariatePolynomialCommitment (mod.rs:153-284): KZG first tier, TIPAWithSSM second tier */
+  RIPP_PC_TRANSPARENT = 1 /* TransparentBivariatePolynomialCommitment (transparent.rs:85-213): Pedersen<G1> first tier,
+                             GIPA with structured scalar message on both tiers */
+} ripp_pc_kind;
+
+/* Division by (X - z): q = (f - f(z)) / (X - z) (len - 1 Fr, q_out_dev; may be NULL when len <= 1) and the remainder
+ * f(z) (one Fr, eval_out_dev, may be NULL), the synthetic division of KZG::open (mod.rs:98-104) as a parallel scan of
+ * its linear recurrence.  coeffs_dev: len Fr, lowest degree first; z_host: one Fr (host).  q must not overlap coeffs.
+ * len = 0 gives f(z) = 0.  Asynchronous on the context's stream. */
+int ripp_fr_div_linear_dev(ripp_ctx* ctx, const void* coeffs_dev, size_t len, const void* z_host, void* q_out_dev,
+                           void* eval_out_dev);
+/* KZG::commit (mod.rs:85): sum_i coeffs[i] powers[i] over the first len of n_powers G1 powers g^(alpha^i) (device);
+ * len > n_powers: RIPP_ERR_ARG; len = 0: the identity.  One affine point to device memory, asynchronous. */
+int ripp_pc_kzg_commit_dev(ripp_ctx* ctx, const void* powers_dev, size_t n_powers, const void* coeffs_dev, size_t len,
+                           void* g1_aff_out_dev);
+/* KZG::open (mod.rs:98-104) at z_host: the quotient on the device, then one MSM.  eval_out_dev (nullable) receives
+ * f(z).  len <= 1 has an empty quotient: the proof is the identity.  Asynchronous. */
+int ripp_pc_kzg_open_dev(ripp_ctx* ctx, const void* powers_dev, size_t n_powers, const void* coeffs_dev, size_t len,
+                         const void* z_host, void* g1_aff_out_dev, void* eval_out_dev);
+/* KZG::verify (mod.rs:120-130) as one two-pair product e(com - g eval, h) e(-proof, h_alpha - h z) == 1.  vsrs: the
+ * VerifierSRS layout of ripp_tipa_verify; com, proof: G1 affine (host, Montgomery); z, eval: Fr (host). */
+int ripp_pc_kzg_verify(ripp_ctx* ctx, const void* vsrs, const void* com, const void* z, const void* eval, const void* proof,
+                       int* accept);
+
+/* Commit (mod.rs:186 / transparent.rs:106-119): the n first-tier commitments of the Y polynomials over the m shared
+ * first-tier bases (trusted: the KZG powers g^(alpha^j); transparent: the Pedersen key) as ONE segmented MSM
+ * (y_coms_dev: n G1 affine, device), then the AFGHO pairing product with the n second-tier G2 keys (trusted: the even
+ * powers h^(beta^(2i)); transparent: the second-tier key).  gt_out: the commitment (576 B, host).  Synchronous.  Apart
+ * from the pairing product's reduction tree (log n depth), the number of kernel launches does not depend on n. */
+int ripp_pc_commit_dev(ripp_ctx* ctx, const void* first_tier_dev, size_t m, const void* second_tier_dev, size_t n,
+                       const void* coeffs_dev, size_t len, void* gt_out, void* y_coms_dev);
+/* Open at (x, y) (host Fr).  trusted (mod.rs:211-241 and on): srs_g2_dev = h_beta_powers (2 n - 1 G2), the argument is
+ * TIPAWithSSM over (y_coms, powers of x) and the KZG opening of y_eval at y; transparent (transparent.rs:137 and on):
+ * srs_g2_dev unused, GIPA MULTIEXP_SSM over (y_coms, powers of x) and GIPA SCALAR_SSM_G1 over (y_eval, powers of y).
+ * Powers, the row combination y_eval, y_eval_comm and the quotient stay on the device.  proof_out: the OpeningProof
+ * bytes (trusted: ip_proof || y_eval_comm || kzg_proof; transparent: second_tier_ip_proof || y_eval_comm ||
+ * first_tier_ip_proof); eval_out (host, nullable): f(x, y).  Synchronous. */
+int ripp_pc_open_dev(ripp_ctx* ctx, int kind, const void* first_tier_dev, size_t m, const void* second_tier_dev, size_t n,
+                     const void* srs_g2_dev, const void* coeffs_dev, size_t len, const void* y_coms_dev, const void* x_host,
+                     const void* y_host, uint8_t* proof_out, size_t proof_cap, size_t* proof_len, void* eval_out);
+/* Verify an opening of com_gt (host GT, as ripp_pc_commit_dev returns it) at (x, y) to eval (host Fr).  trusted
+ * (BivariatePolynomialCommitment::verify): vsrs only (keys and n, m unused), ripp_tipa_verify on com || IdentityOutput(y_eval_comm) plus the
+ * KZG check; transparent (the transparent verify): first / second-tier keys with m, n, two ripp_gipa_verify_dev.
+ * Undecodable bytes: RIPP_ERR_ARG. */
+int ripp_pc_verify(ripp_ctx* ctx, int kind, const void* vsrs, const void* first_tier_dev, size_t m, const void* second_tier_dev,
+                   size_t n, const void* com_gt, const void* x_host, const void* y_host, const void* eval, const uint8_t* proof,
+                   size_t proof_len, int* accept);
+
 /* ---- diagnostics --------------------------------------------------------------------------- */
 /* Element-wise primitive ops on device, used by the GPU parity tests to pin the PTX limb layer:
  * op in ripp_test_op; a, b, r are HOST arrays of n elements of the op's operand size. */

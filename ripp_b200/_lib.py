@@ -36,6 +36,7 @@ class RippError(RuntimeError):
 
 GIPA_PAIRING, GIPA_MULTIEXP_PEDERSEN, GIPA_MULTIEXP_SSM = 0, 1, 2
 GIPA_SCALAR_PEDERSEN_G2_G2, GIPA_SCALAR_PEDERSEN_G2_G1, GIPA_SCALAR_SSM, GIPA_SCALAR_SSM_G1 = 3, 4, 5, 6
+PC_TRUSTED, PC_TRANSPARENT = 0, 1
 
 
 class LengthMismatch(RippError):
@@ -502,6 +503,54 @@ class Context:
         check(lib().ripp_kzg_quotient(_p(transcript), ctypes.c_size_t(len(transcript)), _p(r_shift), _p(z),
                                       ctypes.c_size_t(n_srs), _p(out)))
         return out
+
+    # ---- polynomial commitments (csrc/poly_commit.cuh) ------------------------------------------------
+    def fr_div_linear_dev(self, coeffs_dev, length, z, q_out_dev, eval_out_dev=None):
+        """q = (f - f(z)) / (X - z) (length - 1 Fr) and f(z) on the device; z: (8,) uint32 Montgomery."""
+        check(lib().ripp_fr_div_linear_dev(self.handle, _p(coeffs_dev), ctypes.c_size_t(length), _p(z), _p(q_out_dev),
+                                           _p(eval_out_dev)))
+
+    def pc_kzg_commit_dev(self, powers_dev, n_powers, coeffs_dev, length, out_dev):
+        check(lib().ripp_pc_kzg_commit_dev(self.handle, _p(powers_dev), ctypes.c_size_t(n_powers), _p(coeffs_dev),
+                                           ctypes.c_size_t(length), _p(out_dev)))
+
+    def pc_kzg_open_dev(self, powers_dev, n_powers, coeffs_dev, length, z, out_dev, eval_out_dev=None):
+        check(lib().ripp_pc_kzg_open_dev(self.handle, _p(powers_dev), ctypes.c_size_t(n_powers), _p(coeffs_dev),
+                                         ctypes.c_size_t(length), _p(z), _p(out_dev), _p(eval_out_dev)))
+
+    def pc_kzg_verify(self, vsrs, com, z, evaluation, proof):
+        """com, proof: (24,) uint32 affine; z, evaluation: (8,) uint32 Montgomery.  -> bool"""
+        acc = ctypes.c_int(0)
+        check(lib().ripp_pc_kzg_verify(self.handle, _p(vsrs), _p(com), _p(z), _p(evaluation), _p(proof), ctypes.byref(acc)))
+        return bool(acc.value)
+
+    def pc_commit_dev(self, first_dev, m, second_dev, n, coeffs_dev, length, y_coms_dev):
+        """-> GT (144,) uint32; y_coms_dev receives the n first-tier commitments."""
+        out = np.zeros(144, dtype=np.uint32)
+        check(lib().ripp_pc_commit_dev(self.handle, _p(first_dev), ctypes.c_size_t(m), _p(second_dev), ctypes.c_size_t(n),
+                                       _p(coeffs_dev), ctypes.c_size_t(length), _p(out), _p(y_coms_dev)))
+        return out
+
+    def pc_open_dev(self, kind, first_dev, m, second_dev, n, srs_g2_dev, coeffs_dev, length, y_coms_dev, x, y):
+        """-> (OpeningProof bytes, f(x, y) as (8,) uint32 Montgomery)."""
+        k = max(n.bit_length() - 1, 0) + max(m.bit_length() - 1, 0)
+        cap = 16 * 600 + k * 6 * 600
+        proof = np.empty(cap, dtype=np.uint8)
+        plen = ctypes.c_size_t()
+        ev = np.zeros(8, dtype=np.uint32)
+        check(lib().ripp_pc_open_dev(self.handle, int(kind), _p(first_dev), ctypes.c_size_t(m), _p(second_dev), ctypes.c_size_t(n),
+                                     _p(srs_g2_dev), _p(coeffs_dev), ctypes.c_size_t(length), _p(y_coms_dev), _p(x), _p(y),
+                                     _p(proof), ctypes.c_size_t(cap), ctypes.byref(plen), _p(ev)))
+        return proof[: plen.value].tobytes(), ev
+
+    def pc_verify(self, kind, vsrs, first_dev, m, second_dev, n, com, x, y, evaluation, proof):
+        """com: GT (144,) uint32; x, y, evaluation: (8,) uint32 Montgomery; proof: bytes.  -> bool"""
+        acc = ctypes.c_int(0)
+        pb = self._bytes(proof)
+        check(lib().ripp_pc_verify(self.handle, int(kind), _p(vsrs), _p(first_dev), ctypes.c_size_t(m), _p(second_dev),
+                                   ctypes.c_size_t(n), _p(com), _p(x), _p(y), _p(evaluation), _p(pb), ctypes.c_size_t(len(proof)),
+                                   ctypes.byref(acc)))
+        return bool(acc.value)
 
     # ---- verifiers --------------------------------------------------------------------------------
     def gt_multiexp_dev(self, gt_dev, fr_dev, n, out_dev):

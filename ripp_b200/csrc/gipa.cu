@@ -929,5 +929,6 @@ extern "C" int ripp_sipp_prove(ripp_ctx* ctx, const void* a_aff, const void* b_a
 
 #include "verify.cuh"
 #include "verify_batch.cuh"
+#include "poly_commit.cuh"
 #include "aggregate_batch.cuh"
 #include "sharded.cuh"

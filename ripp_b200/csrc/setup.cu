@@ -79,6 +79,12 @@ __global__ void k_fr_power_seq(Fr s, size_t n, Fr* __restrict__ out) {
   }
   out[i] = acc;
 }
+int ripp_fr_power_seq_internal(ripp_ctx* ctx, const Fr& s, size_t n, void* out_dev) {
+  if (n == 0) return RIPP_OK;
+  k_fr_power_seq<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(s, n, (Fr*)out_dev);
+  LAUNCHED(ctx);
+  return RIPP_OK;
+}
 
 int ripp_scale_base_g1(ripp_ctx* ctx, const G1Aff* base_or_null, const void* sc_dev, size_t n, void* out_dev);
 int ripp_scale_base_g2(ripp_ctx* ctx, const G2Aff* base_or_null, const void* sc_dev, size_t n, void* out_dev);
@@ -137,8 +143,7 @@ static int structured_generators(ripp_ctx* ctx, const void* base_host, const voi
   memcpy(s.v, s_host, sizeof(Fr));
   void* pw;
   OK(scratch(ctx, 25, num * sizeof(Fr) + 256, &pw));
-  k_fr_power_seq<<<(unsigned)((num + 127) / 128), 128, 0, ctx->stream>>>(s, num, (Fr*)pw);
-  LAUNCHED(ctx);
+  OK(ripp_fr_power_seq_internal(ctx, s, num, pw));
   return fixed_base_msm<F>(ctx, base_host, pw, num, out_dev);
 }
 extern "C" int ripp_structured_generators_g1_dev(ripp_ctx* ctx, const void* base_g1_aff, const void* s, size_t num, void* out_dev) {

@@ -1,24 +1,21 @@
-"""Host-side mirror of the polynomial-commitment application (ip_proofs/src/applications/poly_commit/mod.rs:
-KZG :52-131, BivariatePolynomialCommitment :153-284, UnivariatePolynomialCommitment :286-377) over the C ABI.
+"""The polynomial-commitment application (ip_proofs/src/applications/poly_commit/mod.rs: KZG :52-131,
+BivariatePolynomialCommitment :153-284, UnivariatePolynomialCommitment :286-377; transparent.rs) over the C ABI's
+`ripp_pc_*` entry points (csrc/poly_commit.cuh).
 
-Every group operation runs in the CUDA library: KZG commit / open are G1 MSMs over the device-resident powers
-(`ripp_msm_g1_dev`), the second-tier commitment is the AFGHO pairing product (`ripp_pairing_ip_dev`), the opening's
-inner-product argument is the resident TIPAWithSSM prover (`ripp_tipa_prove_dev`, kind MULTIEXP_SSM) and the verifier is
-`ripp_tipa_verify` plus one two-pair product for the KZG check.  The host does what the reference does in scalar code:
-padding, the X-power combination of the Y polynomials' coefficients (mod.rs:221-241) and the synthetic division of
-KZG::open (mod.rs:98-104).  Polynomials are coefficient lists of ints (lowest degree first); a bivariate polynomial is
-the list of its Y polynomials.  Setup takes alpha, beta explicitly (SURVEY.md §8d).  No CPU fallback: the context fails
-without a GPU."""
+Commit is one segmented MSM of the Y polynomials over the shared first-tier bases plus the AFGHO pairing product; open
+keeps the powers of x, the row combination y_eval, y_eval_comm, the KZG quotient and the inner-product arguments on the
+device; verify is `ripp_pc_verify`.  Polynomials are coefficient lists of ints (lowest degree first); a bivariate
+polynomial is the list of its Y polynomials.  The `*_dev` methods take the coefficients already on the device, row-major
+with row length y_degree + 1 (include/ripp_b200.h "Coefficient layout"; a univariate polynomial is already in it), so
+that large polynomials skip the host encoding.  Setup takes alpha, beta explicitly (SURVEY.md §8d).  No CPU fallback:
+the context fails without a GPU."""
 import math
-
-import numpy as np
 
 from . import _lib, codec
 from .inner_products import default_context
 from .ip_proofs import vsrs_enc
 
 R = codec.R
-_GT_ONE = ((1, 0),) + ((0, 0),) * 5
 
 
 def _powers(s, n):
@@ -45,16 +42,19 @@ def _v_srs(ctx, alpha, beta):
     return {"g": codec.g1_dec(g1[0]), "h": codec.g2_dec(g2[0]), "g_beta": codec.g1_dec(g1[1]), "h_alpha": codec.g2_dec(g2[1])}
 
 
-def _msm_g1(ctx, powers, n_powers, coeffs):
-    assert n_powers >= len(coeffs)  # mod.rs:85 / :98
-    sc = ctx.to_device(codec.fr_vec_enc(list(coeffs) + [0] * (n_powers - len(coeffs))))
-    out = ctx.alloc(96)
-    ctx.msm_g1_dev(powers, sc, n_powers, out)
-    ctx.sync()
-    pt = codec.g1_dec(out.download(24))
-    sc.free()
-    out.free()
-    return pt
+def _upload_fr(ctx, vals):
+    """-> (DeviceBuffer or None, length) of Montgomery Fr."""
+    vals = list(vals)
+    return (ctx.to_device(codec.fr_vec_enc(vals)) if vals else None), len(vals)
+
+
+def _flat(y_polynomials, m):
+    """Y polynomials -> the row-major coefficient list of row length m (rows past the given ones are implicit zeros)."""
+    flat = []
+    for yp in y_polynomials:
+        assert len(yp) <= m  # KZG::commit / Pedersen over m bases (mod.rs:85)
+        flat += list(yp) + [0] * (m - len(yp))
+    return flat
 
 
 def quotient_by_linear(coeffs, z):
@@ -68,12 +68,6 @@ def quotient_by_linear(coeffs, z):
     return q
 
 
-def _g1_from_bytes(b):
-    if b[0] & 0x40:
-        return None
-    return (int.from_bytes(b[:48], "big"), int.from_bytes(b[48:96], "big"))
-
-
 class KZG:
     """mod.rs:52-131.  `powers` is a (DeviceBuffer, count) pair of G1 affine points g^(alpha^i)."""
 
@@ -84,26 +78,27 @@ class KZG:
 
     @staticmethod
     def commit(powers, coeffs, ctx=None):
-        return _msm_g1(ctx or default_context(), powers[0], powers[1], coeffs)
+        ctx = ctx or default_context()
+        c, n = _upload_fr(ctx, coeffs)
+        out = ctx.alloc(96)
+        ctx.pc_kzg_commit_dev(powers[0], powers[1], c, n, out)
+        return codec.g1_dec(out.download(24))
 
     @staticmethod
     def open(powers, coeffs, point, ctx=None):
-        return _msm_g1(ctx or default_context(), powers[0], powers[1], quotient_by_linear(coeffs, point))
+        """-> the proof (mod.rs:92-106): the quotient by (X - point) on the device, then one MSM."""
+        ctx = ctx or default_context()
+        c, n = _upload_fr(ctx, coeffs)
+        out = ctx.alloc(96)
+        ctx.pc_kzg_open_dev(powers[0], powers[1], c, n, codec.fr_enc(point % R), out)
+        return codec.g1_dec(out.download(24))
 
     @staticmethod
     def verify(v_srs, com, point, evaluation, proof, ctx=None):
         """mod.rs:120-130: e(com - g eval, h) == e(proof, h_alpha - h point), as ONE two-pair product equal to 1."""
         ctx = ctx or default_context()
-        neg = None if proof is None else (proof[0], (-proof[1]) % codec.P)
-        g1 = ctx.to_device(np.stack([codec.g1_enc(v_srs["g"]), codec.g1_enc(com), codec.g1_enc(neg)]))
-        g2 = ctx.to_device(np.stack([codec.g2_enc(v_srs["h"]), codec.g2_enc(v_srs["h_alpha"])]))
-        # out = hi * c + lo with n = 1: slot 1 <- com - g eval ; G2 slot 1 <- h_alpha - h point
-        ctx.g1_fold_dev(g1.ptr, g1.ptr + 96, codec.fr_enc(-evaluation % R).copy(), 1, g1.ptr + 96)
-        ctx.g2_fold_dev(g2.ptr, g2.ptr + 192, codec.fr_enc(-point % R).copy(), 1, g2.ptr + 192)
-        out = ctx.alloc(576)
-        ctx.pairing_ip_dev(g1.ptr + 96, g2.ptr, 2, out)  # pairs (com - g eval, h), (-proof, h_alpha - h point)
-        ctx.sync()
-        return codec.gt_dec(out.download(144)) == _GT_ONE
+        return ctx.pc_kzg_verify(vsrs_enc(v_srs), codec.g1_enc(com), codec.fr_enc(point % R), codec.fr_enc(evaluation % R),
+                                 codec.g1_enc(proof))
 
 
 class BivariatePolynomialCommitment:
@@ -123,51 +118,53 @@ class BivariatePolynomialCommitment:
         }
 
     @staticmethod
-    def commit(srs, y_polynomials, ctx=None):
+    def commit_dev(srs, coeffs_dev, length, ctx=None):
+        """Coefficients on the device (row-major, row length y_degree + 1).  -> (com: GT, y_polynomial_comms: DeviceBuffer
+        of x_degree + 1 G1 affine points)."""
+        ctx = ctx or default_context()
+        n, m = srs["ck"][1], srs["kzg"][1]
+        y_coms = ctx.alloc(n * 96)
+        com = ctx.pc_commit_dev(srs["kzg"][0], m, srs["ck"][0], n, coeffs_dev, length, y_coms)
+        return codec.gt_dec(com), y_coms
+
+    @classmethod
+    def commit(cls, srs, y_polynomials, ctx=None):
         """-> (com: GT, y_polynomial_coms: list of G1)."""
         ctx = ctx or default_context()
-        n = srs["ck"][1]
-        assert n >= len(y_polynomials)  # mod.rs:186
-        padded = list(y_polynomials) + [[]] * (n - len(y_polynomials))
-        coms = [KZG.commit(srs["kzg"], yp, ctx) for yp in padded]
-        d = ctx.to_device(codec.g1_vec_enc(coms))
-        out = ctx.alloc(576)
-        ctx.pairing_ip_dev(d, srs["ck"][0], n, out)  # AFGHOCommitmentG1::commit(ck, coms) (afgho16/mod.rs:30-32)
-        ctx.sync()
-        return codec.gt_dec(out.download(144)), coms
+        assert srs["ck"][1] >= len(y_polynomials)  # mod.rs:186
+        c, n = _upload_fr(ctx, _flat(y_polynomials, srs["kzg"][1]))
+        com, y_coms = cls.commit_dev(srs, c, n, ctx)
+        return com, codec.g1_vec_dec(y_coms.download((srs["ck"][1], 24)))
 
     @staticmethod
-    def open(srs, y_polynomials, y_polynomial_comms, point, ctx=None):
-        """-> OpeningProof bytes: TIPAWithSSMProof || y_eval_comm || kzg_proof (field order of mod.rs:145-149)."""
+    def open_dev(srs, coeffs_dev, length, y_coms_dev, point, ctx=None):
+        """-> (OpeningProof bytes: TIPAWithSSMProof || y_eval_comm || kzg_proof (mod.rs:145-149), evaluation)."""
         ctx = ctx or default_context()
         x, y = point
         n, m = srs["ck"][1], srs["kzg"][1]
-        assert n >= len(y_polynomials)  # mod.rs:211
-        powers_of_x = _powers(x, n)
-        y_eval_coeffs = [0] * m
-        for i, yp in enumerate(y_polynomials):  # mod.rs:221-241
-            px = powers_of_x[i]
-            for j, c in enumerate(yp):
-                y_eval_coeffs[j] = (y_eval_coeffs[j] + px * c) % R
-        y_eval_comm = _msm_g1(ctx, srs["kzg"][0], m, y_eval_coeffs)
-        a = ctx.to_device(codec.g1_vec_enc(y_polynomial_comms))
-        b = ctx.to_device(codec.fr_vec_enc(powers_of_x))
-        ip_proof = ctx.tipa_prove_dev(_lib.GIPA_MULTIEXP_SSM, None, srs["h_beta_powers"][0], a, b, srs["ck"][0], None, n)
-        kzg_proof = KZG.open(srs["kzg"], y_eval_coeffs, y, ctx)
-        return ip_proof + codec.ser_g1(y_eval_comm) + codec.ser_g1(kzg_proof)
+        proof, ev = ctx.pc_open_dev(_lib.PC_TRUSTED, srs["kzg"][0], m, srs["ck"][0], n, srs["h_beta_powers"][0], coeffs_dev,
+                                    length, y_coms_dev, codec.fr_enc(x % R), codec.fr_enc(y % R))
+        return proof, codec.fr_dec(ev)
+
+    @classmethod
+    def open(cls, srs, y_polynomials, y_polynomial_comms, point, ctx=None):
+        """-> OpeningProof bytes: TIPAWithSSMProof || y_eval_comm || kzg_proof (field order of mod.rs:145-149)."""
+        ctx = ctx or default_context()
+        assert srs["ck"][1] >= len(y_polynomials)  # mod.rs:211
+        c, n = _upload_fr(ctx, _flat(y_polynomials, srs["kzg"][1]))
+        y_coms = ctx.to_device(codec.g1_vec_enc(y_polynomial_comms))
+        return cls.open_dev(srs, c, n, y_coms, point, ctx)[0]
 
     @staticmethod
     def verify(v_srs, com, point, evaluation, proof, ctx=None):
         ctx = ctx or default_context()
         x, y = point
-        ip_proof, y_eval_b, kzg_b = proof[:-192], proof[-192:-96], proof[-96:]
-        statement = codec.ser_gt(com) + codec.ser_identity_output(y_eval_b)
-        ip_ok = ctx.tipa_verify(_lib.GIPA_MULTIEXP_SSM, vsrs_enc(v_srs), statement, ip_proof, codec.fr_enc(x).copy())
-        return ip_ok and KZG.verify(v_srs, _g1_from_bytes(y_eval_b), y, evaluation, _g1_from_bytes(kzg_b), ctx)
+        return ctx.pc_verify(_lib.PC_TRUSTED, vsrs_enc(v_srs), None, 0, None, 0, codec.gt_enc(com), codec.fr_enc(x % R),
+                             codec.fr_enc(y % R), codec.fr_enc(evaluation % R), proof)
 
 
 class UnivariatePolynomialCommitment:
-    """mod.rs:286-377."""
+    """mod.rs:286-377.  The coefficients, read row-major with row length y_degree + 1, are the bivariate form."""
 
     @staticmethod
     def bivariate_degrees(univariate_degree):
@@ -192,14 +189,29 @@ class UnivariatePolynomialCommitment:
         return BivariatePolynomialCommitment.setup(xd, yd, alpha, beta, ctx)
 
     @classmethod
+    def commit_dev(cls, srs, coeffs_dev, length, ctx=None):
+        return BivariatePolynomialCommitment.commit_dev(srs, coeffs_dev, length, ctx)
+
+    @classmethod
     def commit(cls, srs, coeffs, ctx=None):
-        return BivariatePolynomialCommitment.commit(srs, cls.bivariate_form(cls.degrees_from_srs(srs), coeffs), ctx)
+        ctx = ctx or default_context()
+        n, m = srs["ck"][1], srs["kzg"][1]
+        c, length = _upload_fr(ctx, list(coeffs)[: n * m])
+        com, y_coms = cls.commit_dev(srs, c, length, ctx)
+        return com, codec.g1_vec_dec(y_coms.download((n, 24)))
+
+    @classmethod
+    def open_dev(cls, srs, coeffs_dev, length, y_coms_dev, point, ctx=None):
+        """-> (OpeningProof bytes, evaluation at point)."""
+        m = srs["kzg"][1]
+        return BivariatePolynomialCommitment.open_dev(srs, coeffs_dev, length, y_coms_dev, (pow(point, m, R), point), ctx)
 
     @classmethod
     def open(cls, srs, coeffs, y_polynomial_comms, point, ctx=None):
-        xd, yd = cls.degrees_from_srs(srs)
-        return BivariatePolynomialCommitment.open(srs, cls.bivariate_form((xd, yd), coeffs), y_polynomial_comms,
-                                                  (pow(point, yd + 1, R), point), ctx)
+        ctx = ctx or default_context()
+        n, m = srs["ck"][1], srs["kzg"][1]
+        c, length = _upload_fr(ctx, list(coeffs)[: n * m])
+        return cls.open_dev(srs, c, length, ctx.to_device(codec.g1_vec_enc(y_polynomial_comms)), point, ctx)[0]
 
     @classmethod
     def verify(cls, v_srs, max_degree, com, point, evaluation, proof, ctx=None):
@@ -209,15 +221,11 @@ class UnivariatePolynomialCommitment:
 
 # ------------------------------------------------------------------------------------------------
 # Transparent variant (applications/poly_commit/transparent.rs): no trusted setup.  First tier = Pedersen<G1>
-# commitments to the Y polynomials (MSMs over the first-tier key), second tier = AFGHO over them.  Openings are the two
-# GIPAs with structured scalar message (second tier: MULTIEXP_SSM; first tier: SCALAR_SSM_G1), both resident provers;
-# the verifier's final commitment keys are one MSM over each key vector (`ripp_gipa_verify_dev`).
+# commitments to the Y polynomials (one segmented MSM over the first-tier key), second tier = AFGHO over them.  Openings
+# are the two GIPAs with structured scalar message (second tier: MULTIEXP_SSM; first tier: SCALAR_SSM_G1); the
+# verifier's final commitment keys are one MSM over each key vector (`ripp_gipa_verify_dev`).
 # ck = dict(first=(DeviceBuffer, y_degree + 1) G1 points, second=(DeviceBuffer, x_degree + 1) G2 points).
 # ------------------------------------------------------------------------------------------------
-def _gipa_ssm_prove(ctx, kind, a_dev, b_dev, v_dev, n):
-    return ctx.gipa_prove_dev(kind, a_dev, b_dev, v_dev, None, n)[0]
-
-
 class TransparentBivariatePolynomialCommitment:
     """transparent.rs:85-213."""
 
@@ -229,59 +237,45 @@ class TransparentBivariatePolynomialCommitment:
                 "second": (ctx.to_device(codec.g2_vec_enc(second_tier_ck)), len(second_tier_ck))}
 
     @staticmethod
-    def commit(ck, y_polynomials, ctx=None):
+    def commit_dev(ck, coeffs_dev, length, ctx=None):
+        """-> (com: GT, y_polynomial_comms: DeviceBuffer of x_degree + 1 G1 affine points)."""
         ctx = ctx or default_context()
-        n = ck["second"][1]
-        assert n >= len(y_polynomials)  # :106
-        padded = list(y_polynomials) + [[]] * (n - len(y_polynomials))
-        coms = [_msm_g1(ctx, ck["first"][0], ck["first"][1], yp) for yp in padded]  # PedersenCommitment::commit (:119)
-        d = ctx.to_device(codec.g1_vec_enc(coms))
-        out = ctx.alloc(576)
-        ctx.pairing_ip_dev(d, ck["second"][0], n, out)
-        ctx.sync()
-        return codec.gt_dec(out.download(144)), coms
+        n, m = ck["second"][1], ck["first"][1]
+        y_coms = ctx.alloc(n * 96)
+        com = ctx.pc_commit_dev(ck["first"][0], m, ck["second"][0], n, coeffs_dev, length, y_coms)
+        return codec.gt_dec(com), y_coms
+
+    @classmethod
+    def commit(cls, ck, y_polynomials, ctx=None):
+        ctx = ctx or default_context()
+        assert ck["second"][1] >= len(y_polynomials)  # :106
+        c, n = _upload_fr(ctx, _flat(y_polynomials, ck["first"][1]))
+        com, y_coms = cls.commit_dev(ck, c, n, ctx)
+        return com, codec.g1_vec_dec(y_coms.download((ck["second"][1], 24)))
 
     @staticmethod
-    def open(ck, y_polynomials, y_polynomial_comms, point, ctx=None):
-        """-> OpeningProof bytes: second_tier_ip_proof || y_eval_comm || first_tier_ip_proof (:79-83)."""
+    def open_dev(ck, coeffs_dev, length, y_coms_dev, point, ctx=None):
+        """-> (OpeningProof bytes: second_tier_ip_proof || y_eval_comm || first_tier_ip_proof (:79-83), evaluation)."""
         ctx = ctx or default_context()
         x, y = point
         n, m = ck["second"][1], ck["first"][1]
-        assert n >= len(y_polynomials)  # :137
-        powers_of_x = _powers(x, n)
-        y_eval_coeffs = [0] * m
-        for i, yp in enumerate(y_polynomials):
-            px = powers_of_x[i]
-            for j, c in enumerate(yp):
-                y_eval_coeffs[j] = (y_eval_coeffs[j] + px * c) % R
-        y_eval_comm = _msm_g1(ctx, ck["first"][0], m, y_eval_coeffs)
-        a = ctx.to_device(codec.g1_vec_enc(y_polynomial_comms))
-        b = ctx.to_device(codec.fr_vec_enc(powers_of_x))
-        second = _gipa_ssm_prove(ctx, _lib.GIPA_MULTIEXP_SSM, a, b, ck["second"][0], n)
-        a1 = ctx.to_device(codec.fr_vec_enc(y_eval_coeffs))
-        b1 = ctx.to_device(codec.fr_vec_enc(_powers(y, m)))
-        first = _gipa_ssm_prove(ctx, _lib.GIPA_SCALAR_SSM_G1, a1, b1, ck["first"][0], m)
-        return second + codec.ser_g1(y_eval_comm) + first
+        proof, ev = ctx.pc_open_dev(_lib.PC_TRANSPARENT, ck["first"][0], m, ck["second"][0], n, None, coeffs_dev, length,
+                                    y_coms_dev, codec.fr_enc(x % R), codec.fr_enc(y % R))
+        return proof, codec.fr_dec(ev)
 
-    @staticmethod
-    def _split(proof, n):
-        """second-tier GIPAProof length for n = 2^k keys: 8 + k * 2 * (576 + 32 + 8 + 96) + 96 + 32."""
-        k = n.bit_length() - 1
-        s = 8 + k * 2 * (576 + 32 + 8 + 96) + 96 + 32
-        return proof[:s], proof[s:s + 96], proof[s + 96:]
+    @classmethod
+    def open(cls, ck, y_polynomials, y_polynomial_comms, point, ctx=None):
+        ctx = ctx or default_context()
+        assert ck["second"][1] >= len(y_polynomials)  # :137
+        c, n = _upload_fr(ctx, _flat(y_polynomials, ck["first"][1]))
+        return cls.open_dev(ck, c, n, ctx.to_device(codec.g1_vec_enc(y_polynomial_comms)), point, ctx)[0]
 
     @staticmethod
     def verify(ck, com, point, evaluation, proof, ctx=None):
         ctx = ctx or default_context()
         x, y = point
-        second, y_eval_b, first = TransparentBivariatePolynomialCommitment._split(proof, ck["second"][1])
-        st2 = codec.ser_gt(com) + codec.ser_identity_output(y_eval_b)
-        ok2 = ctx.gipa_verify_dev(_lib.GIPA_MULTIEXP_SSM, ck["second"][0], None, ck["second"][1], st2, second,
-                                  codec.fr_enc(x).copy())
-        st1 = y_eval_b + codec.ser_identity_output(codec.ser_fr(evaluation))
-        ok1 = ctx.gipa_verify_dev(_lib.GIPA_SCALAR_SSM_G1, ck["first"][0], None, ck["first"][1], st1, first,
-                                  codec.fr_enc(y).copy())
-        return ok2 and ok1
+        return ctx.pc_verify(_lib.PC_TRANSPARENT, None, ck["first"][0], ck["first"][1], ck["second"][0], ck["second"][1],
+                             codec.gt_enc(com), codec.fr_enc(x % R), codec.fr_enc(y % R), codec.fr_enc(evaluation % R), proof)
 
 
 class TransparentUnivariatePolynomialCommitment:
@@ -298,15 +292,28 @@ class TransparentUnivariatePolynomialCommitment:
         return ck["second"][1] - 1, ck["first"][1] - 1
 
     @classmethod
+    def commit_dev(cls, ck, coeffs_dev, length, ctx=None):
+        return TransparentBivariatePolynomialCommitment.commit_dev(ck, coeffs_dev, length, ctx)
+
+    @classmethod
     def commit(cls, ck, coeffs, ctx=None):
-        form = UnivariatePolynomialCommitment.bivariate_form(cls.degrees_from_ck(ck), coeffs)
-        return TransparentBivariatePolynomialCommitment.commit(ck, form, ctx)
+        ctx = ctx or default_context()
+        n, m = ck["second"][1], ck["first"][1]
+        c, length = _upload_fr(ctx, list(coeffs)[: n * m])
+        com, y_coms = cls.commit_dev(ck, c, length, ctx)
+        return com, codec.g1_vec_dec(y_coms.download((n, 24)))
+
+    @classmethod
+    def open_dev(cls, ck, coeffs_dev, length, y_coms_dev, point, ctx=None):
+        m = ck["first"][1]
+        return TransparentBivariatePolynomialCommitment.open_dev(ck, coeffs_dev, length, y_coms_dev, (pow(point, m, R), point), ctx)
 
     @classmethod
     def open(cls, ck, coeffs, y_polynomial_comms, point, ctx=None):
-        xd, yd = cls.degrees_from_ck(ck)
-        form = UnivariatePolynomialCommitment.bivariate_form((xd, yd), coeffs)
-        return TransparentBivariatePolynomialCommitment.open(ck, form, y_polynomial_comms, (pow(point, yd + 1, R), point), ctx)
+        ctx = ctx or default_context()
+        n, m = ck["second"][1], ck["first"][1]
+        c, length = _upload_fr(ctx, list(coeffs)[: n * m])
+        return cls.open_dev(ck, c, length, ctx.to_device(codec.g1_vec_enc(y_polynomial_comms)), point, ctx)[0]
 
     @classmethod
     def verify(cls, ck, com, point, evaluation, proof, ctx=None):

@@ -19,6 +19,7 @@
 pub mod commitments;
 pub mod inner_products;
 pub mod pack;
+pub mod poly_commit;
 pub mod resident;
 pub mod sipp;
 pub mod sipp377;
