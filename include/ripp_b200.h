@@ -528,7 +528,9 @@ int ripp_pc_commit_dev(ripp_ctx* ctx, const void* first_tier_dev, size_t m, cons
  * srs_g2_dev unused, GIPA MULTIEXP_SSM over (y_coms, powers of x) and GIPA SCALAR_SSM_G1 over (y_eval, powers of y).
  * Powers, the row combination y_eval, y_eval_comm and the quotient stay on the device.  proof_out: the OpeningProof
  * bytes (trusted: ip_proof || y_eval_comm || kzg_proof; transparent: second_tier_ip_proof || y_eval_comm ||
- * first_tier_ip_proof); eval_out (host, nullable): f(x, y).  Synchronous. */
+ * first_tier_ip_proof); eval_out (host, nullable): f(x, y).  The trusted opening needs n >= 2 (a TIPA of one element
+ * has no challenge for its KZG opening; the reference panics at tipa/mod.rs:199): n = 1 gives RIPP_ERR_ARG before any
+ * work is launched.  Synchronous. */
 int ripp_pc_open_dev(ripp_ctx* ctx, int kind, const void* first_tier_dev, size_t m, const void* second_tier_dev, size_t n,
                      const void* srs_g2_dev, const void* coeffs_dev, size_t len, const void* y_coms_dev, const void* x_host,
                      const void* y_host, uint8_t* proof_out, size_t proof_cap, size_t* proof_len, void* eval_out);

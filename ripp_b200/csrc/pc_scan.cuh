@@ -1,5 +1,5 @@
 // The Fr rules of the polynomial-commitment kernels (poly_commit.cuh), host and device, so that a host build
-// (tests/hostsim/hostsim_pc.cpp) can check them against the oracle.
+// (tests/hostsim/hostsim_pc.cpp) can check them against the oracle, and the row combination's grouping.
 //
 // Division by (X - z) (poly_commit/mod.rs:98-104) is the backward linear recurrence
 //   s_N = 0,  s_k = c_k + z s_(k+1)   (k = N-1 .. 0)
@@ -46,6 +46,20 @@ RIPP_HD Fr pow(Fr s, uint64_t e) {
     s = s * s;
   }
   return acc;
+}
+
+static const size_t ROW_THREADS = (size_t)1 << 16;  // threads the row combination aims for (columns x row groups)
+static const size_t MAX_ROW_GROUPS = 65535;         // the groups are k_pc_rows' gridDim.y
+
+// G groups of R rows for the row combination of n rows of m (k_pc_rows / k_pc_rows_combine): G m about ROW_THREADS,
+// G <= MAX_ROW_GROUPS (only n = 2^16, m = 1 hits the cap: R = 2, G = 2^15), G R >= n > (G - 1) R
+RIPP_HD void row_groups(size_t n, size_t m, size_t* G, size_t* R) {
+  size_t g = ROW_THREADS / m;
+  if (g < 1) g = 1;
+  if (g > n) g = n;
+  if (g > MAX_ROW_GROUPS) g = MAX_ROW_GROUPS;
+  *R = (n + g - 1) / g;
+  *G = (n + *R - 1) / *R;
 }
 
 }  // namespace pc

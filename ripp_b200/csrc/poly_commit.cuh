@@ -16,7 +16,6 @@
 int ripp_fr_power_seq_internal(ripp_ctx* ctx, const Fr& s, size_t n, void* out_dev);  // setup.cu: out[i] = s^i
 
 static const size_t PC_CHUNK = 32;      // L: coefficients per thread of the division scan
-static const size_t PC_ROW_THREADS = 1 << 16;  // threads the row combination aims for (columns x row groups)
 
 __global__ void k_pc_div_heads(const Fr* __restrict__ c, size_t N, Fr z, Fr* __restrict__ heads) {
   size_t b = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -93,18 +92,10 @@ static int div_linear(ripp_ctx* ctx, const Fr* c, size_t len, const Fr& z, Fr* t
   return div_scan(ctx, c, len, z, tmp, eval, q);
 }
 
-// G groups of R rows for the row combination
-static void row_groups(size_t n, size_t m, size_t* G, size_t* R) {
-  size_t g = PC_ROW_THREADS / m;
-  if (g < 1) g = 1;
-  if (g > n) g = n;
-  *R = (n + g - 1) / g;
-  *G = (n + *R - 1) / *R;
-}
 // y[j] = sum_i x^i C[i m + j] over n rows, zeros from len on; part: G m Fr (unused when G == 1)
 static int row_combination(ripp_ctx* ctx, const Fr* C, size_t len, size_t m, size_t n, const Fr& x, Fr* part, Fr* y) {
   size_t G, R;
-  row_groups(n, m, &G, &R);
+  pc::row_groups(n, m, &G, &R);
   dim3 grid((unsigned)((m + 127) / 128), (unsigned)G);
   k_pc_rows<<<grid, 128, 0, ctx->stream>>>(C, len, m, n, R, x, G == 1 ? y : part);
   LAUNCHED(ctx);
@@ -244,11 +235,13 @@ extern "C" int ripp_pc_open_dev(ripp_ctx* ctx, int kind, const void* first_tier_
   if (kind != RIPP_PC_TRUSTED && kind != RIPP_PC_TRANSPARENT) return fail(RIPP_ERR_ARG, "bad polynomial-commitment kind");
   if (kind == RIPP_PC_TRUSTED && !srs_g2_dev) return fail(RIPP_ERR_ARG, "the trusted opening needs h_beta_powers");
   OK(pc_shape(n, m, len));
+  // tipa_prove's own check, made before any launch: the reference panics on a one-row TIPA (tipa/mod.rs:199)
+  if (kind == RIPP_PC_TRUSTED && n < 2) return fail(RIPP_ERR_ARG, "the trusted opening needs at least two rows (TIPA of length 1)");
   CU(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const Fr x = fr_host(x_host), y = fr_host(y_host);
   size_t G, R;
-  row_groups(n, m, &G, &R);
+  pc::row_groups(n, m, &G, &R);
   // workspace: powers of x (n) | y_eval (m) | powers of y or the quotient (m) | row partials (G m) | scan (div) |
   // eval (1) | y_eval_comm, kzg proof (2 G1)
   const size_t o_px = 0, o_ye = o_px + n, o_q = o_ye + m, o_part = o_q + m, o_tmp = o_part + (G > 1 ? G * m : 0),

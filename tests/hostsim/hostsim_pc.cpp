@@ -1,6 +1,6 @@
 // Host-simulation build of the polynomial-commitment rules of ripp_b200/csrc/pc_scan.cuh (TEST INFRASTRUCTURE ONLY):
 // the chunked division scan of k_pc_div_heads / k_pc_div_replay, driven level by level as div_scan (poly_commit.cuh)
-// drives it but with the chunk length L as a parameter, and the row combination's Horner step, so that
+// drives it but with the chunk length L as a parameter, and the row combination's Horner step and grouping, so that
 // tests/test_hostsim_pc.py can compare them with the oracle.
 #define RIPP_HOSTSIM 1
 #include "../../ripp_b200/csrc/pc_scan.cuh"
@@ -63,4 +63,7 @@ void hs_rows(const uint32_t* coeffs, size_t len, size_t m, size_t n, size_t R, c
     memcpy(y + 8 * j, &acc, sizeof(Fr));
   }
 }
+
+// the row combination's G groups of R rows for n rows of m (pc::row_groups, as ripp_pc_open_dev picks them)
+void hs_row_groups(size_t n, size_t m, size_t* G, size_t* R) { pc::row_groups(n, m, G, R); }
 }
