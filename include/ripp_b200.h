@@ -542,6 +542,28 @@ int ripp_pc_verify(ripp_ctx* ctx, int kind, const void* vsrs, const void* first_
                    size_t n, const void* com_gt, const void* x_host, const void* y_host, const void* eval, const uint8_t* proof,
                    size_t proof_len, int* accept);
 
+/* Many polynomials under ONE key in one call: count polynomials of the same shape (n, m as ripp_pc_commit_dev).
+ * coeffs_dev: HOST array of count device pointers (NULL allowed iff lens[k] == 0; the same pointer may repeat), lens:
+ * count lengths (layout of "Coefficient layout").  The checks run in the single entry points' order and before any
+ * work is queued: null pointers and a bad kind, then the shape (RIPP_ERR_NOT_POW2 before RIPP_ERR_ARG), then the trusted
+ * opening's n >= 2, then lens[k] <= n m (the message names k).  The single path's limits apply to the whole batch:
+ * count n <= 2^16 and count n m <= 2^24, else RIPP_ERR_ARG.  count == 0 returns RIPP_OK.  The number of kernel
+ * launches and host synchronisations depends on (kind, n, m), not on count.
+ *
+ * Commit: gt_out: count x 576 B (host); y_coms_dev: count x n G1 affine (device), polynomial k at element k n.  Result k
+ * is byte for byte what ripp_pc_commit_dev returns for polynomial k alone.  Synchronous. */
+int ripp_pc_commit_batch_dev(ripp_ctx* ctx, const void* first_tier_dev, size_t m, const void* second_tier_dev, size_t n,
+                             size_t count, const void* const* coeffs_dev, const size_t* lens, void* gt_out, void* y_coms_dev);
+/* Open polynomial k at (x[k], y[k]) (host, count Fr each), y_coms_dev as ripp_pc_commit_batch_dev writes it.  The count
+ * second-tier recursions (and, transparent, the count first-tier ones) run in lock step.  proofs_out: count
+ * OpeningProofs back to back, *proof_len bytes each (the length depends on kind, n, m only); proofs_cap < count x
+ * *proof_len gives RIPP_ERR_ARG with *proof_len set; count == 0 sets *proof_len = 0.  evals_out (host, nullable): count
+ * Fr.  Proof k and eval k are byte for byte what ripp_pc_open_dev returns for instance k alone.  Synchronous. */
+int ripp_pc_open_batch_dev(ripp_ctx* ctx, int kind, const void* first_tier_dev, size_t m, const void* second_tier_dev,
+                           size_t n, const void* srs_g2_dev, size_t count, const void* const* coeffs_dev, const size_t* lens,
+                           const void* y_coms_dev, const void* x_host, const void* y_host, uint8_t* proofs_out,
+                           size_t proofs_cap, size_t* proof_len, void* evals_out);
+
 /* ---- diagnostics --------------------------------------------------------------------------- */
 /* Element-wise primitive ops on device, used by the GPU parity tests to pin the PTX limb layer:
  * op in ripp_test_op; a, b, r are HOST arrays of n elements of the op's operand size. */

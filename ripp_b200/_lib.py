@@ -543,6 +543,43 @@ class Context:
                                      _p(proof), ctypes.c_size_t(cap), ctypes.byref(plen), _p(ev)))
         return proof[: plen.value].tobytes(), ev
 
+    @staticmethod
+    def _pc_batch_args(coeffs_devs, lengths):
+        count = len(coeffs_devs)
+        ptrs = (ctypes.c_void_p * max(count, 1))(*[_p(c).value or 0 for c in coeffs_devs])
+        lens = np.array(list(lengths) or [0], dtype=np.uintp)
+        return count, ptrs, lens
+
+    def pc_commit_batch_dev(self, first_dev, m, second_dev, n, coeffs_devs, lengths, y_coms_dev):
+        """count polynomials under one key -> (count, 144) uint32 GT; y_coms_dev receives count x n G1 (polynomial k at
+        element k n)."""
+        count, ptrs, lens = self._pc_batch_args(coeffs_devs, lengths)
+        out = np.zeros((max(count, 1), 144), dtype=np.uint32)
+        check(lib().ripp_pc_commit_batch_dev(self.handle, _p(first_dev), ctypes.c_size_t(m), _p(second_dev), ctypes.c_size_t(n),
+                                             ctypes.c_size_t(count), ptrs, _p(lens), _p(out), _p(y_coms_dev)))
+        return out[:count]
+
+    def pc_open_batch_dev(self, kind, first_dev, m, second_dev, n, srs_g2_dev, coeffs_devs, lengths, y_coms_dev, xs, ys):
+        """xs, ys: (count, 8) uint32 Montgomery.  -> (list of OpeningProof bytes, (count, 8) uint32 evaluations)."""
+        count, ptrs, lens = self._pc_batch_args(coeffs_devs, lengths)
+        xs = np.ascontiguousarray(np.asarray(xs, dtype=np.uint32).reshape(-1, 8) if count else np.zeros((1, 8), np.uint32))
+        ys = np.ascontiguousarray(np.asarray(ys, dtype=np.uint32).reshape(-1, 8) if count else np.zeros((1, 8), np.uint32))
+        plen = ctypes.c_size_t()
+        # the length depends on (kind, n, m) only: ask with an empty buffer, then open
+        st = lib().ripp_pc_open_batch_dev(self.handle, int(kind), _p(first_dev), ctypes.c_size_t(m), _p(second_dev), ctypes.c_size_t(n),
+                                          _p(srs_g2_dev), ctypes.c_size_t(count), ptrs, _p(lens), _p(y_coms_dev), _p(xs), _p(ys),
+                                          _p(None), ctypes.c_size_t(0), ctypes.byref(plen), _p(None))
+        if count == 0 or st != RIPP_ERR_ARG or plen.value == 0:
+            check(st)
+            return [], np.zeros((0, 8), dtype=np.uint32)
+        proofs = np.empty(count * plen.value, dtype=np.uint8)
+        ev = np.zeros((count, 8), dtype=np.uint32)
+        check(lib().ripp_pc_open_batch_dev(self.handle, int(kind), _p(first_dev), ctypes.c_size_t(m), _p(second_dev), ctypes.c_size_t(n),
+                                           _p(srs_g2_dev), ctypes.c_size_t(count), ptrs, _p(lens), _p(y_coms_dev), _p(xs), _p(ys),
+                                           _p(proofs), ctypes.c_size_t(proofs.nbytes), ctypes.byref(plen), _p(ev)))
+        L = plen.value
+        return [proofs[k * L:(k + 1) * L].tobytes() for k in range(count)], ev
+
     def pc_verify(self, kind, vsrs, first_dev, m, second_dev, n, com, x, y, evaluation, proof):
         """com: GT (144,) uint32; x, y, evaluation: (8,) uint32 Montgomery; proof: bytes.  -> bool"""
         acc = ctypes.c_int(0)

@@ -17,7 +17,7 @@ using namespace ripp;
 // ------------------------------------------------------------------------------------------------
 std::string& ripp_err_slot();
 
-#define RIPP_SCRATCH_SLOTS 48
+#define RIPP_SCRATCH_SLOTS 52
 #define RIPP_MAX_BATCH 8
 #define RIPP_MAX_CHILD 8
 // per-category device-time accounting (CUDA events on the context's stream; off by default)

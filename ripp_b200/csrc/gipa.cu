@@ -931,4 +931,5 @@ extern "C" int ripp_sipp_prove(ripp_ctx* ctx, const void* a_aff, const void* b_a
 #include "verify_batch.cuh"
 #include "poly_commit.cuh"
 #include "aggregate_batch.cuh"
+#include "pc_batch.cuh"
 #include "sharded.cuh"

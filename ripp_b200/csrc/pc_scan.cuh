@@ -62,5 +62,39 @@ RIPP_HD void row_groups(size_t n, size_t m, size_t* G, size_t* R) {
   *G = (n + *R - 1) / *R;
 }
 
+// ---- the batched kernels (pc_batch.cuh): count instances of equal shape, instance k's elements at k x its length ----
+
+// instance k and element e of flat index i over segments of `len` elements
+RIPP_HD void seg_split(size_t i, size_t len, size_t* k, size_t* e) {
+  *k = i / len;
+  *e = i - *k * len;
+}
+
+// G groups of R rows for the row combination of `count` polynomials of n rows of m (k_pc_rows_seg): G m count about
+// ROW_THREADS, G R >= n > (G - 1) R.  The launch is one-dimensional over count G m <= 2^24 threads, so no grid dimension
+// caps G (row_blocks).
+RIPP_HD void row_groups_batch(size_t count, size_t n, size_t m, size_t* G, size_t* R) {
+  size_t g = ROW_THREADS / (m * count);
+  if (g < 1) g = 1;
+  if (g > n) g = n;
+  *R = (n + g - 1) / g;
+  *G = (n + *R - 1) / *R;
+}
+
+// blocks of 128 threads of k_pc_rows_seg: thread i is column j of group g of instance k, i = (k G + g) m + j
+RIPP_HD size_t row_blocks(size_t count, size_t G, size_t m) { return (count * G * m + 127) / 128; }
+
+RIPP_HD void row_index(size_t i, size_t G, size_t m, size_t* k, size_t* g, size_t* j) {
+  size_t r;
+  seg_split(i, G * m, k, &r);
+  seg_split(r, m, g, j);
+}
+
+// s^(2^e): the segmented scan's point at level l is z^(L^l) = z^(2^(5 l)) for chunks of L = 32
+RIPP_HD Fr pow2k(Fr s, unsigned e) {
+  for (unsigned i = 0; i < e; i++) s = s * s;
+  return s;
+}
+
 }  // namespace pc
 }  // namespace ripp

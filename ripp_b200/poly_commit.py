@@ -57,6 +57,40 @@ def _flat(y_polynomials, m):
     return flat
 
 
+def _commit_batch_dev(ctx, first, second, coeffs_devs, lengths):
+    """ripp_pc_commit_batch_dev under the key (first, second) = ((DeviceBuffer, m), (DeviceBuffer, n))."""
+    ctx = ctx or default_context()
+    (f, m), (s, n) = first, second
+    y_coms = ctx.alloc(max(len(coeffs_devs), 1) * n * 96)
+    coms = ctx.pc_commit_batch_dev(f, m, s, n, coeffs_devs, lengths, y_coms)
+    return [codec.gt_dec(c) for c in coms], y_coms
+
+
+def _open_batch_dev(ctx, kind, first, second, srs_g2, coeffs_devs, lengths, y_coms_dev, points):
+    ctx = ctx or default_context()
+    (f, m), (s, n) = first, second
+    xs = [codec.fr_enc(x % R) for x, _ in points]
+    ys = [codec.fr_enc(y % R) for _, y in points]
+    proofs, ev = ctx.pc_open_batch_dev(kind, f, m, s, n, srs_g2, coeffs_devs, lengths, y_coms_dev, xs, ys)
+    return proofs, [codec.fr_dec(e) for e in ev]
+
+
+def _commit_batch(cls, key, flats, n, ctx):
+    """flats[k]: row-major coefficients of polynomial k.  -> list of (com, y_polynomial_coms)."""
+    ctx = ctx or default_context()
+    bufs = [_upload_fr(ctx, c) for c in flats]
+    coms, y_coms = cls.commit_batch_dev(key, [b for b, _ in bufs], [k for _, k in bufs], ctx)
+    ys = y_coms.download((max(len(flats), 1) * n, 24))
+    return [(com, codec.g1_vec_dec(ys[k * n:(k + 1) * n])) for k, com in enumerate(coms)]
+
+
+def _open_batch(cls, key, flats, y_polynomial_comms, points, ctx):
+    ctx = ctx or default_context()
+    bufs = [_upload_fr(ctx, c) for c in flats]
+    y_coms = ctx.to_device(codec.g1_vec_enc([p for coms in y_polynomial_comms for p in coms])) if flats else None
+    return cls.open_batch_dev(key, [b for b, _ in bufs], [k for _, k in bufs], y_coms, points, ctx)[0]
+
+
 def quotient_by_linear(coeffs, z):
     """mod.rs:98-104: polynomial / (X - z), remainder dropped."""
     if len(coeffs) < 2:
@@ -156,6 +190,28 @@ class BivariatePolynomialCommitment:
         return cls.open_dev(srs, c, n, y_coms, point, ctx)[0]
 
     @staticmethod
+    def commit_batch_dev(srs, coeffs_devs, lengths, ctx=None):
+        """Many polynomials under srs in one call.  -> (list of com: GT, y_coms: DeviceBuffer of count x (x_degree + 1) G1,
+        polynomial k at element k (x_degree + 1))."""
+        return _commit_batch_dev(ctx, srs["kzg"], srs["ck"], coeffs_devs, lengths)
+
+    @staticmethod
+    def open_batch_dev(srs, coeffs_devs, lengths, y_coms_dev, points, ctx=None):
+        """points[k] = (x, y).  -> (list of OpeningProof bytes, list of evaluations); entry k as open_dev returns it."""
+        return _open_batch_dev(ctx, _lib.PC_TRUSTED, srs["kzg"], srs["ck"], srs["h_beta_powers"][0], coeffs_devs, lengths,
+                               y_coms_dev, points)
+
+    @classmethod
+    def commit_batch(cls, srs, polynomials, ctx=None):
+        """polynomials[k]: a list of Y polynomials.  -> list of (com, y_polynomial_coms)."""
+        return _commit_batch(cls, srs, [_flat(p, srs["kzg"][1]) for p in polynomials], srs["ck"][1], ctx)
+
+    @classmethod
+    def open_batch(cls, srs, polynomials, y_polynomial_comms, points, ctx=None):
+        """-> list of OpeningProof bytes."""
+        return _open_batch(cls, srs, [_flat(p, srs["kzg"][1]) for p in polynomials], y_polynomial_comms, points, ctx)
+
+    @staticmethod
     def verify(v_srs, com, point, evaluation, proof, ctx=None):
         ctx = ctx or default_context()
         x, y = point
@@ -212,6 +268,27 @@ class UnivariatePolynomialCommitment:
         n, m = srs["ck"][1], srs["kzg"][1]
         c, length = _upload_fr(ctx, list(coeffs)[: n * m])
         return cls.open_dev(srs, c, length, ctx.to_device(codec.g1_vec_enc(y_polynomial_comms)), point, ctx)[0]
+
+    @classmethod
+    def commit_batch_dev(cls, srs, coeffs_devs, lengths, ctx=None):
+        return BivariatePolynomialCommitment.commit_batch_dev(srs, coeffs_devs, lengths, ctx)
+
+    @classmethod
+    def open_batch_dev(cls, srs, coeffs_devs, lengths, y_coms_dev, points, ctx=None):
+        """points[k] = z_k, opened at (z_k^m, z_k)."""
+        m = srs["kzg"][1]
+        return BivariatePolynomialCommitment.open_batch_dev(srs, coeffs_devs, lengths, y_coms_dev,
+                                                            [(pow(z, m, R), z) for z in points], ctx)
+
+    @classmethod
+    def commit_batch(cls, srs, polynomials, ctx=None):
+        n, m = srs["ck"][1], srs["kzg"][1]
+        return _commit_batch(cls, srs, [list(c)[: n * m] for c in polynomials], n, ctx)
+
+    @classmethod
+    def open_batch(cls, srs, polynomials, y_polynomial_comms, points, ctx=None):
+        n, m = srs["ck"][1], srs["kzg"][1]
+        return _open_batch(cls, srs, [list(c)[: n * m] for c in polynomials], y_polynomial_comms, points, ctx)
 
     @classmethod
     def verify(cls, v_srs, max_degree, com, point, evaluation, proof, ctx=None):
@@ -271,6 +348,24 @@ class TransparentBivariatePolynomialCommitment:
         return cls.open_dev(ck, c, n, ctx.to_device(codec.g1_vec_enc(y_polynomial_comms)), point, ctx)[0]
 
     @staticmethod
+    def commit_batch_dev(ck, coeffs_devs, lengths, ctx=None):
+        """-> (list of com: GT, y_coms: DeviceBuffer of count x (x_degree + 1) G1)."""
+        return _commit_batch_dev(ctx, ck["first"], ck["second"], coeffs_devs, lengths)
+
+    @staticmethod
+    def open_batch_dev(ck, coeffs_devs, lengths, y_coms_dev, points, ctx=None):
+        """points[k] = (x, y).  -> (list of OpeningProof bytes, list of evaluations)."""
+        return _open_batch_dev(ctx, _lib.PC_TRANSPARENT, ck["first"], ck["second"], None, coeffs_devs, lengths, y_coms_dev, points)
+
+    @classmethod
+    def commit_batch(cls, ck, polynomials, ctx=None):
+        return _commit_batch(cls, ck, [_flat(p, ck["first"][1]) for p in polynomials], ck["second"][1], ctx)
+
+    @classmethod
+    def open_batch(cls, ck, polynomials, y_polynomial_comms, points, ctx=None):
+        return _open_batch(cls, ck, [_flat(p, ck["first"][1]) for p in polynomials], y_polynomial_comms, points, ctx)
+
+    @staticmethod
     def verify(ck, com, point, evaluation, proof, ctx=None):
         ctx = ctx or default_context()
         x, y = point
@@ -314,6 +409,27 @@ class TransparentUnivariatePolynomialCommitment:
         n, m = ck["second"][1], ck["first"][1]
         c, length = _upload_fr(ctx, list(coeffs)[: n * m])
         return cls.open_dev(ck, c, length, ctx.to_device(codec.g1_vec_enc(y_polynomial_comms)), point, ctx)[0]
+
+    @classmethod
+    def commit_batch_dev(cls, ck, coeffs_devs, lengths, ctx=None):
+        return TransparentBivariatePolynomialCommitment.commit_batch_dev(ck, coeffs_devs, lengths, ctx)
+
+    @classmethod
+    def open_batch_dev(cls, ck, coeffs_devs, lengths, y_coms_dev, points, ctx=None):
+        """points[k] = z_k, opened at (z_k^m, z_k)."""
+        m = ck["first"][1]
+        return TransparentBivariatePolynomialCommitment.open_batch_dev(ck, coeffs_devs, lengths, y_coms_dev,
+                                                                       [(pow(z, m, R), z) for z in points], ctx)
+
+    @classmethod
+    def commit_batch(cls, ck, polynomials, ctx=None):
+        n, m = ck["second"][1], ck["first"][1]
+        return _commit_batch(cls, ck, [list(c)[: n * m] for c in polynomials], n, ctx)
+
+    @classmethod
+    def open_batch(cls, ck, polynomials, y_polynomial_comms, points, ctx=None):
+        n, m = ck["second"][1], ck["first"][1]
+        return _open_batch(cls, ck, [list(c)[: n * m] for c in polynomials], y_polynomial_comms, points, ctx)
 
     @classmethod
     def verify(cls, ck, com, point, evaluation, proof, ctx=None):

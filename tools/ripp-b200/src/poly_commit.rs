@@ -129,6 +129,50 @@ impl PcKeys {
         Ok((buf, pack::get_fr(&ev)))
     }
 
+    /// `commit` of many polynomials under these keys in one call (`ripp_pc_commit_batch_dev`).  -> (the commitments,
+    /// the y_polynomial_comms of polynomial k at elements k (x_degree + 1) .. of one device vector)
+    pub fn commit_batch(&self, coeffs: &[&DeviceVec<Fr>])
+                        -> Result<(Vec<PairingOutput<ark_bls12_381::Bls12_381>>, DeviceVec<G1Affine>), Error> {
+        let (n, m, count) = (self.second.len(), self.first.len(), coeffs.len());
+        let y_coms = DeviceVec::<G1Affine>::alloc(count.max(1) * n)?;
+        let ptrs: Vec<*const c_void> = coeffs.iter().map(|c| c.ptr()).collect();
+        let lens: Vec<usize> = coeffs.iter().map(|c| c.len()).collect();
+        let mut gt = vec![0u64; 72 * count.max(1)];
+        let c = ctx();
+        let st = unsafe {
+            sys::ripp_pc_commit_batch_dev(c.raw(), self.first.ptr(), m, self.second.ptr(), n, count, ptrs.as_ptr(), lens.as_ptr(),
+                                          gt.as_mut_ptr() as *mut c_void, y_coms.ptr_mut())
+        };
+        drop(c);
+        check(st, n, m)?;
+        Ok(((0..count).map(|k| PairingOutput(pack::get_fq12(&gt[72 * k..72 * (k + 1)]))).collect(), y_coms))
+    }
+
+    /// `open` of polynomial k at points[k] for every k in one call (`ripp_pc_open_batch_dev`), `y_coms` as
+    /// `commit_batch` returns it.  -> (OpeningProof bytes, f_k(x_k, y_k)) per polynomial
+    pub fn open_batch(&self, coeffs: &[&DeviceVec<Fr>], y_coms: &DeviceVec<G1Affine>, points: &[(Fr, Fr)])
+                      -> Result<Vec<(Vec<u8>, Fr)>, Error> {
+        let (n, m, count) = (self.second.len(), self.first.len(), coeffs.len());
+        assert_eq!(points.len(), count);
+        let ptrs: Vec<*const c_void> = coeffs.iter().map(|c| c.ptr()).collect();
+        let lens: Vec<usize> = coeffs.iter().map(|c| c.len()).collect();
+        let xs = pack::pack_fr(&points.iter().map(|p| p.0).collect::<Vec<_>>());
+        let ys = pack::pack_fr(&points.iter().map(|p| p.1).collect::<Vec<_>>());
+        let g2 = self.h_beta_powers.as_ref().map_or(std::ptr::null(), |h| h.ptr());
+        let mut buf = vec![0u8; count * proof_capacity(n, m)];
+        let mut len = 0usize;
+        let mut ev = vec![0u64; 4 * count.max(1)];
+        let c = ctx();
+        let st = unsafe {
+            sys::ripp_pc_open_batch_dev(c.raw(), self.kind(), self.first.ptr(), m, self.second.ptr(), n, g2, count, ptrs.as_ptr(),
+                                        lens.as_ptr(), y_coms.ptr(), xs.as_ptr() as *const c_void, ys.as_ptr() as *const c_void,
+                                        buf.as_mut_ptr(), buf.len(), &mut len, ev.as_mut_ptr() as *mut c_void)
+        };
+        drop(c);
+        check(st, n, m)?;
+        Ok((0..count).map(|k| (buf[k * len..(k + 1) * len].to_vec(), pack::get_fr(&ev[4 * k..4 * k + 4]))).collect())
+    }
+
     /// `verify` of an opening of `com` at (x, y) to `evaluation`.
     pub fn verify(&self, com: &PairingOutput<ark_bls12_381::Bls12_381>, point: (&Fr, &Fr), evaluation: &Fr, proof: &[u8])
                   -> Result<bool, Error> {
@@ -172,5 +216,14 @@ impl<'a> Univariate<'a> {
     }
     pub fn verify(&self, com: &PairingOutput<ark_bls12_381::Bls12_381>, z: &Fr, evaluation: &Fr, proof: &[u8]) -> Result<bool, Error> {
         self.0.verify(com, (&self.point(z), z), evaluation, proof)
+    }
+    pub fn commit_batch(&self, coeffs: &[&DeviceVec<Fr>])
+                        -> Result<(Vec<PairingOutput<ark_bls12_381::Bls12_381>>, DeviceVec<G1Affine>), Error> {
+        self.0.commit_batch(coeffs)
+    }
+    /// polynomial k opened at zs[k], i.e. at (zs[k]^(y_degree + 1), zs[k])
+    pub fn open_batch(&self, coeffs: &[&DeviceVec<Fr>], y_coms: &DeviceVec<G1Affine>, zs: &[Fr]) -> Result<Vec<(Vec<u8>, Fr)>, Error> {
+        let points: Vec<(Fr, Fr)> = zs.iter().map(|z| (self.point(z), *z)).collect();
+        self.0.open_batch(coeffs, y_coms, &points)
     }
 }
