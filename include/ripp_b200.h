@@ -563,6 +563,26 @@ int ripp_pc_open_batch_dev(ripp_ctx* ctx, int kind, const void* first_tier_dev, 
                            size_t n, const void* srs_g2_dev, size_t count, const void* const* coeffs_dev, const size_t* lens,
                            const void* y_coms_dev, const void* x_host, const void* y_host, uint8_t* proofs_out,
                            size_t proofs_cap, size_t* proof_len, void* evals_out);
+/* Verify `count` openings in one call, one status per opening: the arguments of ripp_pc_verify once per opening.
+ * com_gts: count x 576 B of GT; x_host, y_host, evals: count Fr each (host, Montgomery); proofs: the OpeningProof bytes
+ * back to back, proof_lens[k] bytes for opening k, proofs_len in all.  The trusted kind uses vsrs only (the keys, n and m
+ * are unused), so trusted openings of different shapes under one VerifierSRS may share a call; the transparent kind
+ * takes the first / second-tier keys with m, n, shared by all openings.
+ * status_out[k] (a ripp_agg_status) is what ripp_pc_verify reports for opening k alone: accept gives RIPP_AGG_OK,
+ * accept = 0 RIPP_AGG_REJECTED, RIPP_ERR_ARG for bytes that do not decode (length, non-canonical element, point off the
+ * curve, a bad com_gt) RIPP_AGG_MALFORMED, RIPP_ERR_ARG for an element outside its prime-order subgroup
+ * RIPP_AGG_NOT_IN_SUBGROUP.  *n_accepted counts the RIPP_AGG_OK.  No status depends on the other openings, and no
+ * randomness is drawn: every check of ripp_pc_verify is decided exactly (DESIGN.md §4).  A false or malformed opening
+ * is data, not an error.  The checks run before any work is queued, in this order: a null ctx or n_accepted, or a bad
+ * kind (RIPP_ERR_ARG); count == 0 (RIPP_OK); other null pointers (RIPP_ERR_ARG); the trusted kind without vsrs
+ * (RIPP_ERR_ARG); transparent: null keys, then the shape of ripp_pc_commit_dev (RIPP_ERR_NOT_POW2 before RIPP_ERR_ARG);
+ * count > 2^16, or transparent count n or count m > 2^24 (RIPP_ERR_ARG); proof_lens that do not sum to proofs_len
+ * (RIPP_ERR_ARG).  The number of kernel launches depends on (kind, n, m) and the longest proof, not on count; two host
+ * synchronisations.  Synchronous. */
+int ripp_pc_verify_batch(ripp_ctx* ctx, int kind, const void* vsrs, const void* first_tier_dev, size_t m,
+                         const void* second_tier_dev, size_t n, size_t count, const void* com_gts, const void* x_host,
+                         const void* y_host, const void* evals, const uint8_t* proofs, size_t proofs_len,
+                         const size_t* proof_lens, uint8_t* status_out, size_t* n_accepted);
 
 /* ---- diagnostics --------------------------------------------------------------------------- */
 /* Element-wise primitive ops on device, used by the GPU parity tests to pin the PTX limb layer:

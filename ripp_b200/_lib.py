@@ -589,6 +589,25 @@ class Context:
                                    ctypes.byref(acc)))
         return bool(acc.value)
 
+    def pc_verify_batch(self, kind, vsrs, first_dev, m, second_dev, n, coms, xs, ys, evaluations, proofs):
+        """coms: (count, 144) uint32 GT; xs, ys, evaluations: (count, 8) uint32 Montgomery; proofs[k]: bytes.  -> np.uint8
+        array of ripp_agg_status, one per opening."""
+        count = len(proofs)
+
+        def rows(a, w):
+            return np.ascontiguousarray(np.asarray(a, dtype=np.uint32).reshape(-1, w) if count else np.zeros((1, w), np.uint32))
+
+        gt, x, y, ev = rows(coms, 144), rows(xs, 8), rows(ys, 8), rows(evaluations, 8)
+        lens = np.array([len(p) for p in proofs] or [0], dtype=np.uintp)
+        data = b"".join(bytes(p) for p in proofs)
+        pb = self._bytes(data)
+        st = np.zeros(max(count, 1), dtype=np.uint8)
+        acc = ctypes.c_size_t()
+        check(lib().ripp_pc_verify_batch(self.handle, int(kind), _p(vsrs), _p(first_dev), ctypes.c_size_t(m), _p(second_dev),
+                                         ctypes.c_size_t(n), ctypes.c_size_t(count), _p(gt), _p(x), _p(y), _p(ev), _p(pb),
+                                         ctypes.c_size_t(len(data)), _p(lens), _p(st), ctypes.byref(acc)))
+        return st[:count]
+
     # ---- verifiers --------------------------------------------------------------------------------
     def gt_multiexp_dev(self, gt_dev, fr_dev, n, out_dev):
         check(lib().ripp_gt_multiexp_dev(self.handle, _p(gt_dev), _p(fr_dev), ctypes.c_size_t(n), _p(out_dev)))

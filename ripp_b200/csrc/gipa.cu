@@ -932,4 +932,5 @@ extern "C" int ripp_sipp_prove(ripp_ctx* ctx, const void* a_aff, const void* b_a
 #include "poly_commit.cuh"
 #include "aggregate_batch.cuh"
 #include "pc_batch.cuh"
+#include "pc_verify_batch.cuh"
 #include "sharded.cuh"

@@ -96,5 +96,13 @@ RIPP_HD Fr pow2k(Fr s, unsigned e) {
   return s;
 }
 
+// exponent e of a GIPA verifier's final commitment key (gipa.rs:365-399, the order of verify.cuh's final_key_exponents):
+// acc times tinv[j] for every bit j set in e, tinv[j] the inverse of transcript element j (last round first)
+RIPP_HD Fr key_exponent(const Fr* tinv, size_t e, Fr acc) {
+  for (unsigned j = 0; e; j++, e >>= 1)
+    if (e & 1) acc = acc * tinv[j];
+  return acc;
+}
+
 }  // namespace pc
 }  // namespace ripp

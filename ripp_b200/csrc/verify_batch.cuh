@@ -96,24 +96,30 @@ static void agg_fiat_shamir(AggBatchItem& a) {
 
 static size_t up256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// Subgroup checks of every decoded element of the aggregates with status OK, one launch per group, failures recorded
-// per aggregate.  The host Fiat-Shamir work runs while the checks do; one synchronisation.
-static int agg_subgroups(ripp_ctx* ctx, std::vector<AggBatchItem>& it) {
+// the elements one reader decoded and the word of the failure flags they set
+struct SubgroupSrc {
+  const Reader* rd;
+  uint32_t owner;
+};
+
+// Subgroup checks of the elements of every source, one launch per group, a failure ORed into (*bad_h)[owner] (K words).
+// host_work runs while the checks do; one synchronisation.
+template <class Fn>
+static int batch_subgroups(ripp_ctx* ctx, const std::vector<SubgroupSrc>& src, size_t K, Fn host_work, std::vector<uint32_t>* bad_h) {
   std::vector<G1Aff> g1;
   std::vector<G2Aff> g2;
   std::vector<Fq12> gt;
   std::vector<uint32_t> o1, o2, ot;
-  for (size_t k = 0; k < it.size(); k++) {
-    if (it[k].status != RIPP_AGG_OK) continue;
-    const Reader& r = it[k].rd;
+  for (const SubgroupSrc& s : src) {
+    const Reader& r = *s.rd;
     g1.insert(g1.end(), r.g1s.begin(), r.g1s.end());
     g2.insert(g2.end(), r.g2s.begin(), r.g2s.end());
     gt.insert(gt.end(), r.gts.begin(), r.gts.end());
-    o1.resize(g1.size(), (uint32_t)k);
-    o2.resize(g2.size(), (uint32_t)k);
-    ot.resize(gt.size(), (uint32_t)k);
+    o1.resize(g1.size(), s.owner);
+    o2.resize(g2.size(), s.owner);
+    ot.resize(gt.size(), s.owner);
   }
-  const size_t K = it.size(), o_g2 = up256(g1.size() * 96), o_gt = o_g2 + up256(g2.size() * 192),
+  const size_t o_g2 = up256(g1.size() * 96), o_gt = o_g2 + up256(g2.size() * 192),
                o_o1 = o_gt + up256(gt.size() * 576), o_o2 = o_o1 + up256(o1.size() * 4), o_ot = o_o2 + up256(o2.size() * 4),
                o_bad = o_ot + up256(ot.size() * 4);
   std::vector<uint8_t> H(o_bad);
@@ -141,17 +147,31 @@ static int agg_subgroups(ripp_ctx* ctx, std::vector<AggBatchItem>& it) {
     LAUNCHED(ctx);
   }
   OK(ripp_gt_check_l6(ctx, D + o_gt, gt.size(), bad, 4u, (const uint32_t*)(D + o_ot)));
-  // tipa_verify_parsed rejects a proof without rounds (its transcript has no first element)
-  for (AggBatchItem& a : it) {
-    if (a.status != RIPP_AGG_OK) continue;
-    if (a.p.pab.gipa.steps.empty() || a.p.pc.gipa.steps.empty())
-      a.status = RIPP_AGG_REJECTED;
-    else
-      agg_fiat_shamir(a);
-  }
-  std::vector<uint32_t> bad_h(K);
-  CU(cudaMemcpyAsync(bad_h.data(), bad, K * 4, cudaMemcpyDeviceToHost, st));
+  host_work();
+  bad_h->assign(K, 0);
+  CU(cudaMemcpyAsync(bad_h->data(), bad, K * 4, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
+  return RIPP_OK;
+}
+
+// Subgroup checks of every decoded element of the aggregates with status OK, failures recorded per aggregate, and the
+// host Fiat-Shamir work while they run.
+static int agg_subgroups(ripp_ctx* ctx, std::vector<AggBatchItem>& it) {
+  const size_t K = it.size();
+  std::vector<SubgroupSrc> src;
+  for (size_t k = 0; k < K; k++)
+    if (it[k].status == RIPP_AGG_OK) src.push_back(SubgroupSrc{&it[k].rd, (uint32_t)k});
+  std::vector<uint32_t> bad_h;
+  OK(batch_subgroups(ctx, src, K, [&] {
+    // tipa_verify_parsed rejects a proof without rounds (its transcript has no first element)
+    for (AggBatchItem& a : it) {
+      if (a.status != RIPP_AGG_OK) continue;
+      if (a.p.pab.gipa.steps.empty() || a.p.pc.gipa.steps.empty())
+        a.status = RIPP_AGG_REJECTED;
+      else
+        agg_fiat_shamir(a);
+    }
+  }, &bad_h));
   for (size_t k = 0; k < K; k++)
     if (bad_h[k] && it[k].status != RIPP_AGG_MALFORMED) it[k].status = RIPP_AGG_NOT_IN_SUBGROUP;
   return RIPP_OK;

@@ -4,7 +4,9 @@ BivariatePolynomialCommitment :153-284, UnivariatePolynomialCommitment :286-377;
 
 Commit is one segmented MSM of the Y polynomials over the shared first-tier bases plus the AFGHO pairing product; open
 keeps the powers of x, the row combination y_eval, y_eval_comm, the KZG quotient and the inner-product arguments on the
-device; verify is `ripp_pc_verify`.  Polynomials are coefficient lists of ints (lowest degree first); a bivariate
+device; verify is `ripp_pc_verify`, and `verify_batch` checks many openings in one call (`ripp_pc_verify_batch`), one
+status per opening: the `AGG_*` constants of `ripp_b200.ip_proofs` (AGG_OK where `verify` accepts, AGG_REJECTED where
+it returns False, AGG_MALFORMED / AGG_NOT_IN_SUBGROUP where it raises on the proof's bytes).  Polynomials are coefficient lists of ints (lowest degree first); a bivariate
 polynomial is the list of its Y polynomials.  The `*_dev` methods take the coefficients already on the device, row-major
 with row length y_degree + 1 (include/ripp_b200.h "Coefficient layout"; a univariate polynomial is already in it), so
 that large polynomials skip the host encoding.  Setup takes alpha, beta explicitly (SURVEY.md §8d).  No CPU fallback:
@@ -13,7 +15,7 @@ import math
 
 from . import _lib, codec
 from .inner_products import default_context
-from .ip_proofs import vsrs_enc
+from .ip_proofs import AGG_MALFORMED, AGG_NOT_IN_SUBGROUP, AGG_OK, AGG_REJECTED, vsrs_enc  # noqa: F401 (re-exported)
 
 R = codec.R
 
@@ -89,6 +91,14 @@ def _open_batch(cls, key, flats, y_polynomial_comms, points, ctx):
     bufs = [_upload_fr(ctx, c) for c in flats]
     y_coms = ctx.to_device(codec.g1_vec_enc([p for coms in y_polynomial_comms for p in coms])) if flats else None
     return cls.open_batch_dev(key, [b for b, _ in bufs], [k for _, k in bufs], y_coms, points, ctx)[0]
+
+
+def _verify_batch(ctx, kind, vsrs, first, second, coms, points, evaluations, proofs):
+    """ripp_pc_verify_batch; first / second: (DeviceBuffer, length) or (None, 0).  -> np.uint8 statuses."""
+    ctx = ctx or default_context()
+    (f, m), (s, n) = first, second
+    return ctx.pc_verify_batch(kind, vsrs, f, m, s, n, [codec.gt_enc(c) for c in coms], [codec.fr_enc(x % R) for x, _ in points],
+                               [codec.fr_enc(y % R) for _, y in points], [codec.fr_enc(e % R) for e in evaluations], proofs)
 
 
 def quotient_by_linear(coeffs, z):
@@ -218,6 +228,12 @@ class BivariatePolynomialCommitment:
         return ctx.pc_verify(_lib.PC_TRUSTED, vsrs_enc(v_srs), None, 0, None, 0, codec.gt_enc(com), codec.fr_enc(x % R),
                              codec.fr_enc(y % R), codec.fr_enc(evaluation % R), proof)
 
+    @staticmethod
+    def verify_batch(v_srs, coms, points, evaluations, proofs, ctx=None):
+        """Opening k is (coms[k], points[k] = (x, y), evaluations[k], proofs[k]); openings of different shapes under one
+        v_srs may share a call.  -> np.uint8 array of AGG_* statuses, entry k as verify decides opening k alone."""
+        return _verify_batch(ctx, _lib.PC_TRUSTED, vsrs_enc(v_srs), (None, 0), (None, 0), coms, points, evaluations, proofs)
+
 
 class UnivariatePolynomialCommitment:
     """mod.rs:286-377.  The coefficients, read row-major with row length y_degree + 1, are the bivariate form."""
@@ -294,6 +310,13 @@ class UnivariatePolynomialCommitment:
     def verify(cls, v_srs, max_degree, com, point, evaluation, proof, ctx=None):
         _, yd = cls.bivariate_degrees(max_degree)
         return BivariatePolynomialCommitment.verify(v_srs, com, (pow(point, yd + 1, R), point), evaluation, proof, ctx)
+
+    @classmethod
+    def verify_batch(cls, v_srs, max_degree, coms, points, evaluations, proofs, ctx=None):
+        """points[k] = z_k, checked at (z_k^(y_degree + 1), z_k).  -> np.uint8 AGG_* statuses."""
+        _, yd = cls.bivariate_degrees(max_degree)
+        return BivariatePolynomialCommitment.verify_batch(v_srs, coms, [(pow(z, yd + 1, R), z) for z in points], evaluations,
+                                                          proofs, ctx)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -372,6 +395,11 @@ class TransparentBivariatePolynomialCommitment:
         return ctx.pc_verify(_lib.PC_TRANSPARENT, None, ck["first"][0], ck["first"][1], ck["second"][0], ck["second"][1],
                              codec.gt_enc(com), codec.fr_enc(x % R), codec.fr_enc(y % R), codec.fr_enc(evaluation % R), proof)
 
+    @staticmethod
+    def verify_batch(ck, coms, points, evaluations, proofs, ctx=None):
+        """Opening k is (coms[k], points[k] = (x, y), evaluations[k], proofs[k]) under ck.  -> np.uint8 AGG_* statuses."""
+        return _verify_batch(ctx, _lib.PC_TRANSPARENT, None, ck["first"], ck["second"], coms, points, evaluations, proofs)
+
 
 class TransparentUnivariatePolynomialCommitment:
     """transparent.rs:215-318."""
@@ -435,3 +463,10 @@ class TransparentUnivariatePolynomialCommitment:
     def verify(cls, ck, com, point, evaluation, proof, ctx=None):
         _, yd = cls.degrees_from_ck(ck)
         return TransparentBivariatePolynomialCommitment.verify(ck, com, (pow(point, yd + 1, R), point), evaluation, proof, ctx)
+
+    @classmethod
+    def verify_batch(cls, ck, coms, points, evaluations, proofs, ctx=None):
+        """points[k] = z_k, checked at (z_k^(y_degree + 1), z_k).  -> np.uint8 AGG_* statuses."""
+        _, yd = cls.degrees_from_ck(ck)
+        return TransparentBivariatePolynomialCommitment.verify_batch(ck, coms, [(pow(z, yd + 1, R), z) for z in points],
+                                                                     evaluations, proofs, ctx)

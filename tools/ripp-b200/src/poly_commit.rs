@@ -191,6 +191,37 @@ impl PcKeys {
         check(st, n, m)?;
         Ok(accept == 1)
     }
+
+    /// `verify` of many openings in one call (`ripp_pc_verify_batch`): opening k is (coms[k], points[k], evaluations[k],
+    /// proofs[k]).  -> one `ripp_agg_status` per opening (0 accepted, 1 malformed, 2 not in the subgroup, 3 rejected),
+    /// entry k as `verify` decides opening k alone.
+    pub fn verify_batch(&self, coms: &[PairingOutput<ark_bls12_381::Bls12_381>], points: &[(Fr, Fr)], evaluations: &[Fr],
+                        proofs: &[&[u8]]) -> Result<Vec<u8>, Error> {
+        let (n, m, count) = (self.second.len(), self.first.len(), proofs.len());
+        assert!(coms.len() == count && points.len() == count && evaluations.len() == count);
+        let vs = self.v_srs.as_ref().map(pack_vsrs);
+        let mut gt = Vec::with_capacity(72 * count);
+        for com in coms {
+            pack::put_fq12(&mut gt, &com.0);
+        }
+        let xs = pack::pack_fr(&points.iter().map(|p| p.0).collect::<Vec<_>>());
+        let ys = pack::pack_fr(&points.iter().map(|p| p.1).collect::<Vec<_>>());
+        let evs = pack::pack_fr(evaluations);
+        let lens: Vec<usize> = proofs.iter().map(|p| p.len()).collect();
+        let bytes: Vec<u8> = proofs.iter().flat_map(|p| p.iter().copied()).collect();
+        let mut status = vec![0u8; count];
+        let mut accepted = 0usize;
+        let c = ctx();
+        let st = unsafe {
+            sys::ripp_pc_verify_batch(c.raw(), self.kind(), vs.as_ref().map_or(std::ptr::null(), |v| v.as_ptr() as *const c_void),
+                                      self.first.ptr(), m, self.second.ptr(), n, count, gt.as_ptr() as *const c_void,
+                                      xs.as_ptr() as *const c_void, ys.as_ptr() as *const c_void, evs.as_ptr() as *const c_void,
+                                      bytes.as_ptr(), bytes.len(), lens.as_ptr(), status.as_mut_ptr(), &mut accepted)
+        };
+        drop(c);
+        check(st, n, m)?;
+        Ok(status)
+    }
 }
 
 /// `UnivariatePolynomialCommitment` (`mod.rs:286-377`) and its transparent twin: the coefficients are the bivariate
@@ -225,5 +256,11 @@ impl<'a> Univariate<'a> {
     pub fn open_batch(&self, coeffs: &[&DeviceVec<Fr>], y_coms: &DeviceVec<G1Affine>, zs: &[Fr]) -> Result<Vec<(Vec<u8>, Fr)>, Error> {
         let points: Vec<(Fr, Fr)> = zs.iter().map(|z| (self.point(z), *z)).collect();
         self.0.open_batch(coeffs, y_coms, &points)
+    }
+    /// opening k checked at (zs[k]^(y_degree + 1), zs[k]); -> one `ripp_agg_status` per opening
+    pub fn verify_batch(&self, coms: &[PairingOutput<ark_bls12_381::Bls12_381>], zs: &[Fr], evaluations: &[Fr], proofs: &[&[u8]])
+                        -> Result<Vec<u8>, Error> {
+        let points: Vec<(Fr, Fr)> = zs.iter().map(|z| (self.point(z), *z)).collect();
+        self.0.verify_batch(coms, &points, evaluations, proofs)
     }
 }

@@ -1,14 +1,15 @@
 """Timing of the batched polynomial commitments (ripp_pc_commit_batch_dev, ripp_pc_open_batch_dev; csrc/pc_batch.cuh)
-against K sequential ripp_pc_commit_dev / ripp_pc_open_dev calls on the same device buffers.  One JSON line per
-measurement:
+and of the batched verifier (ripp_pc_verify_batch; csrc/pc_verify_batch.cuh) against K sequential ripp_pc_commit_dev /
+ripp_pc_open_dev / ripp_pc_verify calls on the same inputs.  One JSON line per measurement:
 
   batch_vs_loop  both kinds, univariate polynomials of 2^10, 2^12 and 2^16 coefficients (the univariate wrappers'
                  bivariate shapes), K = 1, 8, 32 polynomials (seeded, full length, random points): host clock around one
-                 batch call and around K sequential single calls (all synchronous), commit and open separately,
+                 batch call and around K sequential single calls (all synchronous), commit, open and verify separately,
                  alternated, medians of --reps runs after one warm-up of each; the ratio batch / loop.  The bytes of every
-                 batch run are compared with the loop's.
-  split          one open at K = 32 and --split-coeffs coefficients per kind under torch.profiler: device time by kernel
-                 kind.
+                 batch run are compared with the loop's; verify checks the K openings just made (every status accepted,
+                 equal to the loop's verdicts).
+  split          one open and one verify at K = 32 and --split-coeffs coefficients per kind under torch.profiler: device
+                 time by kernel kind.
 device and power_limit_w are read in the same call.
 
 Usage: python tools/time_pc_batch.py [--reps 5] [--coeffs 10,12,16] [--ks 1,8,32] [--split-coeffs 12] [--out pc_batch.jsonl]
@@ -30,13 +31,17 @@ import torch  # noqa: E402
 
 from ripp_b200 import _lib, codec, synth  # noqa: E402
 from ripp_b200 import poly_commit as PC  # noqa: E402
+from ripp_b200.ip_proofs import AGG_OK, AGG_REJECTED, vsrs_enc  # noqa: E402
 
 KINDS = {
-    "pairing": ("k_miller6", "k_reduce6", "k_final_exp", "k_miller18", "k_reduce18"),
+    "pairing": ("k_miller6", "k_reduce6", "k_final_exp", "k_miller18", "k_reduce18", "k_groth16_check"),
     "msm": ("k_msm_",),
     "fold": ("k_fold",),
     "pc_scalar": ("k_pc_",),
     "gather": ("k_gather",),
+    "gt": ("k_gt_",),
+    "subgroup": ("k_subgroup",),
+    "g1_scale_sum": ("k_scale", "k_aff_seg_sum", "k_normalize"),
 }
 R = codec.R
 
@@ -53,13 +58,13 @@ def card():
 
 
 def keys(ctx, kind, lg):
-    """The univariate wrappers' keys for polynomials of 2^lg coefficients: (first, m, second, n, h_beta_powers)."""
+    """The univariate wrappers' keys for polynomials of 2^lg coefficients: (first, m, second, n, h_beta_powers, vsrs)."""
     if kind == _lib.PC_TRUSTED:
         xd, yd = PC.UnivariatePolynomialCommitment.bivariate_degrees((1 << lg) - 1)
         srs = PC.BivariatePolynomialCommitment.setup(xd, yd, 12345, 67890, ctx)
-        return srs["kzg"][0], yd + 1, srs["ck"][0], xd + 1, srs["h_beta_powers"][0]
+        return srs["kzg"][0], yd + 1, srs["ck"][0], xd + 1, srs["h_beta_powers"][0], vsrs_enc(srs["v_srs"])
     xd, yd = PC.TransparentUnivariatePolynomialCommitment.bivariate_degrees((1 << lg) - 1)
-    return synth.g1_points_dev(ctx, "tpcb-1", yd + 1), yd + 1, synth.g2_points_dev(ctx, "tpcb-2", xd + 1), xd + 1, None
+    return synth.g1_points_dev(ctx, "tpcb-1", yd + 1), yd + 1, synth.g2_points_dev(ctx, "tpcb-2", xd + 1), xd + 1, None, None
 
 
 def words(seed, count):
@@ -94,7 +99,7 @@ def main():
     for kind in (_lib.PC_TRUSTED, _lib.PC_TRANSPARENT):
         kname = "trusted" if kind == _lib.PC_TRUSTED else "transparent"
         for lg in (int(x) for x in args.coeffs.split(",")):
-            first, m, second, n, g2 = keys(ctx, kind, lg)
+            first, m, second, n, g2, vsrs = keys(ctx, kind, lg)
             N = n * m
             pool = [ctx.to_device(words(1000 * lg + i, N)) for i in range(kmax)]
             rng = np.random.default_rng(lg)
@@ -119,8 +124,25 @@ def main():
                     r = [ctx.pc_open_dev(kind, first, m, second, n, g2, bufs[i], N, ysingle[i], xs[i], ys[i]) for i in range(K)]
                     return [p for p, _ in r], [e.tolist() for _, e in r]
 
-                for what, batch, loop in (("commit", commit_batch, commit_loop), ("open", open_batch, open_loop)):
+                opened = {}
+
+                def verify_batch():
+                    coms, (proofs, evs) = opened["v"]
+                    return ctx.pc_verify_batch(kind, vsrs, first, m, second, n, coms, xs, ys, evs, proofs).tolist()
+
+                def verify_loop():
+                    coms, (proofs, evs) = opened["v"]
+                    return [AGG_OK if ctx.pc_verify(kind, vsrs, first, m, second, n, coms[i], xs[i], ys[i], evs[i], proofs[i])
+                            else AGG_REJECTED for i in range(K)]
+
+                for what, batch, loop in (("commit", commit_batch, commit_loop), ("open", open_batch, open_loop),
+                                          ("verify", verify_batch, verify_loop)):
+                    if what == "verify":
+                        proofs, evs = open_batch()
+                        opened["v"] = (np.array(commit_batch(), dtype=np.uint32), (proofs, np.array(evs, dtype=np.uint32)))
                     want = loop()
+                    if what == "verify":
+                        assert want == [AGG_OK] * K, "an honest opening was rejected"
                     assert batch() == want, "batch bytes differ from the single calls (%s %s 2^%d, K = %d)" % (kname, what, lg, K)
                     tb, tl = [], []
                     for _ in range(args.reps):
@@ -142,26 +164,30 @@ def main():
 
     for kind in (_lib.PC_TRUSTED, _lib.PC_TRANSPARENT):
         K, lg = 32, args.split_coeffs
-        first, m, second, n, g2 = keys(ctx, kind, lg)
+        first, m, second, n, g2, vsrs = keys(ctx, kind, lg)
         bufs = [ctx.to_device(words(77 + i, n * m)) for i in range(K)]
         yb = ctx.alloc(K * n * 96)
         xs = np.stack([codec.fr_enc(3 + i) for i in range(K)])
         ys = np.stack([codec.fr_enc(5 + i) for i in range(K)])
-        ctx.pc_commit_batch_dev(first, m, second, n, bufs, [n * m] * K, yb)
-        ctx.pc_open_batch_dev(kind, first, m, second, n, g2, bufs, [n * m] * K, yb, xs, ys)
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            ctx.pc_open_batch_dev(kind, first, m, second, n, g2, bufs, [n * m] * K, yb, xs, ys)
-            torch.cuda.synchronize()
-        split = {s: 0.0 for s in KINDS}
-        split["other"] = 0.0
-        for ev in prof.events():
-            if ev.device_type != torch.autograd.DeviceType.CUDA:
-                continue
-            ms = (ev.device_time if hasattr(ev, "device_time") else ev.cuda_time) / 1e3
-            kk = next((s for s, names in KINDS.items() if any(x in ev.name for x in names)), "other")
-            split[kk] += ms
-        emit({"what": "split", "kind": "trusted" if kind == _lib.PC_TRUSTED else "transparent", "coeffs": n * m, "k": K,
-              **{s + "_ms": v for s, v in split.items()}, "kernels_ms": sum(split.values())})
+        coms = np.array(ctx.pc_commit_batch_dev(first, m, second, n, bufs, [n * m] * K, yb), dtype=np.uint32)
+        proofs, evs = ctx.pc_open_batch_dev(kind, first, m, second, n, g2, bufs, [n * m] * K, yb, xs, ys)
+        ctx.pc_verify_batch(kind, vsrs, first, m, second, n, coms, xs, ys, evs, proofs)
+        ops = {"open": lambda: ctx.pc_open_batch_dev(kind, first, m, second, n, g2, bufs, [n * m] * K, yb, xs, ys),
+               "verify": lambda: ctx.pc_verify_batch(kind, vsrs, first, m, second, n, coms, xs, ys, evs, proofs)}
+        for op, run in ops.items():
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                run()
+                torch.cuda.synchronize()
+            split = {s: 0.0 for s in KINDS}
+            split["other"] = 0.0
+            for ev in prof.events():
+                if ev.device_type != torch.autograd.DeviceType.CUDA:
+                    continue
+                ms = (ev.device_time if hasattr(ev, "device_time") else ev.cuda_time) / 1e3
+                kk = next((s for s, names in KINDS.items() if any(x in ev.name for x in names)), "other")
+                split[kk] += ms
+            emit({"what": "split", "kind": "trusted" if kind == _lib.PC_TRUSTED else "transparent", "op": op, "coeffs": n * m,
+                  "k": K, **{s + "_ms": v for s, v in split.items()}, "kernels_ms": sum(split.values())})
     ctx.close()
 
 
